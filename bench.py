@@ -7,6 +7,7 @@ re-expansion (trimmed bases + qualities of every kept read).  F.hmm (Fungi) is m
 the largest present analogue M.hmm (Metazoa, 98 ITS1 profiles) stands in -- stated in `config`.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2] [--scale S] [--impl reference] [--replicas]
+                  [--dump-outputs DIR]
 
 value  reads/s with the reads (bases, qualities, offsets) resident in HBM when the timed region starts
 e2e    reads/s through the C-ABI call with pinned HOST buffers: itsx_run_trim = H2D of bases + qualities + offsets,
@@ -229,6 +230,20 @@ def emit(line):
 
 _REAL_STDOUT = 1
 
+DUMP_MAX_ELEMS = 1 << 20     # two legs x (2 float64 arrays of <= 8 MB + 2 float32 arrays of <= 4 MB): <= 48 MB in all
+
+
+def dump_outputs(dirname, arrays):
+    """Write every array as DIR/<name>.npy so that two builds can be compared output for output: bytes as float32,
+    wider integers as float64 (both exact).  An array longer than DUMP_MAX_ELEMS is cut to the elements at a fixed,
+    seeded, sorted sample of its indices; arrays of equal length are sampled at the same positions."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.size > DUMP_MAX_ELEMS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a.astype(np.float32 if a.dtype.itemsize == 1 else np.float64))
+
 
 def search_stages(ss_sum, sec, dsec, ds, nreads, L, pk, world=1):
     """Per-stage rates from the search / derep counters (cells summed over ranks, seconds = max over ranks)."""
@@ -447,6 +462,10 @@ def run_single(args, rank, world, local):
     l0 = ctx.launch_count()
     ms_dev, ms_wall = timed(step_resident, args.steps)
     launches = ctx.launch_count() - l0
+    # what the last resident step left on the device (untimed; the e2e leg below overwrites it)
+    resident_out = None
+    if rank == 0 and args.dump_outputs:
+        resident_out = dict(zip(("kept_index", "out_off", "out_seq", "out_qual"), ctx.run_fetch()))
     # ---- e2e leg: host buffers in, trimmed records out ----
     rs_e2e = None
     for _ in range(2):
@@ -458,6 +477,12 @@ def run_single(args, rank, world, local):
     ms_e2e_dev, ms_e2e_wall = timed(step_e2e, args.steps)
     clocks = clk.stop()
     rs_e2e = last["e2e"]
+    if rank == 0 and args.dump_outputs:
+        arrays = {}
+        for leg, out, st in (("resident", resident_out, last["run"]), ("e2e", last["e2e_out"], rs_e2e)):
+            arrays.update({"%s_%s" % (leg, k): out[k] for k in ("kept_index", "out_off", "out_seq", "out_qual")})
+            arrays["%s_counts" % leg] = np.array([st.n_reads, st.n_unique, st.n_kept, st.out_bytes], np.int64)
+        dump_outputs(args.dump_outputs, arrays)
 
     total_reads = nreads * world
     value = total_reads / (ms_dev / 1e3 / args.steps)
@@ -802,10 +827,19 @@ def main():
                     help="N > 1: one independent sample per rank (weak scaling, no collective) instead of ONE sample "
                          "sharded over the ranks")
     ap.add_argument("--sharded", action="store_true", help="accepted for compatibility: sharding is the N > 1 default")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step of each timed leg returned (kept index, "
+                         "offsets, trimmed bases and qualities, counts) as DIR/<leg>_<name>.npy in float32 / float64; "
+                         "arrays longer than %d elements as a fixed, seeded sample" % DUMP_MAX_ELEMS)
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or (world > 1 and not args.replicas)):
+        ap.error("--dump-outputs writes the outputs of one GPU's sample: use it on the GPU path with one GPU or "
+                 "--replicas")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return

@@ -19,12 +19,13 @@ def stub(sample, results, tempdir, threads, taxa, region, paired_in, paired_out,
 def main():
     src, out = sys.argv[1], sys.argv[2]
     engine = sys.argv[3] if len(sys.argv) > 3 else "stub"
+    if engine == "oracle":
+        os.environ["ITSX_GZIP"] = "host"        # no device on any rank: zlib writes the .gz output (read at import)
     import torch.distributed as dist
     from itsxpress_b200 import q2_itsxpress as q2
     dist.init_process_group("gloo")
     if engine == "oracle":
         # the REAL per-sample / batched pipeline of every rank, with the CPU oracle standing in for its device
-        os.environ["ITSX_GZIP"] = "host"
         sys.path.insert(0, os.path.join(ROOT, "tests"))
         from itsxpress_b200 import SeqSample
         from oracle import oracle as O

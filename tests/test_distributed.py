@@ -12,6 +12,14 @@ from conftest import ROOT
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 
+def _free_port():
+    """A port nobody holds right now, for the gloo rendezvous of the ranks a test starts."""
+    import socket
+    with socket.socket() as sock:
+        sock.bind(("127.0.0.1", 0))
+        return sock.getsockname()[1]
+
+
 def _single(O, eng, seq, off):
     rep, strand, nu = O.derep(seq, off)
     idx = np.flatnonzero(rep == np.arange(len(rep)))
@@ -30,7 +38,7 @@ def _single(O, eng, seq, off):
 @pytest.mark.parametrize("world", [1, 2, 3])
 def test_run_sharded_equals_single(tmp_path, world):
     import dist_worker as W
-    port = 29650 + world
+    port = _free_port()
     procs = []
     for r in range(world):
         env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port),
@@ -85,7 +93,7 @@ def test_q2_samples_dealt_to_ranks(tmp_path, world):
             sizes[sid] = sizes.get(sid, 0) + os.path.getsize(str(src / fn))
     (src / "MANIFEST").write_text("\n".join(lines) + "\n")
     out = tmp_path / "out"
-    port = 29750 + world
+    port = _free_port()
     procs = []
     for r in range(world):
         env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), LOCAL_RANK=str(r), MASTER_ADDR="127.0.0.1",
@@ -115,10 +123,7 @@ def test_q2_main_sharded_two_ranks_real_pipeline_on_the_oracle(tmp_path, oracle,
     from test_gpu_merge import _make_artifact
     art = _make_artifact(str(tmp_path / "in"), [60, 17, 40, 0, 25])
     out = tmp_path / "out"
-    import socket
-    with socket.socket() as sock:                       # a port nobody holds right now
-        sock.bind(("127.0.0.1", 0))
-        port = sock.getsockname()[1]
+    port = _free_port()
     world = 2
     procs = []
     for r in range(world):
@@ -132,7 +137,7 @@ def test_q2_main_sharded_two_ranks_real_pipeline_on_the_oracle(tmp_path, oracle,
     assert sorted(sum(mine, [])) == ["S0", "S1", "S2", "S3", "S4"] and all(mine)
     ctx = OracleContext(oracle)
     monkeypatch.setattr(SeqSample, "get_context", lambda: ctx)
-    monkeypatch.setenv("ITSX_GZIP", "host")
+    monkeypatch.setattr(fq, "GZIP_BACKEND", "host")
     SeqSample.reset_sessions()
     ref = q2.trim_pair_output_unmerged(q2.PerSampleDir(art), region="ITS2", taxa="M")
     names = sorted(f for f in os.listdir(str(ref)) if f.endswith(".gz"))

@@ -26,7 +26,6 @@ import pytest
 from conftest import HMM_DIR, TD
 
 REP_FA = os.path.join(TD, "ex_tmpdir", "rep.fa")
-REF = "/root/reference"          # exists in the build container only; never on the GPU box (these tests are not gpu-marked)
 
 
 def read_fasta(path):
@@ -170,16 +169,13 @@ def test_oracle_against_a_live_hmmsearch(oracle, tmp_path):
         assert_pinned(res)
 
 
-def _first_existing(*paths):
-    return next((p for p in paths if os.path.exists(p)), None)
+DOMTBL_FIXTURE = os.path.join(TD, "ex_tmpdir", "domtbl.txt")
+F_HMM = os.path.join(HMM_DIR, "F.hmm")
 
 
-DOMTBL_FIXTURE = _first_existing(os.path.join(TD, "ex_tmpdir", "domtbl.txt"), os.path.join(REF, "tests", "test_data", "ex_tmpdir", "domtbl.txt"))
-F_HMM = _first_existing(os.path.join(HMM_DIR, "F.hmm"), os.path.join(REF, "itsxpress", "ITSx_db", "HMMs", "F.hmm"))
-
-
-@pytest.mark.skipif(DOMTBL_FIXTURE is None or F_HMM is None,
-                    reason="the reference's domtbl.txt fixture and F.hmm are missing from the mount (.MISSING_LARGE_BLOBS)")
+@pytest.mark.skipif(not (os.path.exists(DOMTBL_FIXTURE) and os.path.exists(F_HMM)),
+                    reason="the reference's domtbl.txt fixture and F.hmm are not in tests/test_data and ITSx_db "
+                           "(the reference ships neither)")
 def test_oracle_against_the_references_domtbl_fixture(oracle):
     ids, seqs = read_fasta(REP_FA)
     ref = parse_domtbl(DOMTBL_FIXTURE)
