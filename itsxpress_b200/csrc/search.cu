@@ -44,6 +44,12 @@ constexpr int SPEC_C = 5;                  // parser specials kept per row
 constexpr int ENV_ROWF = MAXM + 1;             // floats per envelope row: M[1..45] (cols 0..44), Eraw (col 45)
 constexpr int ENV_ROWBYTES = ENV_ROWF * 32 * 4;    // one row of one warp: 5 888 B, contiguous
 constexpr int ENV_RING = 2;                    // rows of the Backward read-back ring per warp (a power of two; 4 measured slower)
+// The parser specials (d_spec) and the envelope rows (d_envscratch) are sized by the longest searched sequence: about
+// 18 MB and 56 MB per residue at full occupancy, so one read of a few kb would ask for more HBM than the GPU has.  Each
+// buffer is held to a byte budget by running fewer tiles / warps per launch when the sequences are long; neither
+// budget binds below ~600 bp, so short-read samples keep their full occupancy.
+constexpr size_t FB_SCRATCH_BUDGET = (size_t)16 << 30;
+constexpr size_t ENV_SCRATCH_BUDGET = (size_t)32 << 30;
 static_assert((ENV_RING & (ENV_RING - 1)) == 0 && ENV_RING >= 2, "ring depth");
 constexpr double kLn2 = 0.69314718055994529;
 constexpr int ESTRIDE = 52;                // floats per residue row of the shared emission table (48 used)
@@ -2680,8 +2686,9 @@ int search_stage1(itsx_ctx *c)
         CUDA_TRY(c, c->d_env.ensure((size_t)n2 * ITSX_MAXDOM * 2 * 4));
         const size_t slab = (size_t)(Lmax + 1) * SPEC_C * 32 * 4;
         // the slab of a launch holds all its tiles (fbdec_kernel reads them back): a profile's worklist goes in pieces of
-        // at most two tiles per resident warp
-        const int fb_piece_tiles = fb_warps_per_lane * 2;
+        // at most two tiles per resident warp, and no more than fit the scratch budget
+        const int fb_piece_tiles = (int)std::max<size_t>(
+            1, std::min<size_t>((size_t)fb_warps_per_lane * 2, FB_SCRATCH_BUDGET / (slab * NLANE)));
         CUDA_TRY(c, c->d_spec.ensure(slab * (size_t)fb_piece_tiles * NLANE));
         CUDA_TRY(c, c->d_fbscale.ensure((size_t)n2 * 4));
         CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
@@ -2869,12 +2876,15 @@ int search_stage1(itsx_ctx *c)
                 cub::DeviceRadixSort::SortPairs(c->d_tmp.p, tbs, key_in, key_out, wk_in, wk_out, nenv, 0, 12 + pbits, st);
             }
             c->launches += 2;
-            // envelopes are at most Lmax long; scratch per resident warp
+            // envelopes are at most Lmax long; scratch per warp of the grid, whose size the budget bounds
             const int Ldmax = Lmax;
             const size_t eslab = (size_t)(Ldmax + 1) * ENV_ROWF * 32 * 4;
+            const int env_wpc = ENV_THREADS / 32;
+            const int env_warps = (int)std::max<size_t>(
+                env_wpc, std::min<size_t>(env_warps_per_lane, ENV_SCRATCH_BUDGET / (eslab * NLANE) / env_wpc * env_wpc));
             const size_t env_smem = (size_t)(ENV_THREADS / 32) * ENV_RING * (ENV_ROWBYTES + 8);
             CUDA_TRY(c, cudaFuncSetAttribute(env_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env_smem));
-            CUDA_TRY(c, c->d_envscratch.ensure(eslab * env_warps_per_lane * NLANE));
+            CUDA_TRY(c, c->d_envscratch.ensure(eslab * env_warps * NLANE));
             CUDA_TRY(c, cudaEventRecord(c->ev_b, st));
             for (int l = 0; l < NLANE; l++) CUDA_TRY(c, cudaStreamWaitEvent(c->lanes[l], c->ev_b, 0));
             lane_rr = 0;
@@ -2891,14 +2901,13 @@ int search_stage1(itsx_ctx *c)
                 ea.order = d_order; ea.s0 = s0; ea.ns = ns; ea.prof = p;
                 ea.seqw = c->d_seqw.as<uint32_t>(); ea.woff = c->d_seqwoff.as<int64_t>(); ea.seqlen = c->d_seqlen.as<int32_t>();
                 ea.etab = c->d_etab.as<float>() + (size_t)p * (MAXM + 1) * 16;
-                ea.scratch = (float *)(c->d_envscratch.as<char>() + eslab * env_warps_per_lane * l);
+                ea.scratch = (float *)(c->d_envscratch.as<char>() + eslab * env_warps * l);
                 ea.Ldmax = Ldmax;
                 ea.out = c->d_envout.as<float>();
                 ea.out_base = e0;
                 ea.counters = cnt;
                 const int tiles = (cnte + 31) / 32;
-                const int wpc = ENV_THREADS / 32;
-                const int ctas = std::min((tiles + wpc - 1) / wpc, c->sm_count * ENV_CTAS_PER_SM);
+                const int ctas = std::min((tiles + env_wpc - 1) / env_wpc, env_warps / env_wpc);
                 env_kernel<<<ctas, ENV_THREADS, env_smem, c->lanes[l]>>>(c->pconst[p], ea);
                 c->launches++;
             }
