@@ -79,8 +79,7 @@ void itsx_destroy(itsx_ctx *c)
     cudaDeviceSynchronize();
     for (auto s : c->lanes) cudaStreamDestroy(s);
     for (auto e : c->lane_ev) cudaEventDestroy(e);
-    if (c->ev_a) cudaEventDestroy(c->ev_a);
-    if (c->ev_b) cudaEventDestroy(c->ev_b);
+    if (c->lane_fork) cudaEventDestroy(c->lane_fork);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }
@@ -726,24 +725,27 @@ int itsx_trim_gather_resident(itsx_ctx *c, int mode, int64_t *n_kept, int64_t *t
 
 // ---- whole path ------------------------------------------------------------------------------------------
 // derep -> search -> positions -> trim bounds [-> re-expansion of the kept slices when the qualities are resident]
-static int run_device_part(itsx_ctx *c, const itsx_search_params *prm, itsx_run_stats *rs, cudaEvent_t *ev)
+// events of a whole-path call: 0 start, 1 reads resident, 2 derep done, 3 search done, 4 trim done, 5 end, 6 gather done
+typedef Timeline<7> RunTimeline;
+
+static int run_device_part(itsx_ctx *c, const itsx_search_params *prm, itsx_run_stats *rs, const RunTimeline &tl)
 {
     cudaStream_t st = c->stream;
-    CUDA_TRY(c, cudaEventRecord(ev[1], st));
+    CUDA_TRY(c, tl.record(1, st));
     int rc = derep_run(c);
     if (rc) return rc;
     c->shard_first = 0;
     c->shard_n = -1;
     rc = search_build_seqs_from_derep(c);
     if (rc) return rc;
-    CUDA_TRY(c, cudaEventRecord(ev[2], st));
+    CUDA_TRY(c, tl.record(2, st));
     rc = set_params(c, prm);
     if (rc) return rc;
     rc = search_stage1(c);
     if (rc) return rc;
     rc = search_stage2(c);
     if (rc) return rc;
-    CUDA_TRY(c, cudaEventRecord(ev[3], st));
+    CUDA_TRY(c, tl.record(3, st));
     const int64_t n = c->nreads;
     CUDA_TRY(c, c->r_keep.ensure((size_t)n + 16));
     CUDA_TRY(c, c->r_lo.ensure((size_t)n * 4 + 16));
@@ -751,7 +753,7 @@ static int run_device_part(itsx_ctx *c, const itsx_search_params *prm, itsx_run_
     int64_t nk = 0;
     rc = trim_bounds_dev(c, 0, nullptr, n, c->r_keep.as<uint8_t>(), c->r_lo.as<int32_t>(), c->r_hi.as<int32_t>(), &nk);
     if (rc) return rc;
-    CUDA_TRY(c, cudaEventRecord(ev[4], st));
+    CUDA_TRY(c, tl.record(4, st));
     rs->n_reads = n;
     rs->n_unique = c->n_unique;
     rs->n_kept = nk;
@@ -773,19 +775,19 @@ static int run_device_part(itsx_ctx *c, const itsx_search_params *prm, itsx_run_
         if (rc) return rc;
         c->r_gathered = true;
     }
-    CUDA_TRY(c, cudaEventRecord(ev[6], st));
+    CUDA_TRY(c, tl.record(6, st));
     return ITSX_OK;
 }
 
-static void run_times(itsx_run_stats &rs, cudaEvent_t *ev, bool with_copies)
+static void run_times(itsx_run_stats &rs, const RunTimeline &tl, bool with_copies)
 {
-    if (with_copies) cudaEventElapsedTime(&rs.ms_h2d, ev[0], ev[1]);
-    cudaEventElapsedTime(&rs.ms_derep, ev[1], ev[2]);
-    cudaEventElapsedTime(&rs.ms_search, ev[2], ev[3]);
-    cudaEventElapsedTime(&rs.ms_trim, ev[3], ev[4]);
-    cudaEventElapsedTime(&rs.ms_gather, ev[4], ev[6]);
-    if (with_copies) cudaEventElapsedTime(&rs.ms_d2h, ev[6], ev[5]);
-    cudaEventElapsedTime(&rs.ms_total, ev[0], ev[5]);
+    if (with_copies) rs.ms_h2d = tl.ms(0, 1);
+    rs.ms_derep = tl.ms(1, 2);
+    rs.ms_search = tl.ms(2, 3);
+    rs.ms_trim = tl.ms(3, 4);
+    rs.ms_gather = tl.ms(4, 6);
+    if (with_copies) rs.ms_d2h = tl.ms(6, 5);
+    rs.ms_total = tl.ms(0, 5);
 }
 
 int itsx_quals_upload(itsx_ctx *c, const uint8_t *qual)
@@ -807,12 +809,12 @@ int itsx_run(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64_t nreads
     CHECK_CTX(c);
     CUDA_TRY(c, cudaSetDevice(c->device));
     itsx_run_stats rs{};
-    cudaEvent_t ev[7];
-    for (auto &e : ev) CUDA_TRY(c, cudaEventCreate(&e));
+    RunTimeline tl;
+    CUDA_TRY(c, tl.status);
     cudaStream_t st = c->stream;
-    CUDA_TRY(c, cudaEventRecord(ev[0], st));
+    CUDA_TRY(c, tl.record(0, st));
     int rc = itsx_reads_upload(c, seq, off, nreads);
-    if (!rc) rc = run_device_part(c, prm, &rs, ev);
+    if (!rc) rc = run_device_part(c, prm, &rs, tl);
     if (!rc && nreads) {
         if (rep_index) CUDA_TRY(c, cudaMemcpyAsync(rep_index, c->d_rep.p, (size_t)nreads * 4, cudaMemcpyDefault, st));
         if (keep) CUDA_TRY(c, cudaMemcpyAsync(keep, c->r_keep.p, (size_t)nreads, cudaMemcpyDefault, st));
@@ -820,12 +822,11 @@ int itsx_run(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64_t nreads
         if (hi) CUDA_TRY(c, cudaMemcpyAsync(hi, c->r_hi.p, (size_t)nreads * 4, cudaMemcpyDefault, st));
     }
     if (!rc) {
-        CUDA_TRY(c, cudaEventRecord(ev[5], st));
+        CUDA_TRY(c, tl.record(5, st));
         CUDA_TRY(c, cudaStreamSynchronize(st));
-        run_times(rs, ev, true);
+        run_times(rs, tl, true);
         if (out) *out = rs;
     }
-    for (auto &e : ev) cudaEventDestroy(e);
     return rc;
 }
 
@@ -834,18 +835,17 @@ int itsx_run_resident(itsx_ctx *c, const itsx_search_params *prm, itsx_run_stats
     CHECK_CTX(c);
     CUDA_TRY(c, cudaSetDevice(c->device));
     itsx_run_stats rs{};
-    cudaEvent_t ev[7];
-    for (auto &e : ev) CUDA_TRY(c, cudaEventCreate(&e));
+    RunTimeline tl;
+    CUDA_TRY(c, tl.status);
     cudaStream_t st = c->stream;
-    CUDA_TRY(c, cudaEventRecord(ev[0], st));
-    int rc = run_device_part(c, prm, &rs, ev);
+    CUDA_TRY(c, tl.record(0, st));
+    int rc = run_device_part(c, prm, &rs, tl);
     if (!rc) {
-        CUDA_TRY(c, cudaEventRecord(ev[5], st));
+        CUDA_TRY(c, tl.record(5, st));
         CUDA_TRY(c, cudaStreamSynchronize(st));
-        run_times(rs, ev, false);
+        run_times(rs, tl, false);
         if (out) *out = rs;
     }
-    for (auto &e : ev) cudaEventDestroy(e);
     return rc;
 }
 
@@ -875,13 +875,13 @@ int itsx_run_trim(itsx_ctx *c, const uint8_t *seq, const uint8_t *qual, const in
     CUDA_TRY(c, cudaSetDevice(c->device));
     if (nreads > 0 && !qual) { c->err = "run_trim: qualities are required"; return ITSX_EINVAL; }
     itsx_run_stats rs{};
-    cudaEvent_t ev[7];
-    for (auto &e : ev) CUDA_TRY(c, cudaEventCreate(&e));
+    RunTimeline tl;
+    CUDA_TRY(c, tl.status);
     cudaStream_t st = c->stream;
-    CUDA_TRY(c, cudaEventRecord(ev[0], st));
+    CUDA_TRY(c, tl.record(0, st));
     int rc = itsx_reads_upload(c, seq, off, nreads);
     if (!rc) rc = itsx_quals_upload(c, qual);
-    if (!rc) rc = run_device_part(c, prm, &rs, ev);
+    if (!rc) rc = run_device_part(c, prm, &rs, tl);
     if (!rc) {
         const int64_t nk = c->r_nkept, tot = c->r_total;
         if (rep_index && nreads) CUDA_TRY(c, cudaMemcpyAsync(rep_index, c->d_rep.p, (size_t)nreads * 4, cudaMemcpyDefault, st));
@@ -889,12 +889,11 @@ int itsx_run_trim(itsx_ctx *c, const uint8_t *seq, const uint8_t *qual, const in
         if (out_off) CUDA_TRY(c, cudaMemcpyAsync(out_off, c->r_oo.p, (size_t)(nk + 1) * 8, cudaMemcpyDefault, st));
         if (out_seq && tot) CUDA_TRY(c, cudaMemcpyAsync(out_seq, c->r_os.p, (size_t)tot, cudaMemcpyDefault, st));
         if (out_qual && tot) CUDA_TRY(c, cudaMemcpyAsync(out_qual, c->r_oq.p, (size_t)tot, cudaMemcpyDefault, st));
-        CUDA_TRY(c, cudaEventRecord(ev[5], st));
+        CUDA_TRY(c, tl.record(5, st));
         CUDA_TRY(c, cudaStreamSynchronize(st));
-        run_times(rs, ev, true);
+        run_times(rs, tl, true);
         if (out) *out = rs;
     }
-    for (auto &e : ev) cudaEventDestroy(e);
     return rc;
 }
 

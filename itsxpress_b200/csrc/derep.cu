@@ -332,26 +332,26 @@ int derep_run(itsx_ctx *c)
     const unsigned long long mask = (unsigned long long)cap - 1;
     const unsigned long long keymask = c->key_bits >= 64 ? ~0ull : ((1ull << c->key_bits) - 1ull);
 
-    cudaEvent_t ev[7];
-    for (auto &e : ev) CUDA_TRY(c, cudaEventCreate(&e));
+    Timeline<6> tl;     // the ends of pack, hash, insert, verify and compact
+    CUDA_TRY(c, tl.status);
     auto *P = c->d_pack2.as<uint32_t>();
     auto *X = c->d_exc.as<uint16_t>();
     auto *ascii = c->d_ascii.as<uint8_t>();
     auto *off = c->d_off.as<int64_t>();
     unsigned long long *d_ncol = c->d_counters.as<unsigned long long>() + CNT_COLLIDE;
 
-    CUDA_TRY(c, cudaEventRecord(ev[0], st));
+    CUDA_TRY(c, tl.record(0, st));
     CUDA_TRY(c, cudaMemsetAsync(P + nchunk, 0, 8, st));
     CUDA_TRY(c, cudaMemsetAsync(X + nchunk, 0, 4, st));
     pack2_kernel<<<nblk(nchunk, 256), 256, 0, st>>>((const uint4 *)ascii, nchunk, P, X);
-    CUDA_TRY(c, cudaEventRecord(ev[1], st));
+    CUDA_TRY(c, tl.record(1, st));
     const int32_t *d_samp = c->have_samples ? c->d_sample.as<int32_t>() : nullptr;
     hash_kernel<<<nblk(n, 128), 128, 0, st>>>(ascii, off, P, X, n, keymask, d_samp, c->d_key.as<unsigned long long>(),
                                               c->d_flags.as<uint8_t>());
-    CUDA_TRY(c, cudaEventRecord(ev[2], st));
+    CUDA_TRY(c, tl.record(2, st));
     table_init_kernel<<<nblk(cap, 256), 256, 0, st>>>(c->d_table.as<Slot>(), cap);
     insert_kernel<<<nblk(n, 256), 256, 0, st>>>(c->d_key.as<unsigned long long>(), n, c->d_table.as<Slot>(), mask);
-    CUDA_TRY(c, cudaEventRecord(ev[3], st));
+    CUDA_TRY(c, tl.record(3, st));
     CUDA_TRY(c, cudaMemsetAsync(c->d_abund.p, 0, (size_t)n * 4, st));
     CUDA_TRY(c, cudaMemsetAsync(d_ncol, 0, 8, st));
     verify_kernel<<<nblk(n, 128), 128, 0, st>>>(ascii, off, P, c->d_key.as<unsigned long long>(),
@@ -374,16 +374,15 @@ int derep_run(itsx_ctx *c)
         c->launches++;
     }
     ds.n_collided = (int64_t)ncol;
-    CUDA_TRY(c, cudaEventRecord(ev[4], st));
+    CUDA_TRY(c, tl.record(4, st));
 
     // dense ids
     int32_t *flag = c->d_flag.as<int32_t>(), *scan = c->d_scan.as<int32_t>();
     isrep_kernel<<<nblk(n, 256), 256, 0, st>>>(c->d_rep.as<int32_t>(), n, flag);
-    size_t tmpb = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, tmpb, flag, scan, (int)n + 1, st);
-    CUDA_TRY(c, c->d_tmp.ensure(tmpb));
     CUDA_TRY(c, cudaMemsetAsync(flag + n, 0, 4, st));
-    cub::DeviceScan::ExclusiveSum(c->d_tmp.p, tmpb, flag, scan, (int)n + 1, st);
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
+        return cub::DeviceScan::ExclusiveSum(t, b, flag, scan, (int)n + 1, st);
+    }));
     int32_t nu = 0;
     CUDA_TRY(c, cudaMemcpyAsync(&nu, scan + n, 4, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
@@ -392,16 +391,15 @@ int derep_run(itsx_ctx *c)
     first_kernel<<<nblk(n, 256), 256, 0, st>>>(c->d_rep.as<int32_t>(), scan, n, c->d_first.as<int32_t>());
     uid_kernel<<<nblk(n, 256), 256, 0, st>>>(c->d_rep.as<int32_t>(), scan, n, c->d_uid.as<int32_t>());
     c->launches += 5;
-    CUDA_TRY(c, cudaEventRecord(ev[5], st));
+    CUDA_TRY(c, tl.record(5, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     CUDA_TRY(c, cudaGetLastError());
-    cudaEventElapsedTime(&ds.ms_pack, ev[0], ev[1]);
-    cudaEventElapsedTime(&ds.ms_hash, ev[1], ev[2]);
-    cudaEventElapsedTime(&ds.ms_insert, ev[2], ev[3]);
-    cudaEventElapsedTime(&ds.ms_verify, ev[3], ev[4]);
-    cudaEventElapsedTime(&ds.ms_compact, ev[4], ev[5]);
-    cudaEventElapsedTime(&ds.ms_total, ev[0], ev[5]);
-    for (auto &e : ev) cudaEventDestroy(e);
+    ds.ms_pack = tl.ms(0, 1);
+    ds.ms_hash = tl.ms(1, 2);
+    ds.ms_insert = tl.ms(2, 3);
+    ds.ms_verify = tl.ms(3, 4);
+    ds.ms_compact = tl.ms(4, 5);
+    ds.ms_total = tl.ms(0, 5);
     ds.n_unique = nu;
     c->pos_valid = false;
     c->stage1_done = c->stage2_done = false;

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <algorithm>
 #include <string>
 #include <vector>
 #include "../../include/itsx_b200.h"
@@ -191,8 +192,8 @@ struct itsx_ctx {
     DevBuf d_sh_order, d_sh_tmp, d_sh_bases, d_sh_rec;
 
     std::vector<cudaStream_t> lanes;      // side streams for the per-profile launches
-    std::vector<cudaEvent_t> lane_ev;
-    cudaEvent_t ev_a = nullptr, ev_b = nullptr;
+    std::vector<cudaEvent_t> lane_ev;     // ordering-only events: one per lane, and lane_fork on c->stream
+    cudaEvent_t lane_fork = nullptr;
 };
 
 enum { CNT_COLLIDE = 0, CNT_PAST_FWD, CNT_FWD_ROWS, CNT_BCK_ROWS, CNT_ENV_ROWS, CNT_DOM_OVERFLOW, CNT_MULTI,
@@ -206,6 +207,54 @@ enum { CNT_COLLIDE = 0, CNT_PAST_FWD, CNT_FWD_ROWS, CNT_BCK_ROWS, CNT_ENV_ROWS, 
             return ITSX_ECUDA;                                                                \
         }                                                                                     \
     } while (0)
+
+// CUB's two-call temp-storage protocol for one or more operations queued back to back on c->d_tmp.  Each f is a callable
+// (void *tmp, size_t &bytes) -> cudaError_t around one CUB call.  Every f is sized before d_tmp grows, once: growing it
+// between two of them would free storage that the first, already queued, still uses.  Returns the first failure.
+template <typename... F>
+cudaError_t cub_run(itsx_ctx *c, F &&...f)
+{
+    size_t bytes[sizeof...(F)] = {}, need = 0;
+    cudaError_t e = cudaSuccess;
+    int i = 0;
+    auto size = [&](auto &g) { if (e == cudaSuccess) { e = g(nullptr, bytes[i]); need = std::max(need, bytes[i]); } i++; };
+    (size(f), ...);
+    if (e == cudaSuccess) e = c->d_tmp.ensure(need);
+    i = 0;
+    auto run = [&](auto &g) { if (e == cudaSuccess) e = g(c->d_tmp.p, bytes[i]); i++; };
+    (run(f), ...);
+    return e;
+}
+
+// fan-out of c->stream to the side streams lanes[0 .. n) (ensure_lanes creates them), and fan-in back to c->stream
+inline cudaError_t fork_lanes(itsx_ctx *c, int n)
+{
+    cudaError_t e = cudaEventRecord(c->lane_fork, c->stream);
+    for (int l = 0; l < n && e == cudaSuccess; l++) e = cudaStreamWaitEvent(c->lanes[l], c->lane_fork, 0);
+    return e;
+}
+inline cudaError_t join_lanes(itsx_ctx *c, int n)
+{
+    cudaError_t e = cudaSuccess;
+    for (int l = 0; l < n && e == cudaSuccess; l++) {
+        e = cudaEventRecord(c->lane_ev[l], c->lanes[l]);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(c->stream, c->lane_ev[l], 0);
+    }
+    return e;
+}
+
+// N timing events, destroyed with the set; ms(i, j) is the time from event i to event j, 0 if either is not complete
+template <int N>
+struct Timeline {
+    cudaEvent_t ev[N] = {};
+    cudaError_t status = cudaSuccess;     // of the creation
+    Timeline() { for (auto &e : ev) if (status == cudaSuccess) status = cudaEventCreate(&e); }
+    ~Timeline() { for (auto e : ev) if (e) cudaEventDestroy(e); }
+    Timeline(const Timeline &) = delete;            // owns its events
+    Timeline &operator=(const Timeline &) = delete;
+    cudaError_t record(int i, cudaStream_t st) const { return cudaEventRecord(ev[i], st); }
+    float ms(int i, int j) const { float t = 0.f; cudaEventElapsedTime(&t, ev[i], ev[j]); return t; }
+};
 
 #ifdef __CUDACC__
 // byte mover of the trim / re-expansion and shard-exchange kernels: segment j = src[soff[j] .. + len) -> dst[doff[j] ..), one group of

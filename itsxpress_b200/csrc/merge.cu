@@ -377,7 +377,8 @@ int itsx_merge_pairs(itsx_ctx *c, const uint8_t *fseq, const uint8_t *fqual, con
     if (total) *total = 0;
     if (npairs == 0) return ITSX_OK;
     if (npairs > INT32_MAX - 1) { c->err = "merge: more than 2^31 pairs in one call"; return ITSX_ELIMIT; }
-    if (!c->ev_a) { CUDA_TRY(c, cudaEventCreate(&c->ev_a)); CUDA_TRY(c, cudaEventCreate(&c->ev_b)); }
+    Timeline<2> tl;     // merge_kernel alone
+    CUDA_TRY(c, tl.status);
 
     const int64_t ftot = itsx_peek_i64(foff + npairs), rtot = itsx_peek_i64(roff + npairs);
     CUDA_TRY(c, c->d_mg_foff.ensure((size_t)(npairs + 1) * 8));
@@ -408,11 +409,8 @@ int itsx_merge_pairs(itsx_ctx *c, const uint8_t *fseq, const uint8_t *fqual, con
         cub::TransformInputIterator<int, Diff, cub::CountingInputIterator<int64_t>> itF(cnt, Diff{c->d_mg_foff.as<int64_t>()}),
             itR(cnt, Diff{c->d_mg_roff.as<int64_t>()});
         int *d_max = (int *)c->d_mg_kscan.p;
-        size_t tb = 0;
-        cub::DeviceReduce::Max(nullptr, tb, itF, d_max, (int)npairs, st);
-        CUDA_TRY(c, c->d_tmp.ensure(tb + 256));
-        cub::DeviceReduce::Max(c->d_tmp.p, tb, itF, d_max, (int)npairs, st);
-        cub::DeviceReduce::Max(c->d_tmp.p, tb, itR, d_max + 1, (int)npairs, st);
+        CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceReduce::Max(t, b, itF, d_max, (int)npairs, st); },
+                            [&](void *t, size_t &b) { return cub::DeviceReduce::Max(t, b, itR, d_max + 1, (int)npairs, st); }));
         c->launches += 2;
         int h[2] = {0, 0};
         CUDA_TRY(c, cudaMemcpyAsync(h, d_max, 8, cudaMemcpyDeviceToHost, st));
@@ -467,19 +465,15 @@ int itsx_merge_pairs(itsx_ctx *c, const uint8_t *fseq, const uint8_t *fqual, con
     per_sm = std::max(per_sm, 1);
     const int64_t want = (npairs + MG_WARPS - 1) / MG_WARPS;
     const unsigned grid = (unsigned)std::min<int64_t>(want, (int64_t)c->sm_count * per_sm);   // persistent: whole waves of resident CTAs
-    CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
+    CUDA_TRY(c, tl.record(0, st));
     merge_kernel<<<grid, MG_WARPS * 32, smem, st>>>(a);
-    CUDA_TRY(c, cudaEventRecord(c->ev_b, st));
+    CUDA_TRY(c, tl.record(1, st));
     // compaction: merged pairs in input order, back to back
     int32_t *flag = c->d_mg_flag.as<int32_t>(), *ks = c->d_mg_kscan.as<int32_t>();
     int64_t *l64 = c->d_mg_len64.as<int64_t>(), *ls = c->d_mg_lscan.as<int64_t>();
     merge_flag_kernel<<<nblk(npairs + 1, 256), 256, 0, st>>>(a.merged_len, npairs, flag, l64);
-    size_t t1 = 0, t2 = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, t1, flag, ks, (int)npairs + 1, st);
-    cub::DeviceScan::ExclusiveSum(nullptr, t2, l64, ls, (int)npairs + 1, st);
-    CUDA_TRY(c, c->d_tmp.ensure(std::max(t1, t2)));
-    cub::DeviceScan::ExclusiveSum(c->d_tmp.p, t1, flag, ks, (int)npairs + 1, st);
-    cub::DeviceScan::ExclusiveSum(c->d_tmp.p, t2, l64, ls, (int)npairs + 1, st);
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, flag, ks, (int)npairs + 1, st); },
+                        [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, l64, ls, (int)npairs + 1, st); }));
     c->launches += 4;
     int32_t nk = 0;
     int64_t tot = 0;
@@ -502,14 +496,12 @@ int itsx_merge_pairs(itsx_ctx *c, const uint8_t *fseq, const uint8_t *fqual, con
     if (reason) CUDA_TRY(c, cudaMemcpyAsync(reason, a.reason, (size_t)npairs, cudaMemcpyDefault, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     CUDA_TRY(c, cudaGetLastError());
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, c->ev_a, c->ev_b);
     c->mg_nmerged = nk;
     c->mg_total = tot;
     c->mgstats.n_merged = nk;
     c->mgstats.bytes_in = 2 * (ftot + rtot);
     c->mgstats.bytes_out = 2 * tot;
-    c->mgstats.ms_kernel = ms;
+    c->mgstats.ms_kernel = tl.ms(0, 1);
     for (int r = 0; r < 16; r++) c->mgstats.by_reason[r] = (int64_t)hist[r];
     if (n_merged) *n_merged = nk;
     if (total) *total = tot;

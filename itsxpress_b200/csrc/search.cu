@@ -2318,14 +2318,12 @@ static int build_seqs(itsx_ctx *c, const uint8_t *d_ascii, const int64_t *d_off,
     int64_t *nw = c->d_scan.as<int64_t>();
     seqlen_kernel<<<nblk(nseq, 256), 256, 0, st>>>(d_off, d_first, nseq, c->d_seqlen.as<int32_t>(), nw);
     CUDA_TRY(c, cudaMemsetAsync(nw + nseq, 0, 8, st));
-    size_t tmpb = 0, tmpb2 = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, tmpb, nw, c->d_seqwoff.as<int64_t>(), (int)nseq + 1, st);
     CUDA_TRY(c, c->d_counters.ensure(64 * 8));
     int32_t *d_max = (int32_t *)(c->d_counters.as<unsigned long long>() + 40);
-    cub::DeviceReduce::Max(nullptr, tmpb2, c->d_seqlen.as<int32_t>(), d_max, (int)nseq, st);
-    CUDA_TRY(c, c->d_tmp.ensure(std::max(tmpb, tmpb2)));
-    cub::DeviceScan::ExclusiveSum(c->d_tmp.p, tmpb, nw, c->d_seqwoff.as<int64_t>(), (int)nseq + 1, st);
-    cub::DeviceReduce::Max(c->d_tmp.p, tmpb2, c->d_seqlen.as<int32_t>(), d_max, (int)nseq, st);
+    int64_t *woff = c->d_seqwoff.as<int64_t>();
+    int32_t *len = c->d_seqlen.as<int32_t>();
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, nw, woff, (int)nseq + 1, st); },
+                        [&](void *t, size_t &b) { return cub::DeviceReduce::Max(t, b, len, d_max, (int)nseq, st); }));
     int64_t totw = 0;
     int32_t lmax = 0;
     CUDA_TRY(c, cudaMemcpyAsync(&totw, c->d_seqwoff.as<int64_t>() + nseq, 8, cudaMemcpyDeviceToHost, st));
@@ -2395,6 +2393,8 @@ int search_build_seqs_from_host(itsx_ctx *c, const uint8_t *seq, const int64_t *
     return build_seqs(c, t_ascii.as<uint8_t>(), t_off.as<int64_t>(), nullptr, nseq);
 }
 
+constexpr int NLANE = 8;                   // side streams of the per-profile launches
+
 static int ensure_lanes(itsx_ctx *c, int n)
 {
     while ((int)c->lanes.size() < n) {
@@ -2405,10 +2405,502 @@ static int ensure_lanes(itsx_ctx *c, int n)
         c->lanes.push_back(s);
         c->lane_ev.push_back(e);
     }
-    if (!c->ev_a) {
-        CUDA_TRY(c, cudaEventCreateWithFlags(&c->ev_a, cudaEventDisableTiming));
-        CUDA_TRY(c, cudaEventCreateWithFlags(&c->ev_b, cudaEventDisableTiming));
+    if (!c->lane_fork) CUDA_TRY(c, cudaEventCreateWithFlags(&c->lane_fork, cudaEventDisableTiming));
+    return ITSX_OK;
+}
+
+// the shard of the sequence set that a search covers: sequences q0 .. q0 + qn (itsx_search_shard)
+static int shard_range(itsx_ctx *c, int64_t &q0, int64_t &qn)
+{
+    q0 = c->shard_first;
+    qn = c->shard_n < 0 ? c->nseq - q0 : c->shard_n;
+    if (q0 < 0 || qn < 0 || q0 + qn > c->nseq) { c->err = "search: shard outside the sequence set"; return ITSX_EINVAL; }
+    return ITSX_OK;
+}
+
+// position table, arg-max keys and the winners' multidomain flags of the shard's qn sequences; init: reset them to "no hit"
+static int pos_reset(itsx_ctx *c, int64_t qn, bool init)
+{
+    const size_t n = (size_t)std::max<int64_t>(qn, 1);
+    c->npos = qn;
+    CUDA_TRY(c, c->d_pos.ensure(n * 9 * 4));
+    CUDA_TRY(c, c->d_best.ensure(n * 2 * 8));
+    CUDA_TRY(c, c->d_selmulti.ensure(n * 2 + 16));
+    if (init && qn > 0) {
+        pos_init_kernel<<<nblk(qn, 256), 256, 0, c->stream>>>(c->d_pos.as<int32_t>(), c->d_best.as<unsigned long long>(),
+                                                              c->d_selmulti.as<uint8_t>(), qn);
+        c->launches++;
     }
+    return ITSX_OK;
+}
+
+// ---- stage 1: the filter cascade, chunk by chunk over the shard's sequences ------------------------------------------
+// Events of the stage clocks.  A stage's span runs from the event that ends the stage before it to its own last event;
+// the Forward stage's clock starts at S1_FILT, recorded by the bias stage or, when it runs, after the Viterbi stage.
+enum { S1_CALL0, S1_MSV0, S1_MSV1, S1_FILT, S1_VIT0, S1_VIT1, S1_FB, S1_MD, S1_ENV, S1_SCORE, S1_CALL1, S1_NEV };
+
+struct S1Call {                           // what every chunk of one search_stage1 shares
+    int64_t q0 = 0, qn = 0;               // the shard
+    int P = 0;
+    int32_t *d_order = nullptr;           // the shard's sequences sorted by length
+    unsigned long long *cnt = nullptr;    // device counters (CNT_*)
+    int32_t *d_nsel = nullptr;            // survivor counts of the compactions (in d_counters)
+    bool multi_sample = false;
+    double lnP_certain = 0;
+    Timeline<S1_NEV> tl;                  // the stages add their spans to c->sstats.ms_*
+};
+
+struct S1Chunk {                          // d_order[s0 .. s0 + ns) and its survivors
+    int64_t s0 = 0;
+    int ns = 0;
+    int32_t n1 = 0, n2 = 0, nenv = 0;     // pairs past MSV, past bias (and Viterbi); envelopes
+    std::vector<int32_t> h_bounds;        // [P + 1] per-profile slices of list2
+};
+
+// residues of the shard (cell accounting), and d_order: the shard's sequences in order of length, so that the 32 pairs
+// of a warp run the same number of rows
+static int s1_order(itsx_ctx *c, S1Call &s)
+{
+    cudaStream_t st = c->stream;
+    const int64_t q0 = s.q0, qn = s.qn;
+    int32_t *len = c->d_seqlen.as<int32_t>() + q0;
+    long long *d_sum = (long long *)(s.cnt + 41);
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceReduce::Sum(t, b, len, d_sum, (int)qn, st); }));
+    long long h = 0;
+    CUDA_TRY(c, cudaMemcpyAsync(&h, d_sum, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    double sumM = 0;
+    for (auto &hp : c->prof) sumM += hp.M;
+    c->sstats.msv_cells = (double)h * sumM;
+    CUDA_TRY(c, c->d_order.ensure((size_t)qn * 4 * 4));
+    int32_t *d_order = s.d_order = c->d_order.as<int32_t>();
+    int32_t *idx_in = d_order + qn, *len_in = d_order + 2 * qn, *len_out = d_order + 3 * qn;
+    iota_kernel<<<nblk(qn, 256), 256, 0, st>>>(idx_in, (int32_t)q0, qn);
+    CUDA_TRY(c, cudaMemcpyAsync(len_in, len, (size_t)qn * 4, cudaMemcpyDeviceToDevice, st));
+    int lbits = 1;
+    while ((1 << lbits) <= c->Lmax) lbits++;
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
+        return cub::DeviceRadixSort::SortPairs(t, b, len_in, len_out, idx_in, d_order, (int)qn, 0, lbits, st);
+    }));
+    c->launches += 2;
+    return ITSX_OK;
+}
+
+// MSV over the chunk's pairs, then the list of the pairs that pass it (n1; its compaction is on the bias stage's clock)
+static int s1_msv(itsx_ctx *c, const S1Call &s, S1Chunk &k)
+{
+    cudaStream_t st = c->stream;
+    const size_t npair = (size_t)k.ns * s.P;
+    const size_t msv_smem = (size_t)MSV_TP * MSV_TABW * 4;
+    CUDA_TRY(c, cudaFuncSetAttribute(msv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msv_smem));
+    CUDA_TRY(c, s.tl.record(S1_MSV0, st));
+    CUDA_TRY(c, c->d_msvres.ensure(npair));
+    CUDA_TRY(c, c->d_flag.ensure(npair + 16));
+    dim3 grid(nblk(k.ns, MSV_THREADS), (s.P + MSV_TP - 1) / MSV_TP);
+    msv_kernel<<<grid, MSV_THREADS, msv_smem, st>>>(c->d_seqw.as<uint32_t>(), c->d_seqwoff.as<int64_t>(),
+                                                    c->d_seqlen.as<int32_t>(), s.d_order, k.s0, k.ns, c->d_msvtab.as<uint32_t>(),
+                                                    c->d_pscal.as<ProfScalars>(), s.P, c->d_tjb.as<uint8_t>(),
+                                                    c->d_nullsc.as<float>(), c->prm.F1,
+                                                    c->d_msvres.as<uint8_t>(), c->d_flag.as<uint8_t>());
+    c->launches++;
+    CUDA_TRY(c, s.tl.record(S1_MSV1, st));
+    CUDA_TRY(c, c->d_list.ensure(npair * 4 + 16));
+    cub::CountingInputIterator<int32_t> iota(0);
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
+        return cub::DeviceSelect::Flagged(t, b, iota, c->d_flag.as<uint8_t>(), c->d_list.as<int32_t>(), s.d_nsel, (int)npair, st);
+    }));
+    CUDA_TRY(c, cudaMemcpyAsync(&k.n1, s.d_nsel, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    c->sstats.n_past_msv += k.n1;
+    c->sstats.ms_msv += s.tl.ms(S1_MSV0, S1_MSV1);
+    return ITSX_OK;
+}
+
+// entries of (list, sc) whose flag is set, in order, to (list_out, sc_out); *d_n receives their number
+static cudaError_t compact_list_sc(itsx_ctx *c, int32_t *list, float *sc, uint8_t *flag, int32_t *list_out, float *sc_out,
+                                   int32_t *d_n, int n)
+{
+    cudaStream_t st = c->stream;
+    return cub_run(c, [&](void *t, size_t &b) { return cub::DeviceSelect::Flagged(t, b, list, flag, list_out, d_n, n, st); },
+                   [&](void *t, size_t &b) { return cub::DeviceSelect::Flagged(t, b, sc, flag, sc_out, d_n, n, st); });
+}
+
+// bias filter over the n1 MSV survivors: list2 / fsc2 hold the n2 that pass, h_bounds their per-profile slices
+static int s1_bias(itsx_ctx *c, const S1Call &s, S1Chunk &k)
+{
+    cudaStream_t st = c->stream;
+    const int P = s.P, n1 = k.n1;
+    CUDA_TRY(c, c->d_filtersc.ensure((size_t)n1 * 4));
+    CUDA_TRY(c, c->d_ndom.ensure((size_t)n1 + 16));   // reused as flag2 here
+    bias_kernel<<<nblk(n1, 128), 128, 0, st>>>(c->d_list.as<int32_t>(), s.d_nsel, s.d_order, k.s0, k.ns, c->d_seqw.as<uint32_t>(),
+                                               c->d_seqwoff.as<int64_t>(), c->d_seqlen.as<int32_t>(),
+                                               c->d_pscal.as<ProfScalars>(), c->d_msvres.as<uint8_t>(),
+                                               c->d_tjb.as<uint8_t>(), c->prm.F1, c->prm.F2, c->d_filtersc.as<float>(),
+                                               c->d_ndom.as<uint8_t>(), s.cnt);
+    CUDA_TRY(c, c->d_list2.ensure((size_t)n1 * 4 + 16));
+    CUDA_TRY(c, c->d_fsc2.ensure((size_t)n1 * 4 + 16));
+    int32_t *d_nsel2 = s.d_nsel + 1;
+    CUDA_TRY(c, compact_list_sc(c, c->d_list.as<int32_t>(), c->d_filtersc.as<float>(), c->d_ndom.as<uint8_t>(),
+                                c->d_list2.as<int32_t>(), c->d_fsc2.as<float>(), d_nsel2, n1));
+    CUDA_TRY(c, c->d_bounds.ensure((size_t)(P + 1) * 8));
+    bounds_kernel<<<nblk(P + 1, 128), 128, 0, st>>>(c->d_list2.as<int32_t>(), d_nsel2, k.ns, P, c->d_bounds.as<int32_t>());
+    c->launches += 2;
+    k.h_bounds.resize((size_t)P + 1);
+    CUDA_TRY(c, cudaMemcpyAsync(&k.n2, d_nsel2, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaMemcpyAsync(k.h_bounds.data(), c->d_bounds.p, (size_t)(P + 1) * 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, s.tl.record(S1_FILT, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    c->sstats.n_past_bias += k.n2;
+    c->sstats.ms_bias += s.tl.ms(S1_MSV1, S1_FILT);
+    return ITSX_OK;
+}
+
+// Viterbi filter for the entries with F2 < P(MSV + bias) <= F1 (never under the reference's F1 == F2): list2 / fsc2 and
+// h_bounds keep the n2 entries that pass it
+static int s1_viterbi(itsx_ctx *c, const S1Call &s, S1Chunk &k)
+{
+    cudaStream_t st = c->stream;
+    const int P = s.P, n1 = k.n1, n2 = k.n2;
+    CUDA_TRY(c, s.tl.record(S1_VIT0, st));
+    // the "needs the filter" marks of the surviving entries, compacted like the list itself
+    CUDA_TRY(c, c->d_vneed.ensure((size_t)n1 + 16));
+    CUDA_TRY(c, c->d_vpass.ensure((size_t)n2 + 16));
+    int32_t *d_nsel3 = s.d_nsel + 2;
+    uint8_t *d_run = c->d_ndom.as<uint8_t>();      // the bias flags; once consumed, the "run" marks
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
+        return cub::DeviceSelect::Flagged(t, b, d_run, d_run, c->d_vneed.as<uint8_t>(), d_nsel3, n1, st);
+    }));
+    // worklist of the entries the filter has to look at (full warps), its per-profile slices
+    CUDA_TRY(c, c->d_list.ensure((size_t)n2 * 4 * 2 + 64));
+    vneed_flag_kernel<<<nblk(n2, 256), 256, 0, st>>>(c->d_vneed.as<uint8_t>(), n2, d_run, c->d_vpass.as<uint8_t>());
+    int32_t *d_vidx = c->d_list.as<int32_t>() + n2;         // second half of d_list (first half: compaction output below)
+    int32_t *d_nv = s.d_nsel + 3;
+    cub::CountingInputIterator<int32_t> iota0(0);
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceSelect::Flagged(t, b, iota0, d_run, d_vidx, d_nv, n2, st); }));
+    vbounds_kernel<<<nblk(P + 1, 128), 128, 0, st>>>(c->d_list2.as<int32_t>(), d_vidx, d_nv, k.ns, P,
+                                                     c->d_bounds.as<int32_t>() + (P + 1));
+    std::vector<int32_t> h_vb((size_t)P + 1);
+    CUDA_TRY(c, cudaMemcpyAsync(h_vb.data(), c->d_bounds.as<int32_t>() + (P + 1), (size_t)(P + 1) * 4,
+                                cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    c->launches += 3;
+    CUDA_TRY(c, fork_lanes(c, NLANE));
+    int vrr = 0;
+    for (int p = 0; p < P; p++) {
+        const int b0 = h_vb[p], cntp = h_vb[p + 1] - b0;
+        if (cntp <= 0) continue;
+        VitArgs va;
+        va.list = c->d_list2.as<int32_t>(); va.filtersc = c->d_fsc2.as<float>();
+        va.vidx = d_vidx + b0; va.count = cntp;
+        va.order = s.d_order; va.s0 = k.s0; va.ns = k.ns; va.prof = p;
+        va.seqw = c->d_seqw.as<uint32_t>(); va.woff = c->d_seqwoff.as<int64_t>(); va.seqlen = c->d_seqlen.as<int32_t>();
+        va.vtab = c->d_vtab.as<int32_t>() + (size_t)p * VIT_WORDS;
+        va.xwmove = c->d_xwmove.as<int16_t>();
+        va.xw_E = (int)roundf(500.0f / (float)kLn2 * (-(float)kLn2));
+        va.vmu = c->prof[p].ev[EV_VMU]; va.vlambda = c->prof[p].ev[EV_VLAMBDA];
+        va.F2 = c->prm.F2;
+        va.pass = c->d_vpass.as<uint8_t>();
+        va.counters = s.cnt;
+        vit_kernel<<<nblk(cntp, 128), 128, 0, c->lanes[vrr++ % NLANE]>>>(va);
+        c->launches++;
+    }
+    CUDA_TRY(c, join_lanes(c, NLANE));
+    // survivors: list2 / fsc2 compacted by the pass flags (through the bias stage's buffers, then back)
+    CUDA_TRY(c, compact_list_sc(c, c->d_list2.as<int32_t>(), c->d_fsc2.as<float>(), c->d_vpass.as<uint8_t>(),
+                                c->d_list.as<int32_t>(), c->d_filtersc.as<float>(), d_nsel3, n2));
+    int32_t n3 = 0;
+    CUDA_TRY(c, cudaMemcpyAsync(&n3, d_nsel3, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    if (n3 > 0) {
+        CUDA_TRY(c, cudaMemcpyAsync(c->d_list2.p, c->d_list.p, (size_t)n3 * 4, cudaMemcpyDeviceToDevice, st));
+        CUDA_TRY(c, cudaMemcpyAsync(c->d_fsc2.p, c->d_filtersc.p, (size_t)n3 * 4, cudaMemcpyDeviceToDevice, st));
+    }
+    bounds_kernel<<<nblk(P + 1, 128), 128, 0, st>>>(c->d_list2.as<int32_t>(), d_nsel3, k.ns, P, c->d_bounds.as<int32_t>());
+    c->launches += 3;
+    CUDA_TRY(c, cudaMemcpyAsync(k.h_bounds.data(), c->d_bounds.p, (size_t)(P + 1) * 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, s.tl.record(S1_VIT1, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    c->sstats.ms_vit += s.tl.ms(S1_VIT0, S1_VIT1);
+    k.n2 = n3;
+    CUDA_TRY(c, s.tl.record(S1_FILT, st));
+    return ITSX_OK;
+}
+
+// Forward / Backward / posterior decoding of the n2 entries: one launch per profile (in pieces) over the side streams
+static int s1_fwdbck(itsx_ctx *c, const S1Call &s, const S1Chunk &k)
+{
+    const int n2 = k.n2, Lmax = c->Lmax;
+    CUDA_TRY(c, c->d_fwdsc.ensure((size_t)n2 * 4));
+    CUDA_TRY(c, c->d_pairout.ensure((size_t)n2 * 4));
+    CUDA_TRY(c, c->d_ndom.ensure((size_t)n2 + 16));
+    CUDA_TRY(c, c->d_env.ensure((size_t)n2 * ITSX_MAXDOM * 2 * 4));
+    const size_t slab = (size_t)(Lmax + 1) * SPEC_C * 32 * 4;
+    // the slab of a launch holds all its tiles (fbdec_kernel reads them back): a profile's worklist goes in pieces of
+    // at most two tiles per resident warp, and no more than fit the scratch budget
+    const int fb_warps_per_lane = c->sm_count * FB_CTAS_PER_SM * (FB_THREADS / 32);
+    const int fb_piece_tiles = (int)std::max<size_t>(
+        1, std::min<size_t>((size_t)fb_warps_per_lane * 2, FB_SCRATCH_BUDGET / (slab * NLANE)));
+    CUDA_TRY(c, c->d_spec.ensure(slab * (size_t)fb_piece_tiles * NLANE));
+    CUDA_TRY(c, c->d_fbscale.ensure((size_t)n2 * 4));
+    CUDA_TRY(c, fork_lanes(c, NLANE));
+    int lane_rr = 0;
+    for (int p = 0; p < s.P; p++) {
+        const int b0 = k.h_bounds[p], cntp = k.h_bounds[p + 1] - b0;
+        if (cntp <= 0) continue;
+        const int l = lane_rr++ % NLANE;
+        FbArgs fa;
+        fa.order = s.d_order; fa.s0 = k.s0; fa.ns = k.ns; fa.prof = p;
+        fa.seqw = c->d_seqw.as<uint32_t>(); fa.woff = c->d_seqwoff.as<int64_t>(); fa.seqlen = c->d_seqlen.as<int32_t>();
+        fa.etab = c->d_etab.as<float>() + (size_t)p * (MAXM + 1) * 16;
+        fa.Lmax = Lmax;
+        fa.tau = c->prof[p].ev[EV_FTAU]; fa.lambda = c->prof[p].ev[EV_FLAMBDA];
+        fa.F3 = c->prm.F3;
+        fa.e_move = expf(-(float)kLn2);
+        fa.counters = s.cnt;
+        const int wpc = FB_THREADS / 32;
+        fa.spec = (float *)(c->d_spec.as<char>() + slab * (size_t)fb_piece_tiles * l);
+        for (int e0 = 0; e0 < cntp; e0 += fb_piece_tiles * 32) {
+            FbArgs fp = fa;
+            const int o = b0 + e0;          // the piece: entries o .. o + count of list2
+            fp.count = std::min(cntp - e0, fb_piece_tiles * 32);
+            fp.list = c->d_list2.as<int32_t>() + o; fp.filtersc = c->d_fsc2.as<float>() + o;
+            fp.fwdsc = c->d_fwdsc.as<float>() + o; fp.bcksc = c->d_pairout.as<float>() + o;
+            fp.ndom = c->d_ndom.as<uint8_t>() + o; fp.env = c->d_env.as<int32_t>() + (size_t)o * ITSX_MAXDOM * 2;
+            fp.scale = c->d_fbscale.as<float>() + o;
+            const int tiles = (fp.count + 31) / 32;
+            const int ctas = std::min((tiles + wpc - 1) / wpc, c->sm_count * FB_CTAS_PER_SM);
+            fb_kernel<<<ctas, FB_THREADS, 0, c->lanes[l]>>>(c->pconst[p], fp);
+            fbdec_kernel<<<(tiles + 3) / 4, 128, 0, c->lanes[l]>>>(fp);
+            c->launches += 2;
+        }
+    }
+    CUDA_TRY(c, join_lanes(c, NLANE));
+    CUDA_TRY(c, s.tl.record(S1_FB, c->stream));
+    return ITSX_OK;
+}
+
+// multidomain regions: stochastic-traceback clustering replaces the region by its cluster envelopes
+static int s1_multidomain(itsx_ctx *c, const S1Call &s, const S1Chunk &k)
+{
+    cudaStream_t st = c->stream;
+    const int n2 = k.n2;
+    CUDA_TRY(c, c->d_envdc.ensure((size_t)n2 * ITSX_MAXDOM * 4));
+    CUDA_TRY(c, c->d_n2reg.ensure((size_t)n2 * 4));
+    CUDA_TRY(c, cudaMemsetAsync(c->d_n2reg.p, 0, (size_t)n2 * 4, st));
+    // flagged regions per entry -> prefix sum -> region list in entry order
+    int32_t h_nregions = 0, *d_base = nullptr;
+    if (c->prm.resolve_multidomain) {
+        CUDA_TRY(c, c->d_mdlist.ensure((size_t)(n2 + 1) * 2 * 4));
+        int32_t *d_nreg = c->d_mdlist.as<int32_t>();
+        d_base = d_nreg + (n2 + 1);
+        mdcount_kernel<<<nblk(n2 + 1, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), c->d_env.as<int32_t>(), n2, d_nreg);
+        CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, d_nreg, d_base, n2 + 1, st); }));
+        c->launches += 2;
+        CUDA_TRY(c, cudaMemcpyAsync(&h_nregions, d_base + n2, 4, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(c, cudaStreamSynchronize(st));
+    }
+    if (h_nregions > 0) {
+        const int NR = h_nregions;
+        CUDA_TRY(c, c->d_mdreg.ensure(((size_t)NR * 3 + (size_t)(NR + 1) * 2) * 4));
+        int32_t *reg_ent = c->d_mdreg.as<int32_t>(), *reg_i = reg_ent + NR, *reg_j = reg_i + NR,
+                *reg_rows = reg_j + NR, *reg_row = reg_rows + (NR + 1);
+        CUDA_TRY(c, cudaMemsetAsync(reg_rows + NR, 0, 4, st));
+        mdregs_kernel<<<nblk(n2, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), c->d_env.as<int32_t>(), n2, d_base,
+                                                    reg_ent, reg_i, reg_j, reg_rows);
+        CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, reg_rows, reg_row, NR + 1, st); }));
+        c->launches += 2;
+        std::vector<int32_t> h_row((size_t)NR + 1);
+        CUDA_TRY(c, cudaMemcpyAsync(h_row.data(), reg_row, (size_t)(NR + 1) * 4, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(c, cudaStreamSynchronize(st));
+        CUDA_TRY(c, c->d_mdres.ensure((size_t)NR * sizeof(MdRes)));
+        MdStreams streams;
+        const uint32_t x0 = md_rng_state0(42u);
+        for (int t = 0; t < MD_NSAMPLES; t++) streams.x[t] = md_rng_jump(x0, (uint64_t)t << MD_STREAM_LOG2);
+        MdArgs ma;
+        ma.reg_ent = reg_ent; ma.reg_i = reg_i; ma.reg_j = reg_j; ma.reg_row = reg_row;
+        ma.list = c->d_list2.as<int32_t>(); ma.order = s.d_order; ma.s0 = k.s0; ma.ns = k.ns;
+        ma.seqw = c->d_seqw.as<uint32_t>(); ma.woff = c->d_seqwoff.as<int64_t>(); ma.seqlen = c->d_seqlen.as<int32_t>();
+        ma.mdtab = c->d_mdtab.as<float>(); ma.etab = c->d_etab.as<float>(); ma.pscal = c->d_pscal.as<ProfScalars>();
+        ma.res = c->d_mdres.as<MdRes>();
+        ma.e_move = expf(-(float)kLn2);
+        ma.counters = s.cnt;
+        // chunks of regions: slabs (matrix + row tables) and trace records within a fixed HBM budget; consecutive
+        // chunks alternate between two side streams with their own buffers, so that the latency-bound Forward fill of
+        // one chunk runs under the issue-bound tracebacks / clustering of the other
+        const size_t row_bytes = (size_t)MD_W * 16 + sizeof(MdRow), reg_bytes = (size_t)MD_TRACE_BYTES;
+        const size_t budget = (size_t)3 << 30;
+        struct MdChunk { int r0, r1, maxrows, ctas; size_t rows; };
+        std::vector<MdChunk> chunks;
+        const size_t cl_smem = sizeof(MdClustSmem) * MDC_WARPS;
+        CUDA_TRY(c, cudaFuncSetAttribute(mdclust_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cl_smem));
+        int cl_per_sm = 0;      // resident CTAs per SM at this shared-memory size: the grid is ONE wave
+        CUDA_TRY(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cl_per_sm, mdclust_kernel, MDC_WARPS * 32, cl_smem));
+        size_t need_cell[2] = {0, 0}, need_trace[2] = {0, 0}, need_scr[2] = {0, 0};
+        for (int r0 = 0; r0 < NR;) {
+            int r1 = r0 + 1;
+            while (r1 < NR && (size_t)(h_row[r1 + 1] - h_row[r0]) * row_bytes + (size_t)(r1 + 1 - r0) * reg_bytes <= budget)
+                r1++;
+            MdChunk ch;
+            ch.r0 = r0; ch.r1 = r1; ch.rows = (size_t)(h_row[r1] - h_row[r0]); ch.maxrows = 0;
+            for (int r = r0; r < r1; r++) ch.maxrows = std::max(ch.maxrows, h_row[r + 1] - h_row[r]);
+            ch.ctas = std::min((r1 - r0 + MDC_WARPS - 1) / MDC_WARPS, c->sm_count * std::max(cl_per_sm, 1));
+            const int par = (int)(chunks.size() & 1);
+            need_cell[par] = std::max(need_cell[par], ch.rows * row_bytes);
+            need_trace[par] = std::max(need_trace[par], (size_t)(r1 - r0) * reg_bytes);
+            need_scr[par] = std::max(need_scr[par], md_clust_bytes(ch.maxrows) * (size_t)ch.ctas * MDC_WARPS);
+            chunks.push_back(ch);
+            r0 = r1;
+        }
+        for (int par = 0; par < 2; par++) {
+            CUDA_TRY(c, c->d_mdcell[par].ensure(need_cell[par]));
+            CUDA_TRY(c, c->d_mdtrace[par].ensure(need_trace[par]));
+            CUDA_TRY(c, c->d_mdscratch[par].ensure(need_scr[par]));
+        }
+        CUDA_TRY(c, fork_lanes(c, 2));
+        for (size_t ci = 0; ci < chunks.size(); ci++) {
+            const MdChunk &ch = chunks[ci];
+            const int par = (int)(ci & 1);
+            cudaStream_t ms = c->lanes[par];
+            ma.r0 = ch.r0; ma.r1 = ch.r1; ma.row0 = h_row[ch.r0];
+            ma.cell = c->d_mdcell[par].as<float4>();
+            ma.rowrec = (MdRow *)(c->d_mdcell[par].as<char>() + ch.rows * MD_W * 16);
+            ma.trace = c->d_mdtrace[par].as<char>();
+            ma.maxrows = ch.maxrows;
+            ma.per_thread = md_clust_bytes(ch.maxrows);
+            ma.scratch = c->d_mdscratch[par].as<char>();
+            mdfwd_kernel<<<nblk(ch.r1 - ch.r0, 64), 64, 0, ms>>>(ma);
+            mdtrace_kernel<<<nblk((int64_t)(ch.r1 - ch.r0) * MD_NSAMPLES, 128), 128, 0, ms>>>(ma, streams);
+            mdclust_kernel<<<ch.ctas, MDC_WARPS * 32, cl_smem, ms>>>(ma);
+            c->launches += 3;
+        }
+        CUDA_TRY(c, join_lanes(c, 2));
+        mdapply_kernel<<<nblk(n2, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), c->d_env.as<int32_t>(), n2, d_base,
+                                                     c->d_mdres.as<MdRes>(), c->d_envdc.as<float>(),
+                                                     c->d_n2reg.as<float>(), s.cnt);
+        c->launches++;
+    }
+    CUDA_TRY(c, s.tl.record(S1_MD, st));
+    return ITSX_OK;
+}
+
+// envelope worklist (sorted by profile and envelope length) and unihit rescoring of every envelope (nenv)
+static int s1_envelopes(itsx_ctx *c, const S1Call &s, S1Chunk &k)
+{
+    cudaStream_t st = c->stream;
+    const int P = s.P, n2 = k.n2;
+    CUDA_TRY(c, c->d_scan.ensure((size_t)(n2 + 1) * 4));
+    CUDA_TRY(c, c->d_envoff.ensure((size_t)(n2 + 1) * 4));
+    ndom_widen_kernel<<<nblk(n2 + 1, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), n2, c->d_scan.as<int32_t>());
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
+        return cub::DeviceScan::ExclusiveSum(t, b, c->d_scan.as<int32_t>(), c->d_envoff.as<int32_t>(), n2 + 1, st);
+    }));
+    gather_bounds_kernel<<<nblk(P + 1, 128), 128, 0, st>>>(c->d_envoff.as<int32_t>(), c->d_bounds.as<int32_t>(), P,
+                                                           c->d_bounds.as<int32_t>() + (P + 1));
+    c->launches += 2;
+    std::vector<int32_t> h_envb((size_t)P + 1);
+    CUDA_TRY(c, cudaMemcpyAsync(h_envb.data(), c->d_bounds.as<int32_t>() + (P + 1), (size_t)(P + 1) * 4,
+                                cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    const int nenv = k.nenv = h_envb[P];
+    if (nenv > 0) {
+        CUDA_TRY(c, c->d_envout.ensure((size_t)nenv * 20 * 4));
+        // worklist sorted by (profile, envelope length): two ping-pong buffers for the radix sort
+        CUDA_TRY(c, c->d_envwork.ensure((size_t)nenv * 4 * 4));
+        int32_t *wk_in = c->d_envwork.as<int32_t>(), *wk_out = wk_in + nenv;
+        uint32_t *key_in = (uint32_t *)(wk_in + 2 * (size_t)nenv), *key_out = key_in + nenv;
+        envwork_kernel<<<nblk(n2, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), c->d_envoff.as<int32_t>(), n2,
+                                                      c->d_list2.as<int32_t>(), k.ns, c->d_env.as<int32_t>(), wk_in,
+                                                      key_in);
+        int pbits = 1;
+        while ((1 << pbits) < P) pbits++;
+        CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
+            return cub::DeviceRadixSort::SortPairs(t, b, key_in, key_out, wk_in, wk_out, nenv, 0, 12 + pbits, st);
+        }));
+        c->launches += 2;
+        // envelopes are at most Lmax long; scratch per warp of the grid, whose size the budget bounds
+        const size_t eslab = (size_t)(c->Lmax + 1) * ENV_ROWF * 32 * 4;
+        const int env_wpc = ENV_THREADS / 32;
+        const int env_warps = (int)std::max<size_t>(
+            env_wpc, std::min<size_t>(c->sm_count * ENV_CTAS_PER_SM * env_wpc,
+                                      ENV_SCRATCH_BUDGET / (eslab * NLANE) / env_wpc * env_wpc));
+        const size_t env_smem = (size_t)(ENV_THREADS / 32) * ENV_RING * (ENV_ROWBYTES + 8);
+        CUDA_TRY(c, cudaFuncSetAttribute(env_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env_smem));
+        CUDA_TRY(c, c->d_envscratch.ensure(eslab * env_warps * NLANE));
+        CUDA_TRY(c, fork_lanes(c, NLANE));
+        int lane_rr = 0;
+        for (int p = 0; p < P; p++) {
+            const int e0 = h_envb[p], cnte = h_envb[p + 1] - e0;
+            if (cnte <= 0) continue;
+            const int l = lane_rr++ % NLANE;
+            EnvArgs ea;
+            ea.work = wk_out + e0;
+            ea.envoff = c->d_envoff.as<int32_t>();
+            ea.count = cnte;
+            ea.list = c->d_list2.as<int32_t>();
+            ea.env = c->d_env.as<int32_t>();
+            ea.order = s.d_order; ea.s0 = k.s0; ea.ns = k.ns; ea.prof = p;
+            ea.seqw = c->d_seqw.as<uint32_t>(); ea.woff = c->d_seqwoff.as<int64_t>(); ea.seqlen = c->d_seqlen.as<int32_t>();
+            ea.etab = c->d_etab.as<float>() + (size_t)p * (MAXM + 1) * 16;
+            ea.scratch = (float *)(c->d_envscratch.as<char>() + eslab * env_warps * l);
+            ea.Ldmax = c->Lmax;
+            ea.out = c->d_envout.as<float>();
+            ea.out_base = e0;
+            ea.counters = s.cnt;
+            const int tiles = (cnte + 31) / 32;
+            const int ctas = std::min((tiles + env_wpc - 1) / env_wpc, env_warps / env_wpc);
+            env_kernel<<<ctas, ENV_THREADS, env_smem, c->lanes[l]>>>(c->pconst[p], ea);
+            c->launches++;
+        }
+        CUDA_TRY(c, join_lanes(c, NLANE));
+    }
+    CUDA_TRY(c, s.tl.record(S1_ENV, st));
+    return ITSX_OK;
+}
+
+// sequence and domain scores of the chunk's envelopes; in compact mode (keep_rows 2) the per-sequence selection too.
+// The chunk's work ends here: the Forward, resolver, envelope and score spans are read after its synchronisation.
+static int s1_scores(itsx_ctx *c, const S1Call &s, const S1Chunk &k)
+{
+    cudaStream_t st = c->stream;
+    itsx_search_stats &ss = c->sstats;
+    if (k.nenv > 0) {
+        CUDA_TRY(c, c->d_doms.ensure((size_t)(c->ndom + k.nenv) * sizeof(DomRec), true, st));
+        FinalArgs fa;
+        fa.list = c->d_list2.as<int32_t>(); fa.n = k.n2; fa.order = s.d_order; fa.s0 = k.s0; fa.ns = k.ns;
+        fa.seqw = c->d_seqw.as<uint32_t>(); fa.woff = c->d_seqwoff.as<int64_t>(); fa.seqlen = c->d_seqlen.as<int32_t>();
+        fa.pscal = c->d_pscal.as<ProfScalars>(); fa.nullsctab = c->d_nullsc.as<float>();
+        fa.logsum = c->d_logsum.as<float>(); fa.fwdsc = c->d_fwdsc.as<float>();
+        fa.ndom = c->d_ndom.as<uint8_t>(); fa.envoff = c->d_envoff.as<int32_t>(); fa.env = c->d_env.as<int32_t>();
+        fa.envdc = c->d_envdc.as<float>(); fa.n2reg = c->d_n2reg.as<float>();
+        fa.envout = c->d_envout.as<float>(); fa.T = c->prm.T;
+        fa.doms = c->d_doms.as<DomRec>() + (c->compact ? 0 : c->ndom);
+        fa.nrep = c->d_nrep.as<int32_t>(); fa.counters = s.cnt;
+        fa.seq_sample = s.multi_sample ? c->d_seq_sample.as<int32_t>() : nullptr; fa.P = s.P;
+        fa.compact = c->compact ? 1 : 0;
+        fa.best = c->d_best.as<unsigned long long>(); fa.nseq = s.qn; fa.seq_first = s.q0;
+        fa.lnP_certain = s.lnP_certain;
+        final_kernel<<<nblk(k.n2, 128), 128, 0, st>>>(fa);
+        c->launches++;
+        ss.n_domains += k.nenv;
+        if (c->compact) {
+            compact_select_kernel<<<nblk(k.n2, 128), 128, 0, st>>>(fa, s.cnt + CNT_NDOM, c->d_pos.as<int32_t>(),
+                                                                  c->d_selmulti.as<uint8_t>());
+            c->launches++;
+            unsigned long long cur = 0;
+            CUDA_TRY(c, cudaMemcpyAsync(&cur, s.cnt + CNT_NDOM, 8, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(c, cudaStreamSynchronize(st));
+            c->ndom = (int64_t)cur;
+        } else {
+            c->ndom += k.nenv;
+        }
+    }
+    CUDA_TRY(c, s.tl.record(S1_SCORE, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    CUDA_TRY(c, cudaGetLastError());
+    ss.ms_fwd += s.tl.ms(S1_FILT, S1_FB);
+    ss.ms_mdom += s.tl.ms(S1_FB, S1_MD);
+    ss.ms_env += s.tl.ms(S1_MD, S1_ENV);
+    ss.ms_final += s.tl.ms(S1_ENV, S1_SCORE);
     return ITSX_OK;
 }
 
@@ -2417,20 +2909,20 @@ int search_stage1(itsx_ctx *c)
     cudaStream_t st = c->stream;
     int rc = search_upload_profiles(c);
     if (rc) return rc;
-    const int P = (int)c->prof.size();
+    S1Call s;
+    const int P = s.P = (int)c->prof.size();
     itsx_search_stats &ss = c->sstats;
     ss = itsx_search_stats{};
     c->ndom = 0;
     c->stage1_done = c->stage2_done = false;
     c->pos_valid = false;
-    const int64_t q0 = c->shard_first;
-    const int64_t qn = c->shard_n < 0 ? c->nseq - q0 : c->shard_n;
-    if (q0 < 0 || qn < 0 || q0 + qn > c->nseq) { c->err = "search: shard outside the sequence set"; return ITSX_EINVAL; }
+    if ((rc = shard_range(c, s.q0, s.qn))) return rc;
+    const int64_t qn = s.qn;
     ss.n_seq = qn; ss.n_prof = P; ss.n_pairs = qn * P;
     CUDA_TRY(c, c->d_counters.ensure(64 * 8));
     CUDA_TRY(c, cudaMemsetAsync(c->d_counters.p, 0, 32 * 8, st));
-    const bool multi_sample = c->have_samples && c->n_samples > 1 && c->d_seq_sample.p != nullptr;
-    const size_t nrep_n = (size_t)P * (multi_sample ? c->n_samples : 1);
+    s.multi_sample = c->have_samples && c->n_samples > 1 && c->d_seq_sample.p != nullptr;
+    const size_t nrep_n = (size_t)P * (s.multi_sample ? c->n_samples : 1);
     CUDA_TRY(c, c->d_nrep.ensure(std::max<size_t>(nrep_n, 1) * 4));
     CUDA_TRY(c, cudaMemsetAsync(c->d_nrep.p, 0, std::max<size_t>(nrep_n, 1) * 4, st));
     c->h_nrep.assign(nrep_n, 0);
@@ -2441,534 +2933,42 @@ int search_stage1(itsx_ctx *c)
     c->compact = c->prm.keep_rows == 2 || (c->prm.keep_rows == 0 && qn > 200000);
     // position table, arg-max keys and the winners' multidomain flags live from stage 1 on (compact mode fills them as
     // it goes; mode 1 re-initialises them in stage 2, which may then be repeated with another domZ)
-    c->npos = qn;
-    CUDA_TRY(c, c->d_pos.ensure((size_t)qn * 9 * 4));
-    CUDA_TRY(c, c->d_best.ensure((size_t)qn * 2 * 8));
-    CUDA_TRY(c, c->d_selmulti.ensure((size_t)qn * 2 + 16));
-    pos_init_kernel<<<nblk(qn, 256), 256, 0, st>>>(c->d_pos.as<int32_t>(), c->d_best.as<unsigned long long>(),
-                                                   c->d_selmulti.as<uint8_t>(), qn);
-    c->launches++;
+    if ((rc = pos_reset(c, qn, true))) return rc;
     const double domz_upper = c->prm.domz_upper > 0 ? (double)c->prm.domz_upper : (double)qn;
-    const double lnP_certain = log(c->prm.domE / std::max(domz_upper, 1.0));
-    int64_t total_env = 0;
-    const int NLANE = 8;
-    rc = ensure_lanes(c, NLANE);
-    if (rc) return rc;
-    unsigned long long *cnt = c->d_counters.as<unsigned long long>();
-
-    cudaEvent_t ev[9];
-    for (auto &e : ev) CUDA_TRY(c, cudaEventCreate(&e));
-    float acc_ms[6] = {0, 0, 0, 0, 0, 0};
-    CUDA_TRY(c, cudaEventRecord(ev[0], st));
-
-    const int ntile_p = (P + MSV_TP - 1) / MSV_TP;
-    const size_t msv_smem = (size_t)MSV_TP * MSV_TABW * 4;
-    CUDA_TRY(c, cudaFuncSetAttribute(msv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msv_smem));
+    s.lnP_certain = log(c->prm.domE / std::max(domz_upper, 1.0));
+    if ((rc = ensure_lanes(c, NLANE))) return rc;
+    s.cnt = c->d_counters.as<unsigned long long>();
+    s.d_nsel = (int32_t *)(s.cnt + 42);
+    CUDA_TRY(c, s.tl.status);
+    CUDA_TRY(c, s.tl.record(S1_CALL0, st));
+    if ((rc = s1_order(c, s))) return rc;
 
     // a chunk's scratch grows with its survivors (up to ~half of the pairs on amplicons: 64 B of envelope list + ~110 B
     // of rescoring output each), so chunks are capped at 2^27 pairs (~12 GB of scratch at 45 % survival)
     int64_t chunk = std::min<int64_t>(qn, std::max<int64_t>(1024, (1LL << 27) / P));
     chunk = std::min<int64_t>(chunk, 1LL << 22);
-    const int Lmax = c->Lmax;
-    // total residues of the shard, for cell accounting
-    double sumL = 0;
-    {
-        size_t tmpb = 0;
-        long long *d_sum = (long long *)(c->d_counters.as<unsigned long long>() + 41);
-        cub::DeviceReduce::Sum(nullptr, tmpb, c->d_seqlen.as<int32_t>() + q0, d_sum, (int)qn, st);
-        CUDA_TRY(c, c->d_tmp.ensure(tmpb));
-        cub::DeviceReduce::Sum(c->d_tmp.p, tmpb, c->d_seqlen.as<int32_t>() + q0, d_sum, (int)qn, st);
-        long long h = 0;
-        CUDA_TRY(c, cudaMemcpyAsync(&h, d_sum, 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(c, cudaStreamSynchronize(st));
-        sumL = (double)h;
-    }
-    double sumM = 0;
-    for (auto &h : c->prof) sumM += h.M;
-    ss.msv_cells = sumL * sumM;
-    // visit the shard's sequences in order of length: the 32 pairs of a warp then run the same number of rows
-    CUDA_TRY(c, c->d_order.ensure((size_t)qn * 4 * 4));
-    int32_t *d_order = c->d_order.as<int32_t>();
-    {
-        int32_t *idx_in = d_order + qn, *len_in = d_order + 2 * qn, *len_out = d_order + 3 * qn;
-        iota_kernel<<<nblk(qn, 256), 256, 0, st>>>(idx_in, (int32_t)q0, qn);
-        CUDA_TRY(c, cudaMemcpyAsync(len_in, c->d_seqlen.as<int32_t>() + q0, (size_t)qn * 4, cudaMemcpyDeviceToDevice, st));
-        int lbits = 1;
-        while ((1 << lbits) <= c->Lmax) lbits++;
-        size_t tbs = 0;
-        cub::DeviceRadixSort::SortPairs(nullptr, tbs, len_in, len_out, idx_in, d_order, (int)qn, 0, lbits, st);
-        CUDA_TRY(c, c->d_tmp.ensure(tbs));
-        cub::DeviceRadixSort::SortPairs(c->d_tmp.p, tbs, len_in, len_out, idx_in, d_order, (int)qn, 0, lbits, st);
-        c->launches += 2;
-    }
-
-    const int fb_warps_per_lane = c->sm_count * FB_CTAS_PER_SM * (FB_THREADS / 32);
-    const int env_warps_per_lane = c->sm_count * ENV_CTAS_PER_SM * (ENV_THREADS / 32);
-    std::vector<int32_t> h_bounds((size_t)P + 1), h_envb((size_t)P + 1);
-    int32_t *d_nsel = (int32_t *)(c->d_counters.as<unsigned long long>() + 42);
-
     for (int64_t s0 = 0; s0 < qn; s0 += chunk) {          // s0: offset into d_order
-        const int ns = (int)std::min<int64_t>(chunk, qn - s0);
-        const size_t npair = (size_t)ns * P;
-        // ---- MSV ----
-        CUDA_TRY(c, cudaEventRecord(ev[1], st));
-        CUDA_TRY(c, c->d_msvres.ensure(npair));
-        CUDA_TRY(c, c->d_flag.ensure(npair + 16));
-        dim3 grid(nblk(ns, MSV_THREADS), ntile_p);
-        msv_kernel<<<grid, MSV_THREADS, msv_smem, st>>>(c->d_seqw.as<uint32_t>(), c->d_seqwoff.as<int64_t>(),
-                                                        c->d_seqlen.as<int32_t>(), d_order, s0, ns, c->d_msvtab.as<uint32_t>(),
-                                                        c->d_pscal.as<ProfScalars>(), P, c->d_tjb.as<uint8_t>(),
-                                                        c->d_nullsc.as<float>(), c->prm.F1,
-                                                        c->d_msvres.as<uint8_t>(), c->d_flag.as<uint8_t>());
-        c->launches++;
-        CUDA_TRY(c, cudaEventRecord(ev[2], st));
-        // ---- compact MSV survivors ----
-        CUDA_TRY(c, c->d_list.ensure(npair * 4 + 16));
-        size_t tmpb = 0;
-        cub::CountingInputIterator<int32_t> iota(0);
-        cub::DeviceSelect::Flagged(nullptr, tmpb, iota, c->d_flag.as<uint8_t>(), c->d_list.as<int32_t>(), d_nsel,
-                                   (int)npair, st);
-        CUDA_TRY(c, c->d_tmp.ensure(tmpb));
-        cub::DeviceSelect::Flagged(c->d_tmp.p, tmpb, iota, c->d_flag.as<uint8_t>(), c->d_list.as<int32_t>(), d_nsel,
-                                   (int)npair, st);
-        int32_t n1 = 0;
-        CUDA_TRY(c, cudaMemcpyAsync(&n1, d_nsel, 4, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(c, cudaStreamSynchronize(st));
-        ss.n_past_msv += n1;
-        if (n1 == 0) {
-            CUDA_TRY(c, cudaEventRecord(ev[3], st));
-            CUDA_TRY(c, cudaEventSynchronize(ev[3]));
-            float ms;
-            cudaEventElapsedTime(&ms, ev[1], ev[2]); acc_ms[0] += ms;
-            continue;
-        }
-        // ---- bias filter ----
-        CUDA_TRY(c, c->d_filtersc.ensure((size_t)n1 * 4));
-        CUDA_TRY(c, c->d_ndom.ensure((size_t)n1 + 16));   // reused as flag2 here
-        bias_kernel<<<nblk(n1, 128), 128, 0, st>>>(c->d_list.as<int32_t>(), d_nsel, d_order, s0, ns, c->d_seqw.as<uint32_t>(),
-                                                   c->d_seqwoff.as<int64_t>(), c->d_seqlen.as<int32_t>(),
-                                                   c->d_pscal.as<ProfScalars>(), c->d_msvres.as<uint8_t>(),
-                                                   c->d_tjb.as<uint8_t>(), c->prm.F1, c->prm.F2, c->d_filtersc.as<float>(),
-                                                   c->d_ndom.as<uint8_t>(), cnt);
-        CUDA_TRY(c, c->d_list2.ensure((size_t)n1 * 4 + 16));
-        CUDA_TRY(c, c->d_fsc2.ensure((size_t)n1 * 4 + 16));
-        int32_t *d_nsel2 = d_nsel + 1;
-        size_t tb1 = 0, tb2 = 0;
-        cub::DeviceSelect::Flagged(nullptr, tb1, c->d_list.as<int32_t>(), c->d_ndom.as<uint8_t>(),
-                                   c->d_list2.as<int32_t>(), d_nsel2, n1, st);
-        cub::DeviceSelect::Flagged(nullptr, tb2, c->d_filtersc.as<float>(), c->d_ndom.as<uint8_t>(),
-                                   c->d_fsc2.as<float>(), d_nsel2, n1, st);
-        CUDA_TRY(c, c->d_tmp.ensure(std::max(tb1, tb2)));
-        cub::DeviceSelect::Flagged(c->d_tmp.p, tb1, c->d_list.as<int32_t>(), c->d_ndom.as<uint8_t>(),
-                                   c->d_list2.as<int32_t>(), d_nsel2, n1, st);
-        cub::DeviceSelect::Flagged(c->d_tmp.p, tb2, c->d_filtersc.as<float>(), c->d_ndom.as<uint8_t>(),
-                                   c->d_fsc2.as<float>(), d_nsel2, n1, st);
-        CUDA_TRY(c, c->d_bounds.ensure((size_t)(P + 1) * 8));
-        bounds_kernel<<<nblk(P + 1, 128), 128, 0, st>>>(c->d_list2.as<int32_t>(), d_nsel2, ns, P,
-                                                        c->d_bounds.as<int32_t>());
-        c->launches += 2;
-        int32_t n2 = 0;
-        CUDA_TRY(c, cudaMemcpyAsync(&n2, d_nsel2, 4, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(c, cudaMemcpyAsync(h_bounds.data(), c->d_bounds.p, (size_t)(P + 1) * 4, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(c, cudaEventRecord(ev[3], st));
-        CUDA_TRY(c, cudaStreamSynchronize(st));
-        ss.n_past_bias += n2;
-        {
-            float ms;
-            cudaEventElapsedTime(&ms, ev[1], ev[2]); acc_ms[0] += ms;
-            cudaEventElapsedTime(&ms, ev[2], ev[3]); acc_ms[1] += ms;
-        }
-        if (n2 == 0) continue;
-
-        // ---- Viterbi filter: only for F2 < P(MSV + bias) <= F1 (never under the reference's F1 == F2) ----
-        if (c->prm.F2 < c->prm.F1) {
-            cudaEvent_t v0, v1;
-            CUDA_TRY(c, cudaEventCreate(&v0));
-            CUDA_TRY(c, cudaEventCreate(&v1));
-            CUDA_TRY(c, cudaEventRecord(v0, st));
-            // the "needs the filter" marks of the surviving entries, compacted like the list itself
-            CUDA_TRY(c, c->d_vneed.ensure((size_t)n1 + 16));
-            CUDA_TRY(c, c->d_vpass.ensure((size_t)n2 + 16));
-            int32_t *d_nsel3 = d_nsel + 2;
-            size_t tv = 0;
-            cub::DeviceSelect::Flagged(nullptr, tv, c->d_ndom.as<uint8_t>(), c->d_ndom.as<uint8_t>(), c->d_vneed.as<uint8_t>(),
-                                       d_nsel3, n1, st);
-            CUDA_TRY(c, c->d_tmp.ensure(tv));
-            cub::DeviceSelect::Flagged(c->d_tmp.p, tv, c->d_ndom.as<uint8_t>(), c->d_ndom.as<uint8_t>(),
-                                       c->d_vneed.as<uint8_t>(), d_nsel3, n1, st);
-            // worklist of the entries the filter has to look at (full warps), its per-profile slices
-            CUDA_TRY(c, c->d_list.ensure((size_t)n2 * 4 * 2 + 64));
-            uint8_t *d_run = c->d_ndom.as<uint8_t>();              // (the bias flags are consumed: reuse as "run" marks)
-            vneed_flag_kernel<<<nblk(n2, 256), 256, 0, st>>>(c->d_vneed.as<uint8_t>(), n2, d_run, c->d_vpass.as<uint8_t>());
-            int32_t *d_vidx = c->d_list.as<int32_t>() + n2;         // second half of d_list (first half: compaction output below)
-            int32_t *d_nv = d_nsel + 3;
-            {
-                cub::CountingInputIterator<int32_t> iota0(0);
-                size_t tq = 0;
-                cub::DeviceSelect::Flagged(nullptr, tq, iota0, d_run, d_vidx, d_nv, n2, st);
-                CUDA_TRY(c, c->d_tmp.ensure(tq));
-                cub::DeviceSelect::Flagged(c->d_tmp.p, tq, iota0, d_run, d_vidx, d_nv, n2, st);
-            }
-            CUDA_TRY(c, c->d_bounds.ensure((size_t)(P + 1) * 8));
-            vbounds_kernel<<<nblk(P + 1, 128), 128, 0, st>>>(c->d_list2.as<int32_t>(), d_vidx, d_nv, ns, P,
-                                                             c->d_bounds.as<int32_t>() + (P + 1));
-            std::vector<int32_t> h_vb((size_t)P + 1);
-            CUDA_TRY(c, cudaMemcpyAsync(h_vb.data(), c->d_bounds.as<int32_t>() + (P + 1), (size_t)(P + 1) * 4,
-                                        cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(c, cudaStreamSynchronize(st));
-            c->launches += 3;
-            CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
-            for (int l = 0; l < NLANE; l++) CUDA_TRY(c, cudaStreamWaitEvent(c->lanes[l], c->ev_a, 0));
-            int vrr = 0;
-            for (int p = 0; p < P; p++) {
-                const int b0 = h_vb[p], cntp = h_vb[p + 1] - b0;
-                if (cntp <= 0) continue;
-                VitArgs va;
-                va.list = c->d_list2.as<int32_t>(); va.filtersc = c->d_fsc2.as<float>();
-                va.vidx = d_vidx + b0; va.count = cntp;
-                va.order = d_order; va.s0 = s0; va.ns = ns; va.prof = p;
-                va.seqw = c->d_seqw.as<uint32_t>(); va.woff = c->d_seqwoff.as<int64_t>(); va.seqlen = c->d_seqlen.as<int32_t>();
-                va.vtab = c->d_vtab.as<int32_t>() + (size_t)p * VIT_WORDS;
-                va.xwmove = c->d_xwmove.as<int16_t>();
-                {
-                    const float scale_w = 500.0f / (float)kLn2;
-                    va.xw_E = (int)roundf(scale_w * (-(float)kLn2));
-                }
-                va.vmu = c->prof[p].ev[EV_VMU]; va.vlambda = c->prof[p].ev[EV_VLAMBDA];
-                va.F2 = c->prm.F2;
-                va.pass = c->d_vpass.as<uint8_t>();
-                va.counters = cnt;
-                vit_kernel<<<nblk(cntp, 128), 128, 0, c->lanes[vrr++ % NLANE]>>>(va);
-                c->launches++;
-            }
-            for (int l = 0; l < NLANE; l++) {
-                CUDA_TRY(c, cudaEventRecord(c->lane_ev[l], c->lanes[l]));
-                CUDA_TRY(c, cudaStreamWaitEvent(st, c->lane_ev[l], 0));
-            }
-            // survivors: list2 / fsc2 compacted by the pass flags (through the bias stage's buffers, then back)
-            size_t t1 = 0, t2 = 0;
-            cub::DeviceSelect::Flagged(nullptr, t1, c->d_list2.as<int32_t>(), c->d_vpass.as<uint8_t>(), c->d_list.as<int32_t>(),
-                                       d_nsel3, n2, st);
-            cub::DeviceSelect::Flagged(nullptr, t2, c->d_fsc2.as<float>(), c->d_vpass.as<uint8_t>(), c->d_filtersc.as<float>(),
-                                       d_nsel3, n2, st);
-            CUDA_TRY(c, c->d_tmp.ensure(std::max(t1, t2)));
-            cub::DeviceSelect::Flagged(c->d_tmp.p, t1, c->d_list2.as<int32_t>(), c->d_vpass.as<uint8_t>(),
-                                       c->d_list.as<int32_t>(), d_nsel3, n2, st);
-            cub::DeviceSelect::Flagged(c->d_tmp.p, t2, c->d_fsc2.as<float>(), c->d_vpass.as<uint8_t>(),
-                                       c->d_filtersc.as<float>(), d_nsel3, n2, st);
-            int32_t n3 = 0;
-            CUDA_TRY(c, cudaMemcpyAsync(&n3, d_nsel3, 4, cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(c, cudaStreamSynchronize(st));
-            if (n3 > 0) {
-                CUDA_TRY(c, cudaMemcpyAsync(c->d_list2.p, c->d_list.p, (size_t)n3 * 4, cudaMemcpyDeviceToDevice, st));
-                CUDA_TRY(c, cudaMemcpyAsync(c->d_fsc2.p, c->d_filtersc.p, (size_t)n3 * 4, cudaMemcpyDeviceToDevice, st));
-            }
-            bounds_kernel<<<nblk(P + 1, 128), 128, 0, st>>>(c->d_list2.as<int32_t>(), d_nsel3, ns, P, c->d_bounds.as<int32_t>());
-            c->launches += 3;
-            CUDA_TRY(c, cudaMemcpyAsync(h_bounds.data(), c->d_bounds.p, (size_t)(P + 1) * 4, cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(c, cudaEventRecord(v1, st));
-            CUDA_TRY(c, cudaStreamSynchronize(st));
-            float msv = 0.f;
-            cudaEventElapsedTime(&msv, v0, v1);
-            ss.ms_vit += msv;
-            cudaEventDestroy(v0);
-            cudaEventDestroy(v1);
-            n2 = n3;
-            CUDA_TRY(c, cudaEventRecord(ev[3], st));        // (the Forward stage's clock starts here)
-        }
-        ss.n_past_vit += n2;
-        if (n2 == 0) continue;
-
-        // ---- Forward / Backward / regions: one launch per profile over side streams ----
-        CUDA_TRY(c, c->d_fwdsc.ensure((size_t)n2 * 4));
-        CUDA_TRY(c, c->d_pairout.ensure((size_t)n2 * 4));
-        CUDA_TRY(c, c->d_ndom.ensure((size_t)n2 + 16));
-        CUDA_TRY(c, c->d_env.ensure((size_t)n2 * ITSX_MAXDOM * 2 * 4));
-        const size_t slab = (size_t)(Lmax + 1) * SPEC_C * 32 * 4;
-        // the slab of a launch holds all its tiles (fbdec_kernel reads them back): a profile's worklist goes in pieces of
-        // at most two tiles per resident warp, and no more than fit the scratch budget
-        const int fb_piece_tiles = (int)std::max<size_t>(
-            1, std::min<size_t>((size_t)fb_warps_per_lane * 2, FB_SCRATCH_BUDGET / (slab * NLANE)));
-        CUDA_TRY(c, c->d_spec.ensure(slab * (size_t)fb_piece_tiles * NLANE));
-        CUDA_TRY(c, c->d_fbscale.ensure((size_t)n2 * 4));
-        CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
-        for (int l = 0; l < NLANE; l++) CUDA_TRY(c, cudaStreamWaitEvent(c->lanes[l], c->ev_a, 0));
-        int lane_rr = 0;
-        for (int p = 0; p < P; p++) {
-            const int b0 = h_bounds[p], cntp = h_bounds[p + 1] - b0;
-            if (cntp <= 0) continue;
-            const int l = lane_rr++ % NLANE;
-            FbArgs fa;
-            fa.list = c->d_list2.as<int32_t>() + b0;
-            fa.filtersc = c->d_fsc2.as<float>() + b0;
-            fa.count = cntp; fa.order = d_order; fa.s0 = s0; fa.ns = ns; fa.prof = p;
-            fa.seqw = c->d_seqw.as<uint32_t>(); fa.woff = c->d_seqwoff.as<int64_t>(); fa.seqlen = c->d_seqlen.as<int32_t>();
-            fa.etab = c->d_etab.as<float>() + (size_t)p * (MAXM + 1) * 16;
-            fa.Lmax = Lmax;
-            fa.tau = c->prof[p].ev[EV_FTAU]; fa.lambda = c->prof[p].ev[EV_FLAMBDA];
-            fa.F3 = c->prm.F3;
-            fa.e_move = expf(-(float)kLn2);
-            fa.fwdsc = c->d_fwdsc.as<float>() + b0;
-            fa.bcksc = c->d_pairout.as<float>() + b0;
-            fa.ndom = c->d_ndom.as<uint8_t>() + b0;
-            fa.env = c->d_env.as<int32_t>() + (size_t)b0 * ITSX_MAXDOM * 2;
-            fa.counters = cnt;
-            fa.scale = nullptr;
-            const int wpc = FB_THREADS / 32;
-            fa.spec = (float *)(c->d_spec.as<char>() + slab * (size_t)fb_piece_tiles * l);
-            for (int e0 = 0; e0 < cntp; e0 += fb_piece_tiles * 32) {
-                FbArgs fp = fa;
-                fp.count = std::min(cntp - e0, fb_piece_tiles * 32);
-                fp.list = fa.list + e0; fp.filtersc = fa.filtersc + e0; fp.fwdsc = fa.fwdsc + e0; fp.bcksc = fa.bcksc + e0;
-                fp.ndom = fa.ndom + e0; fp.env = fa.env + (size_t)e0 * ITSX_MAXDOM * 2;
-                fp.scale = c->d_fbscale.as<float>() + b0 + e0;
-                const int tiles = (fp.count + 31) / 32;
-                const int ctas = std::min((tiles + wpc - 1) / wpc, c->sm_count * FB_CTAS_PER_SM);
-                fb_kernel<<<ctas, FB_THREADS, 0, c->lanes[l]>>>(c->pconst[p], fp);
-                fbdec_kernel<<<(tiles + 3) / 4, 128, 0, c->lanes[l]>>>(fp);
-                c->launches += 2;
-            }
-        }
-        for (int l = 0; l < NLANE; l++) {
-            CUDA_TRY(c, cudaEventRecord(c->lane_ev[l], c->lanes[l]));
-            CUDA_TRY(c, cudaStreamWaitEvent(st, c->lane_ev[l], 0));
-        }
-        CUDA_TRY(c, cudaEventRecord(ev[4], st));
-
-        // ---- multidomain regions: stochastic-traceback clustering replaces the region by its cluster envelopes ----
-        CUDA_TRY(c, c->d_envdc.ensure((size_t)n2 * ITSX_MAXDOM * 4));
-        CUDA_TRY(c, c->d_n2reg.ensure((size_t)n2 * 4));
-        CUDA_TRY(c, cudaMemsetAsync(c->d_n2reg.p, 0, (size_t)n2 * 4, st));
-        if (c->prm.resolve_multidomain) {
-            // flagged regions per entry -> prefix sum -> region list in entry order
-            CUDA_TRY(c, c->d_mdlist.ensure((size_t)(n2 + 1) * 2 * 4));
-            int32_t *d_nreg = c->d_mdlist.as<int32_t>(), *d_base = d_nreg + (n2 + 1);
-            mdcount_kernel<<<nblk(n2 + 1, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), c->d_env.as<int32_t>(), n2, d_nreg);
-            size_t tbm = 0;
-            cub::DeviceScan::ExclusiveSum(nullptr, tbm, d_nreg, d_base, n2 + 1, st);
-            CUDA_TRY(c, c->d_tmp.ensure(tbm));
-            cub::DeviceScan::ExclusiveSum(c->d_tmp.p, tbm, d_nreg, d_base, n2 + 1, st);
-            c->launches += 2;
-            int32_t h_nregions = 0;
-            CUDA_TRY(c, cudaMemcpyAsync(&h_nregions, d_base + n2, 4, cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(c, cudaStreamSynchronize(st));
-            if (h_nregions > 0) {
-                const int NR = h_nregions;
-                CUDA_TRY(c, c->d_mdreg.ensure(((size_t)NR * 3 + (size_t)(NR + 1) * 2) * 4));
-                int32_t *reg_ent = c->d_mdreg.as<int32_t>(), *reg_i = reg_ent + NR, *reg_j = reg_i + NR,
-                        *reg_rows = reg_j + NR, *reg_row = reg_rows + (NR + 1);
-                CUDA_TRY(c, cudaMemsetAsync(reg_rows + NR, 0, 4, st));
-                mdregs_kernel<<<nblk(n2, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), c->d_env.as<int32_t>(), n2, d_base,
-                                                            reg_ent, reg_i, reg_j, reg_rows);
-                cub::DeviceScan::ExclusiveSum(nullptr, tbm, reg_rows, reg_row, NR + 1, st);
-                CUDA_TRY(c, c->d_tmp.ensure(tbm));
-                cub::DeviceScan::ExclusiveSum(c->d_tmp.p, tbm, reg_rows, reg_row, NR + 1, st);
-                c->launches += 2;
-                std::vector<int32_t> h_row((size_t)NR + 1);
-                CUDA_TRY(c, cudaMemcpyAsync(h_row.data(), reg_row, (size_t)(NR + 1) * 4, cudaMemcpyDeviceToHost, st));
-                CUDA_TRY(c, cudaStreamSynchronize(st));
-                CUDA_TRY(c, c->d_mdres.ensure((size_t)NR * sizeof(MdRes)));
-                MdStreams streams;
-                {
-                    const uint32_t x0 = md_rng_state0(42u);
-                    for (int t = 0; t < MD_NSAMPLES; t++) streams.x[t] = md_rng_jump(x0, (uint64_t)t << MD_STREAM_LOG2);
-                }
-                MdArgs ma;
-                ma.reg_ent = reg_ent; ma.reg_i = reg_i; ma.reg_j = reg_j; ma.reg_row = reg_row;
-                ma.list = c->d_list2.as<int32_t>(); ma.order = d_order; ma.s0 = s0; ma.ns = ns;
-                ma.seqw = c->d_seqw.as<uint32_t>(); ma.woff = c->d_seqwoff.as<int64_t>(); ma.seqlen = c->d_seqlen.as<int32_t>();
-                ma.mdtab = c->d_mdtab.as<float>(); ma.etab = c->d_etab.as<float>(); ma.pscal = c->d_pscal.as<ProfScalars>();
-                ma.res = c->d_mdres.as<MdRes>();
-                ma.e_move = expf(-(float)kLn2);
-                ma.counters = cnt;
-                // chunks of regions: slabs (matrix + row tables) and trace records within a fixed HBM budget; consecutive
-                // chunks alternate between two side streams with their own buffers, so that the latency-bound Forward fill of
-                // one chunk runs under the issue-bound tracebacks / clustering of the other
-                const size_t row_bytes = (size_t)MD_W * 16 + sizeof(MdRow), reg_bytes = (size_t)MD_TRACE_BYTES;
-                const size_t budget = (size_t)3 << 30;
-                struct MdChunk { int r0, r1, maxrows, ctas; size_t rows; };
-                std::vector<MdChunk> chunks;
-                const size_t cl_smem = sizeof(MdClustSmem) * MDC_WARPS;
-                CUDA_TRY(c, cudaFuncSetAttribute(mdclust_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cl_smem));
-                int cl_per_sm = 0;      // resident CTAs per SM at this shared-memory size: the grid is ONE wave
-                CUDA_TRY(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cl_per_sm, mdclust_kernel, MDC_WARPS * 32, cl_smem));
-                size_t need_cell[2] = {0, 0}, need_trace[2] = {0, 0}, need_scr[2] = {0, 0};
-                for (int r0 = 0; r0 < NR;) {
-                    int r1 = r0 + 1;
-                    while (r1 < NR && (size_t)(h_row[r1 + 1] - h_row[r0]) * row_bytes + (size_t)(r1 + 1 - r0) * reg_bytes <= budget)
-                        r1++;
-                    MdChunk ch;
-                    ch.r0 = r0; ch.r1 = r1; ch.rows = (size_t)(h_row[r1] - h_row[r0]); ch.maxrows = 0;
-                    for (int r = r0; r < r1; r++) ch.maxrows = std::max(ch.maxrows, h_row[r + 1] - h_row[r]);
-                    ch.ctas = std::min((r1 - r0 + MDC_WARPS - 1) / MDC_WARPS, c->sm_count * std::max(cl_per_sm, 1));
-                    const int par = (int)(chunks.size() & 1);
-                    need_cell[par] = std::max(need_cell[par], ch.rows * row_bytes);
-                    need_trace[par] = std::max(need_trace[par], (size_t)(r1 - r0) * reg_bytes);
-                    need_scr[par] = std::max(need_scr[par], md_clust_bytes(ch.maxrows) * (size_t)ch.ctas * MDC_WARPS);
-                    chunks.push_back(ch);
-                    r0 = r1;
-                }
-                for (int par = 0; par < 2; par++) {
-                    CUDA_TRY(c, c->d_mdcell[par].ensure(need_cell[par]));
-                    CUDA_TRY(c, c->d_mdtrace[par].ensure(need_trace[par]));
-                    CUDA_TRY(c, c->d_mdscratch[par].ensure(need_scr[par]));
-                }
-                CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
-                for (int par = 0; par < 2; par++) CUDA_TRY(c, cudaStreamWaitEvent(c->lanes[par], c->ev_a, 0));
-                for (size_t ci = 0; ci < chunks.size(); ci++) {
-                    const MdChunk &ch = chunks[ci];
-                    const int par = (int)(ci & 1);
-                    cudaStream_t ms = c->lanes[par];
-                    ma.r0 = ch.r0; ma.r1 = ch.r1; ma.row0 = h_row[ch.r0];
-                    ma.cell = c->d_mdcell[par].as<float4>();
-                    ma.rowrec = (MdRow *)(c->d_mdcell[par].as<char>() + ch.rows * MD_W * 16);
-                    ma.trace = c->d_mdtrace[par].as<char>();
-                    ma.maxrows = ch.maxrows;
-                    ma.per_thread = md_clust_bytes(ch.maxrows);
-                    ma.scratch = c->d_mdscratch[par].as<char>();
-                    mdfwd_kernel<<<nblk(ch.r1 - ch.r0, 64), 64, 0, ms>>>(ma);
-                    mdtrace_kernel<<<nblk((int64_t)(ch.r1 - ch.r0) * MD_NSAMPLES, 128), 128, 0, ms>>>(ma, streams);
-                    mdclust_kernel<<<ch.ctas, MDC_WARPS * 32, cl_smem, ms>>>(ma);
-                    c->launches += 3;
-                }
-                for (int par = 0; par < 2; par++) {
-                    CUDA_TRY(c, cudaEventRecord(c->lane_ev[par], c->lanes[par]));
-                    CUDA_TRY(c, cudaStreamWaitEvent(st, c->lane_ev[par], 0));
-                }
-                mdapply_kernel<<<nblk(n2, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), c->d_env.as<int32_t>(), n2, d_base,
-                                                             c->d_mdres.as<MdRes>(), c->d_envdc.as<float>(),
-                                                             c->d_n2reg.as<float>(), cnt);
-                c->launches++;
-            }
-        }
-        CUDA_TRY(c, cudaEventRecord(ev[8], st));
-
-        // ---- envelope worklist ----
-        CUDA_TRY(c, c->d_scan.ensure((size_t)(n2 + 1) * 4));
-        CUDA_TRY(c, c->d_envoff.ensure((size_t)(n2 + 1) * 4));
-        ndom_widen_kernel<<<nblk(n2 + 1, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), n2, c->d_scan.as<int32_t>());
-        size_t tb3 = 0;
-        cub::DeviceScan::ExclusiveSum(nullptr, tb3, c->d_scan.as<int32_t>(), c->d_envoff.as<int32_t>(), n2 + 1, st);
-        CUDA_TRY(c, c->d_tmp.ensure(tb3));
-        cub::DeviceScan::ExclusiveSum(c->d_tmp.p, tb3, c->d_scan.as<int32_t>(), c->d_envoff.as<int32_t>(), n2 + 1, st);
-        gather_bounds_kernel<<<nblk(P + 1, 128), 128, 0, st>>>(c->d_envoff.as<int32_t>(), c->d_bounds.as<int32_t>(), P,
-                                                               c->d_bounds.as<int32_t>() + (P + 1));
-        c->launches += 2;
-        CUDA_TRY(c, cudaMemcpyAsync(h_envb.data(), c->d_bounds.as<int32_t>() + (P + 1), (size_t)(P + 1) * 4,
-                                    cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(c, cudaStreamSynchronize(st));
-        const int nenv = h_envb[P];
-        if (nenv > 0) {
-            CUDA_TRY(c, c->d_envout.ensure((size_t)nenv * 20 * 4));
-            // worklist sorted by (profile, envelope length): two ping-pong buffers for the radix sort
-            CUDA_TRY(c, c->d_envwork.ensure((size_t)nenv * 4 * 4));
-            int32_t *wk_in = c->d_envwork.as<int32_t>(), *wk_out = wk_in + nenv;
-            uint32_t *key_in = (uint32_t *)(wk_in + 2 * (size_t)nenv), *key_out = key_in + nenv;
-            envwork_kernel<<<nblk(n2, 256), 256, 0, st>>>(c->d_ndom.as<uint8_t>(), c->d_envoff.as<int32_t>(), n2,
-                                                          c->d_list2.as<int32_t>(), ns, c->d_env.as<int32_t>(), wk_in,
-                                                          key_in);
-            {
-                int pbits = 1;
-                while ((1 << pbits) < P) pbits++;
-                size_t tbs = 0;
-                cub::DeviceRadixSort::SortPairs(nullptr, tbs, key_in, key_out, wk_in, wk_out, nenv, 0, 12 + pbits, st);
-                CUDA_TRY(c, c->d_tmp.ensure(tbs));
-                cub::DeviceRadixSort::SortPairs(c->d_tmp.p, tbs, key_in, key_out, wk_in, wk_out, nenv, 0, 12 + pbits, st);
-            }
-            c->launches += 2;
-            // envelopes are at most Lmax long; scratch per warp of the grid, whose size the budget bounds
-            const int Ldmax = Lmax;
-            const size_t eslab = (size_t)(Ldmax + 1) * ENV_ROWF * 32 * 4;
-            const int env_wpc = ENV_THREADS / 32;
-            const int env_warps = (int)std::max<size_t>(
-                env_wpc, std::min<size_t>(env_warps_per_lane, ENV_SCRATCH_BUDGET / (eslab * NLANE) / env_wpc * env_wpc));
-            const size_t env_smem = (size_t)(ENV_THREADS / 32) * ENV_RING * (ENV_ROWBYTES + 8);
-            CUDA_TRY(c, cudaFuncSetAttribute(env_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env_smem));
-            CUDA_TRY(c, c->d_envscratch.ensure(eslab * env_warps * NLANE));
-            CUDA_TRY(c, cudaEventRecord(c->ev_b, st));
-            for (int l = 0; l < NLANE; l++) CUDA_TRY(c, cudaStreamWaitEvent(c->lanes[l], c->ev_b, 0));
-            lane_rr = 0;
-            for (int p = 0; p < P; p++) {
-                const int e0 = h_envb[p], cnte = h_envb[p + 1] - e0;
-                if (cnte <= 0) continue;
-                const int l = lane_rr++ % NLANE;
-                EnvArgs ea;
-                ea.work = wk_out + e0;
-                ea.envoff = c->d_envoff.as<int32_t>();
-                ea.count = cnte;
-                ea.list = c->d_list2.as<int32_t>();
-                ea.env = c->d_env.as<int32_t>();
-                ea.order = d_order; ea.s0 = s0; ea.ns = ns; ea.prof = p;
-                ea.seqw = c->d_seqw.as<uint32_t>(); ea.woff = c->d_seqwoff.as<int64_t>(); ea.seqlen = c->d_seqlen.as<int32_t>();
-                ea.etab = c->d_etab.as<float>() + (size_t)p * (MAXM + 1) * 16;
-                ea.scratch = (float *)(c->d_envscratch.as<char>() + eslab * env_warps * l);
-                ea.Ldmax = Ldmax;
-                ea.out = c->d_envout.as<float>();
-                ea.out_base = e0;
-                ea.counters = cnt;
-                const int tiles = (cnte + 31) / 32;
-                const int ctas = std::min((tiles + env_wpc - 1) / env_wpc, env_warps / env_wpc);
-                env_kernel<<<ctas, ENV_THREADS, env_smem, c->lanes[l]>>>(c->pconst[p], ea);
-                c->launches++;
-            }
-            for (int l = 0; l < NLANE; l++) {
-                CUDA_TRY(c, cudaEventRecord(c->lane_ev[l], c->lanes[l]));
-                CUDA_TRY(c, cudaStreamWaitEvent(st, c->lane_ev[l], 0));
-            }
-        }
-        CUDA_TRY(c, cudaEventRecord(ev[5], st));
-        // ---- scores ----
-        if (nenv > 0) {
-            CUDA_TRY(c, c->d_doms.ensure((size_t)(c->ndom + nenv) * sizeof(DomRec), true, st));
-            FinalArgs fa;
-            fa.list = c->d_list2.as<int32_t>(); fa.n = n2; fa.order = d_order; fa.s0 = s0; fa.ns = ns;
-            fa.seqw = c->d_seqw.as<uint32_t>(); fa.woff = c->d_seqwoff.as<int64_t>(); fa.seqlen = c->d_seqlen.as<int32_t>();
-            fa.pscal = c->d_pscal.as<ProfScalars>(); fa.nullsctab = c->d_nullsc.as<float>();
-            fa.logsum = c->d_logsum.as<float>(); fa.fwdsc = c->d_fwdsc.as<float>();
-            fa.ndom = c->d_ndom.as<uint8_t>(); fa.envoff = c->d_envoff.as<int32_t>(); fa.env = c->d_env.as<int32_t>();
-            fa.envdc = c->d_envdc.as<float>(); fa.n2reg = c->d_n2reg.as<float>();
-            fa.envout = c->d_envout.as<float>(); fa.T = c->prm.T;
-            fa.doms = c->d_doms.as<DomRec>() + (c->compact ? 0 : c->ndom);
-            fa.nrep = c->d_nrep.as<int32_t>(); fa.counters = cnt;
-            fa.seq_sample = multi_sample ? c->d_seq_sample.as<int32_t>() : nullptr; fa.P = P;
-            fa.compact = c->compact ? 1 : 0;
-            fa.best = c->d_best.as<unsigned long long>(); fa.nseq = qn; fa.seq_first = q0;
-            fa.lnP_certain = lnP_certain;
-            final_kernel<<<nblk(n2, 128), 128, 0, st>>>(fa);
-            c->launches++;
-            total_env += nenv;
-            if (c->compact) {
-                compact_select_kernel<<<nblk(n2, 128), 128, 0, st>>>(fa, cnt + CNT_NDOM, c->d_pos.as<int32_t>(),
-                                                                    c->d_selmulti.as<uint8_t>());
-                c->launches++;
-                unsigned long long cur = 0;
-                CUDA_TRY(c, cudaMemcpyAsync(&cur, cnt + CNT_NDOM, 8, cudaMemcpyDeviceToHost, st));
-                CUDA_TRY(c, cudaStreamSynchronize(st));
-                c->ndom = (int64_t)cur;
-            } else {
-                c->ndom += nenv;
-            }
-        }
-        CUDA_TRY(c, cudaEventRecord(ev[6], st));
-        CUDA_TRY(c, cudaStreamSynchronize(st));
-        CUDA_TRY(c, cudaGetLastError());
-        {
-            float ms;
-            cudaEventElapsedTime(&ms, ev[3], ev[4]); acc_ms[2] += ms;
-            cudaEventElapsedTime(&ms, ev[4], ev[8]); acc_ms[5] += ms;
-            cudaEventElapsedTime(&ms, ev[8], ev[5]); acc_ms[3] += ms;
-            cudaEventElapsedTime(&ms, ev[5], ev[6]); acc_ms[4] += ms;
-        }
+        S1Chunk k{s0, (int)std::min<int64_t>(chunk, qn - s0)};
+        if ((rc = s1_msv(c, s, k))) return rc;
+        if (k.n1 == 0) continue;
+        if ((rc = s1_bias(c, s, k))) return rc;
+        if (k.n2 == 0) continue;
+        if (c->prm.F2 < c->prm.F1 && (rc = s1_viterbi(c, s, k))) return rc;
+        ss.n_past_vit += k.n2;
+        if (k.n2 == 0) continue;
+        if ((rc = s1_fwdbck(c, s, k)) || (rc = s1_multidomain(c, s, k)) || (rc = s1_envelopes(c, s, k)) ||
+            (rc = s1_scores(c, s, k)))
+            return rc;
     }
-    CUDA_TRY(c, cudaEventRecord(ev[7], st));
+
+    CUDA_TRY(c, s.tl.record(S1_CALL1, st));
     unsigned long long h_cnt[CNT_N];
-    CUDA_TRY(c, cudaMemcpyAsync(h_cnt, cnt, sizeof(h_cnt), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaMemcpyAsync(h_cnt, s.cnt, sizeof(h_cnt), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(c, cudaMemcpyAsync(c->h_nrep.data(), c->d_nrep.p, nrep_n * 4, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     CUDA_TRY(c, cudaGetLastError());
     ss.n_past_fwd = (int64_t)h_cnt[CNT_PAST_FWD];
     ss.n_hits_reported = (int64_t)h_cnt[CNT_HITS_REPORTED];
-    ss.n_domains = total_env;
     c->n_certain_rows = (int64_t)h_cnt[CNT_CERTAIN];
     ss.n_multidomain_regions = (int64_t)h_cnt[CNT_MULTI];
     ss.n_dom_overflow = (int64_t)h_cnt[CNT_DOM_OVERFLOW];
@@ -2978,10 +2978,7 @@ int search_stage1(itsx_ctx *c)
     ss.fwd_cells = (double)h_cnt[CNT_FWD_ROWS] * MAXM;
     ss.bck_cells = (double)h_cnt[CNT_BCK_ROWS] * MAXM;
     ss.env_cells = (double)h_cnt[CNT_ENV_ROWS] * MAXM * 2;
-    ss.ms_msv = acc_ms[0]; ss.ms_bias = acc_ms[1]; ss.ms_fwd = acc_ms[2]; ss.ms_env = acc_ms[3]; ss.ms_final = acc_ms[4];
-    ss.ms_mdom = acc_ms[5];
-    cudaEventElapsedTime(&ss.ms_total, ev[0], ev[7]);
-    for (auto &e : ev) cudaEventDestroy(e);
+    ss.ms_total = s.tl.ms(S1_CALL0, S1_CALL1);
     c->stage1_done = true;
     if (ss.n_dom_overflow > 0) {
         c->err = "search: a hit had more than ITSX_MAXDOM envelopes";
@@ -2995,30 +2992,19 @@ int search_stage2(itsx_ctx *c)
     if (!c->stage1_done) { c->err = "search: stage2 before stage1"; return ITSX_EINVAL; }
     cudaStream_t st = c->stream;
     const int P = (int)c->prof.size();
-    {
-        // itsx_profiles_set_sides after stage1 (ItsPosition learns the region only now): refresh the tables
-        int rc = search_upload_profiles(c);
-        if (rc) return rc;
-    }
-    const int64_t q0 = c->shard_first;
-    const int64_t qn = c->shard_n < 0 ? c->nseq - q0 : c->shard_n;
+    // itsx_profiles_set_sides after stage1 (ItsPosition learns the region only now): refresh the tables
+    int rc = search_upload_profiles(c);
+    if (rc) return rc;
+    int64_t q0, qn;
+    if ((rc = shard_range(c, q0, qn))) return rc;
     if (c->compact && c->stage2_applied) {
         c->err = "search: stage 2 was already applied to this compact search (keep_rows 2); run stage 1 again";
         return ITSX_EINVAL;
     }
-    c->npos = qn;
-    CUDA_TRY(c, c->d_pos.ensure((size_t)std::max<int64_t>(qn, 1) * 9 * 4));
-    CUDA_TRY(c, c->d_best.ensure((size_t)std::max<int64_t>(qn, 1) * 2 * 8));
-    CUDA_TRY(c, c->d_selmulti.ensure((size_t)std::max<int64_t>(qn, 1) * 2 + 16));
-    cudaEvent_t e0, e1;
-    CUDA_TRY(c, cudaEventCreate(&e0));
-    CUDA_TRY(c, cudaEventCreate(&e1));
-    CUDA_TRY(c, cudaEventRecord(e0, st));
-    if (qn > 0 && !c->compact) {
-        pos_init_kernel<<<nblk(qn, 256), 256, 0, st>>>(c->d_pos.as<int32_t>(), c->d_best.as<unsigned long long>(),
-                                                       c->d_selmulti.as<uint8_t>(), qn);
-        c->launches++;
-    }
+    Timeline<2> tl;
+    CUDA_TRY(c, tl.status);
+    CUDA_TRY(c, tl.record(0, st));
+    if ((rc = pos_reset(c, qn, !c->compact))) return rc;
     unsigned long long *cnt = c->d_counters.as<unsigned long long>();
     c->sstats.n_domains_reported = c->compact ? c->n_certain_rows : 0;
     c->sstats.n_selected_multidomain = 0;
@@ -3047,15 +3033,12 @@ int search_stage2(itsx_ctx *c)
         c->sstats.n_selected_multidomain = (int64_t)nsm;
     }
     c->stage2_applied = true;
-    CUDA_TRY(c, cudaEventRecord(e1, st));
+    CUDA_TRY(c, tl.record(1, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     CUDA_TRY(c, cudaGetLastError());
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, e0, e1);
+    const float ms = tl.ms(0, 1);
     c->sstats.ms_final += ms;
     c->sstats.ms_total += ms;
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
     c->stage2_done = true;
     c->pos_valid = true;
     return ITSX_OK;

@@ -168,11 +168,10 @@ int itsx_shard_plan(itsx_ctx *c, int G, int64_t *rec_counts, int64_t *byte_count
                                                     c->d_off.as<int64_t>(), nu, G, own_in, idx_in, d_cnt);
         int bits = 1;
         while ((1 << bits) < G) bits++;
-        size_t tb = 0;
         // stable: inside a bucket the uniques stay in first-occurrence order = ascending global read index
-        cub::DeviceRadixSort::SortPairs(nullptr, tb, own_in, own_out, idx_in, c->d_sh_order.as<int32_t>(), (int)nu, 0, bits, st);
-        CUDA_TRY(c, c->d_tmp.ensure(tb));
-        cub::DeviceRadixSort::SortPairs(c->d_tmp.p, tb, own_in, own_out, idx_in, c->d_sh_order.as<int32_t>(), (int)nu, 0, bits, st);
+        CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
+            return cub::DeviceRadixSort::SortPairs(t, b, own_in, own_out, idx_in, c->d_sh_order.as<int32_t>(), (int)nu, 0, bits, st);
+        }));
         c->launches += 2;
     }
     unsigned long long h[2 * 64];
@@ -208,10 +207,7 @@ int itsx_shard_pack(itsx_ctx *c, int64_t first_global_index, uint64_t *rec, uint
     CUDA_TRY(c, c->d_sh_bases.ensure((size_t)c->sh_bytes + 64));
     record_kernel<<<nblk(nu + 1, 256), 256, 0, st>>>(c->d_sh_order.as<int32_t>(), c->d_first.as<int32_t>(),
                                                      c->d_off.as<int64_t>(), nu, first_global_index, d_rec, d_len);
-    size_t tb = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, tb, d_len, d_doff, (int)nu + 1, st);
-    CUDA_TRY(c, c->d_tmp.ensure(tb));
-    cub::DeviceScan::ExclusiveSum(c->d_tmp.p, tb, d_len, d_doff, (int)nu + 1, st);
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, d_len, d_doff, (int)nu + 1, st); }));
     pack_bases_kernel<<<nblk(nu * 32, 256), 256, 0, st>>>(c->d_ascii.as<uint8_t>(), c->d_off.as<int64_t>(),
                                                           c->d_sh_order.as<int32_t>(), c->d_first.as<int32_t>(), d_doff,
                                                           nu, c->d_sh_bases.as<uint8_t>());
@@ -251,10 +247,9 @@ int itsx_shard_owner_derep(itsx_ctx *c, const uint64_t *rec, int64_t nrec, const
         CUDA_TRY(c, c->d_sh_tmp.ensure((size_t)(nrec + 1) * 8));
         int64_t *d_len = c->d_sh_tmp.as<int64_t>();
         reclen_kernel<<<nblk(nrec + 1, 256), 256, 0, st>>>(c->d_sh_rec.as<unsigned long long>(), nrec, d_len);
-        size_t tb = 0;
-        cub::DeviceScan::ExclusiveSum(nullptr, tb, d_len, c->d_off.as<int64_t>(), (int)nrec + 1, st);
-        CUDA_TRY(c, c->d_tmp.ensure(tb));
-        cub::DeviceScan::ExclusiveSum(c->d_tmp.p, tb, d_len, c->d_off.as<int64_t>(), (int)nrec + 1, st);
+        CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
+            return cub::DeviceScan::ExclusiveSum(t, b, d_len, c->d_off.as<int64_t>(), (int)nrec + 1, st);
+        }));
         c->launches += 2;
         int64_t tot = 0;
         CUDA_TRY(c, cudaMemcpyAsync(&tot, c->d_off.as<int64_t>() + nrec, 8, cudaMemcpyDeviceToHost, st));

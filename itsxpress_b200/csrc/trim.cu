@@ -119,12 +119,8 @@ int trim_bounds_dev(itsx_ctx *c, int mode, const int64_t *d_off_sliced, int64_t 
                                                      d_keep, d_lo, d_hi, kf, ol);
     CUDA_TRY(c, cudaMemsetAsync(kf + nreads, 0, 4, st));
     CUDA_TRY(c, cudaMemsetAsync(ol + nreads, 0, 8, st));
-    size_t t1 = 0, t2 = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, t1, kf, ks, (int)nreads + 1, st);
-    cub::DeviceScan::ExclusiveSum(nullptr, t2, ol, os, (int)nreads + 1, st);
-    CUDA_TRY(c, c->d_tmp.ensure(std::max(t1, t2)));
-    cub::DeviceScan::ExclusiveSum(c->d_tmp.p, t1, kf, ks, (int)nreads + 1, st);
-    cub::DeviceScan::ExclusiveSum(c->d_tmp.p, t2, ol, os, (int)nreads + 1, st);
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, kf, ks, (int)nreads + 1, st); },
+                        [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, ol, os, (int)nreads + 1, st); }));
     c->launches += 3;
     int32_t nk = 0;
     CUDA_TRY(c, cudaMemcpyAsync(&nk, ks + nreads, 4, cudaMemcpyDeviceToHost, st));
