@@ -47,6 +47,7 @@ extern "C" {
 
 #define ITSX_MAXM      45  /* longest profile the DP kernels hold in registers (all ITSx_db profiles) */
 #define ITSX_MAXDOM     8  /* envelopes kept per (sequence, profile) hit */
+#define ITSX_CLUSTER_MAXD 64  /* largest edit band of itsx_cluster: reads up to ~6.4 kb at id 0.99 */
 
 typedef struct itsx_ctx itsx_ctx;
 
@@ -330,6 +331,41 @@ int  itsx_derep_resident(itsx_ctx *ctx, int build_search_set, int64_t *n_unique)
 int  itsx_run_resident(itsx_ctx *ctx, const itsx_search_params *prm, itsx_run_stats *st);
 int  itsx_run_fetch(itsx_ctx *ctx, int64_t *n_kept, int64_t *total, int32_t *kept_index, int64_t *out_off,
                     uint8_t *out_seq, uint8_t *out_qual);
+/* ---- clustering below 100 % identity: replaces `vsearch --cluster_size --id X --strand both` (SeqSample.py:133-176) ----
+ * Runs on the exact classes of the resident derep (itsx_derep / itsx_derep_resident, one sample).  Classes are taken in
+ * `order` (unique indices in processing order; NULL = abundance descending, then first occurrence).  ed is unit-cost
+ * Levenshtein distance over the derep's normalised residues, min over both strands of the later class ('+' on a tie);
+ * with L the longer length a pair is accepted iff (L - ed) / L >= id.  A class becomes a centroid iff no earlier centroid
+ * accepts it; otherwise it joins the accepted earlier centroid of highest identity, the earliest on a tie.  Exhaustive:
+ * no k-mer heuristics, terminal gaps count (DESIGN.md §6).
+ * Afterwards the search set is the centroids' first reads in processing order (row r = r-th centroid), and the resident
+ * read -> row map that itsx_trim_* / itsx_derep_map read gives every read its centroid's row; itsx_derep_clusters still
+ * returns the exact classes.  ITSX_ELIMIT when the longest class allows more than ITSX_CLUSTER_MAXD edits,
+ * ITSX_EINVAL with sample ids set.  The next itsx_derep* / itsx_reads_upload / itsx_reads_begin resets the clustering. */
+typedef struct {
+    double  id;             /* identity threshold, 0.5 < id <= 1 */
+    int32_t strand_both;    /* must be 1 */
+    int32_t reserved;
+} itsx_cluster_params;
+typedef struct {
+    int64_t n_unique, n_centroids;
+    int64_t n_segments;     /* pigeonhole index entries */
+    int64_t n_candidates;   /* candidate pairs emitted by the index lookups (with repeats) */
+    int64_t n_verified;     /* distinct candidate pairs given to the banded edit distance */
+    int64_t n_accepted;     /* pairs within the identity threshold */
+    int64_t n_rounds;       /* resolution rounds */
+    int32_t d_max;          /* D(L) of the longest class */
+    int32_t n_len_slots;    /* partner lengths looked up per class and strand */
+    float   ms_index, ms_candidates, ms_verify, ms_resolve, ms_remap, ms_total;
+} itsx_cluster_stats;
+int  itsx_cluster(itsx_ctx *ctx, const itsx_cluster_params *prm, const int32_t *order, int64_t *n_centroids);
+/* per unique (first-occurrence order): row of its centroid, strand relative to it (0 '+', 1 '-'), ed to it; per row:
+ * the unique index of the centroid.  Any pointer may be NULL. */
+int  itsx_cluster_fetch(itsx_ctx *ctx, int32_t *centroid_row_of_unique, uint8_t *strand_of_unique, int32_t *ed_of_unique,
+                        int32_t *unique_of_row);
+int  itsx_cluster_get_stats(const itsx_ctx *ctx, itsx_cluster_stats *st);
+/* host only: dmax[L] = the largest ed with (L - ed) / L >= id for L = 0 .. lmax (the acceptance table of itsx_cluster) */
+int  itsx_cluster_dtable(double id, int32_t lmax, int32_t *dmax);
 /* number of kernel launches issued by this ctx so far (bench.py's gpu_launches) */
 int64_t itsx_launch_count(const itsx_ctx *ctx);
 

@@ -157,12 +157,66 @@ class SeqSample:
         self.fastq = self.seq_file = self.r1 = oriented
 
     def cluster(self, threads, cluster_id=0.995):
-        """vsearch --cluster_size (SeqSample.py:133-176); approximate clustering is not part of the GPU path."""
-        self.uc_file = os.path.join(self.tempdir, "uc.txt")
-        self.rep_file = os.path.join(self.tempdir, "rep.fa")
-        _external("Vsearch", ["vsearch", "--cluster_size", self.seq_file, "--centroids", self.rep_file, "--uc",
-                              self.uc_file, "--strand", "both", "--id", str(cluster_id), "--threads",
-                              str(threads)], "clustering")
+        """Greedy clustering of the reads at ``cluster_id`` identity on the GPU; writes ``uc.txt`` and ``rep.fa`` in the
+        layout of `vsearch --cluster_size --strand both` (replaces SeqSample.py:133-176).
+
+        The exact derep runs first (in memory or streamed) and its classes are clustered (``itsx_cluster``): classes are
+        taken by abundance descending, then by label as ``host.cluster_order`` sorts them (first occurrence for a
+        streamed input); a class becomes a centroid unless an earlier centroid is within ``cluster_id`` identity (edit
+        distance over the longer length, both strands), else it joins the closest such centroid, the earliest on a tie.
+        The search then runs on the centroids only, and every read is trimmed with its centroid's positions.
+        Deliberate differences from vsearch (DESIGN.md §6): abundance comes from the exact derep (vsearch, given raw
+        reads without --sizein, sees abundance 1 everywhere and sorts by label); the search is exhaustive (no
+        --maxaccepts / --maxrejects k-mer heuristics); terminal gaps count (vsearch's default --iddef 2 ignores them,
+        so a truncated read would join a longer centroid at 100 % and be cut at coordinates that are not its own).
+        The H rows of uc.txt carry '*' in the CIGAR column.  ``threads`` is accepted for the reference's signature.
+        ITSX_CLUSTER=vsearch runs the vsearch command of the reference instead."""
+        if os.environ.get("ITSX_CLUSTER", "gpu") == "vsearch":
+            self.uc_file = os.path.join(self.tempdir, "uc.txt")
+            self.rep_file = os.path.join(self.tempdir, "rep.fa")
+            _external("Vsearch", ["vsearch", "--cluster_size", self.seq_file, "--centroids", self.rep_file, "--uc",
+                                  self.uc_file, "--strand", "both", "--id", str(cluster_id), "--threads",
+                                  str(threads)], "clustering")
+            return
+        self.deduplicate(threads)
+        try:
+            s = self._session
+            ctx = get_context()
+            ids = None
+            if s.streamed:
+                order = None
+            else:
+                ids = s.ids
+                order = np.searchsorted(s.first, host.cluster_order(s.rep, ids)).astype(np.int32)
+            nu = s.n_unique
+            nc = ctx.cluster(cluster_id, order)
+            crow, cstrand, ced, unique_of_row = ctx.cluster_fetch(nu, nc)
+            if not s.streamed:
+                cls = s.uid                                  # read -> exact class
+                cfirst = s.first[unique_of_row]              # centroid row -> its first read
+                s.uid = crow[cls] if len(cls) else cls
+                s.first = cfirst
+                s.rep = cfirst[s.uid] if len(cls) else s.rep
+                if s.files:
+                    batch = s.batch
+                    dstrand = ctx.derep_map(batch.n)[1]
+                    strand = dstrand ^ cstrand[cls]
+                    L = batch.s_len.astype(np.int64)
+                    Lc = np.maximum(L, L[s.rep])
+                    ident = np.where(Lc > 0, 100.0 * (Lc - ced[cls]) / np.maximum(Lc, 1), 100.0)
+                    with open(self.rep_file, "wb") as f:
+                        f.write(host.write_rep_fasta(batch, cfirst.astype(np.int64), ids))
+                    with open(self.uc_file, "wb") as f:
+                        f.write(host.write_uc_py(s.rep, strand, ids, batch.s_len, cfirst, identity=ident))
+            s.n_unique = nc
+            s.seq_ids = None
+            st = ctx.cluster_stats()
+            logging.info("GPU clustering at %.4g identity: %d unique sequences -> %d centroids (%d candidate pairs, %d "
+                         "distinct, %d accepted, %d rounds), %.2f ms on device" %
+                         (cluster_id, nu, nc, st.n_candidates, st.n_verified, st.n_accepted, st.n_rounds, st.ms_total))
+        except Exception as e:
+            logging.exception("Could not perform clustering on the GPU.")
+            raise e
 
     # -- the hot path ---------------------------------------------------------------------------------------
     def deduplicate(self, threads=1):

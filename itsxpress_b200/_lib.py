@@ -50,6 +50,20 @@ class DerepStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class ClusterParams(C.Structure):
+    _fields_ = [("id", C.c_double), ("strand_both", C.c_int32), ("reserved", C.c_int32)]
+
+
+class ClusterStats(C.Structure):
+    _fields_ = [(n, C.c_int64) for n in ("n_unique", "n_centroids", "n_segments", "n_candidates", "n_verified",
+                                          "n_accepted", "n_rounds")] + \
+               [("d_max", C.c_int32), ("n_len_slots", C.c_int32)] + \
+               [(n, C.c_float) for n in ("ms_index", "ms_candidates", "ms_verify", "ms_resolve", "ms_remap", "ms_total")]
+
+    def asdict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 class MergeParams(C.Structure):
     _fields_ = [("maxdiffs", C.c_int32), ("allow_stagger", C.c_int32), ("qmax", C.c_int32), ("minovlen", C.c_int32),
                 ("qmaxout", C.c_int32), ("qminout", C.c_int32), ("ascii", C.c_int32), ("reserved", C.c_int32),
@@ -99,6 +113,7 @@ SYMBOLS = [
     "itsx_gz_open", "itsx_gz_read", "itsx_gz_eof", "itsx_gz_close", "itsx_gz_tune", "itsx_gz_stat",
     "itsx_host_last_error", "itsx_fastq_index", "itsx_fastq_cut", "itsx_bytes_gather", "itsx_fastq_format", "itsx_domtbl_format",
     "itsx_fastq_labels", "itsx_uc_format", "itsx_repfa_format",
+    "itsx_cluster", "itsx_cluster_fetch", "itsx_cluster_get_stats", "itsx_cluster_dtable",
 ]
 
 
@@ -138,6 +153,10 @@ def lib():
     L.itsx_derep_unique_keys.argtypes = [vp, vp]
     L.itsx_derep_get_stats.argtypes = [vp, C.POINTER(DerepStats)]
     L.itsx_derep_set_key_bits.argtypes = [vp, C.c_int]
+    L.itsx_cluster.argtypes = [vp, C.POINTER(ClusterParams), vp, vp]
+    L.itsx_cluster_fetch.argtypes = [vp, vp, vp, vp, vp]
+    L.itsx_cluster_get_stats.argtypes = [vp, C.POINTER(ClusterStats)]
+    L.itsx_cluster_dtable.argtypes = [C.c_double, i32, vp]
     L.itsx_search_default_params.argtypes = [C.POINTER(SearchParams)]
     L.itsx_search_default_params.restype = None
     L.itsx_search.argtypes = [vp, C.POINTER(SearchParams)]
@@ -228,6 +247,16 @@ def merge_params(allow_stagger=False, **kw):
     for k, v in kw.items():
         setattr(prm, k, v)
     return prm
+
+
+def cluster_dtable(cluster_id, lmax):
+    """D[L] for L = 0 .. lmax: the largest edit distance a pair whose longer member has length L may have and still be
+    accepted at identity ``cluster_id`` (the table itsx_cluster uses)."""
+    D = np.empty(int(lmax) + 1, np.int32)
+    rc = lib().itsx_cluster_dtable(float(cluster_id), int(lmax), _p(D))
+    if rc < 0:
+        raise ItsxError(rc, "cluster_dtable: id must be in (0.5, 1] and lmax >= 0")
+    return D
 
 
 def default_params():
@@ -383,6 +412,29 @@ class Context:
 
     def set_key_bits(self, bits):
         self._chk(lib().itsx_derep_set_key_bits(self._h, int(bits)))
+
+    # ---- clustering ---------------------------------------------------------------------------
+    def cluster(self, cluster_id, order=None):
+        """Greedy clustering of the resident derep's classes at identity ``cluster_id`` (itsx_cluster).  ``order``: unique
+        indices in processing order (None: abundance descending, then first occurrence).  Returns the centroid count;
+        the search set becomes the centroids and the read -> row map their rows."""
+        prm = ClusterParams(float(cluster_id), 1, 0)
+        o = None if order is None else np.ascontiguousarray(order, dtype=np.int32)
+        nc = C.c_int64()
+        self._chk(lib().itsx_cluster(self._h, C.byref(prm), _p(o), C.byref(nc)))
+        return int(nc.value)
+
+    def cluster_fetch(self, n_unique, n_centroids):
+        """(centroid_row_of_unique, strand_of_unique, ed_of_unique, unique_of_row) of the last itsx_cluster."""
+        row, strand = np.empty(n_unique, np.int32), np.empty(n_unique, np.uint8)
+        ed, uor = np.empty(n_unique, np.int32), np.empty(n_centroids, np.int32)
+        self._chk(lib().itsx_cluster_fetch(self._h, _p(row), _p(strand), _p(ed), _p(uor)))
+        return row, strand, ed, uor
+
+    def cluster_stats(self):
+        st = ClusterStats()
+        self._chk(lib().itsx_cluster_get_stats(self._h, C.byref(st)))
+        return st
 
     # ---- search -----------------------------------------------------------------------------
     def search(self, params=None):

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libitsx_b200.so")
-SOURCES = ["api.cu", "derep.cu", "search.cu", "trim.cu", "shard.cu", "merge.cu", "deflate.cu", "hmmfile.cpp", "fastq_host.cpp", "inflate_host.cpp"]
+SOURCES = ["api.cu", "derep.cu", "cluster.cu", "search.cu", "trim.cu", "shard.cu", "merge.cu", "deflate.cu", "hmmfile.cpp", "fastq_host.cpp", "inflate_host.cpp"]
 HEADERS = [os.path.join(CSRC, "itsx_internal.h"), os.path.join(CSRC, "deflate_core.h"), os.path.join(HERE, "..", "include", "itsx_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-fmad=false",

@@ -176,6 +176,7 @@ int itsx_reads_upload(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64
     c->nreads = nreads;
     c->total_bases = total;
     c->n_unique = 0;
+    c->cl_active = false;
     c->map_external = false;
     c->pos_valid = false;
     c->qual_resident = false;
@@ -222,6 +223,7 @@ int itsx_reads_begin(itsx_ctx *c, int64_t nreads_hint, int64_t bases_hint)
     c->nreads = 0;
     c->total_bases = 0;
     c->n_unique = 0;
+    c->cl_active = false;
     c->map_external = false;
     c->pos_valid = false;
     c->qual_resident = false;
@@ -302,7 +304,7 @@ int itsx_trim_gather_range(itsx_ctx *c, int mode, int64_t first, int64_t count, 
     if (c->stream_open) { c->err = "trim: a streamed upload is still open (itsx_reads_end)"; return ITSX_EINVAL; }
     if (mode != 0) { c->err = "trim_gather_range: only mode 0 (the dereplicated reads themselves)"; return ITSX_EINVAL; }
     if (c->map_external) { c->err = "trim_gather_range: no reads are resident"; return ITSX_EINVAL; }
-    if (c->npos != c->n_unique) { c->err = "trim: position table does not cover every unique sequence"; return ITSX_EINVAL; }
+    if (c->npos != map_rows(c)) { c->err = "trim: position table does not cover every unique sequence"; return ITSX_EINVAL; }
     if (first < 0 || count < 0 || first + count > c->nreads) { c->err = "trim_gather_range: range outside the reads"; return ITSX_EINVAL; }
     if (!n_kept || !total) return ITSX_EINVAL;
     cudaStream_t st = c->stream;
@@ -419,6 +421,46 @@ int itsx_derep_set_key_bits(itsx_ctx *c, int bits)
     CHECK_CTX(c);
     if (bits < 1 || bits > 64) return ITSX_EINVAL;
     c->key_bits = bits;
+    return ITSX_OK;
+}
+
+// ---- clustering below 100 % identity (cluster.cu; replaces vsearch --cluster_size, SeqSample.py:133-176) --------------
+int itsx_cluster(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *order, int64_t *n_centroids)
+{
+    CHECK_CTX(c);
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    return cluster_run(c, prm, order, n_centroids);
+}
+
+int itsx_cluster_fetch(itsx_ctx *c, int32_t *centroid_row_of_unique, uint8_t *strand_of_unique, int32_t *ed_of_unique,
+                       int32_t *unique_of_row)
+{
+    CHECK_CTX(c);
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    if (!c->cl_active) { c->err = "cluster_fetch: no clustering of the resident derep (itsx_cluster first)"; return ITSX_EINVAL; }
+    const int64_t nu = c->n_unique, nc = c->cl_ncent;
+    cudaStream_t st = c->stream;
+    const int32_t *crow = c->d_cl_out.as<int32_t>(), *ced = crow + std::max<int64_t>(nu, 1);
+    const uint8_t *cstrand = (const uint8_t *)(ced + std::max<int64_t>(nu, 1));
+    if (nu && centroid_row_of_unique) CUDA_TRY(c, cudaMemcpyAsync(centroid_row_of_unique, crow, (size_t)nu * 4, cudaMemcpyDefault, st));
+    if (nu && strand_of_unique) CUDA_TRY(c, cudaMemcpyAsync(strand_of_unique, cstrand, (size_t)nu, cudaMemcpyDefault, st));
+    if (nu && ed_of_unique) CUDA_TRY(c, cudaMemcpyAsync(ed_of_unique, ced, (size_t)nu * 4, cudaMemcpyDefault, st));
+    if (nc && unique_of_row) CUDA_TRY(c, cudaMemcpyAsync(unique_of_row, c->d_cl_crow.p, (size_t)nc * 4, cudaMemcpyDefault, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    return ITSX_OK;
+}
+
+int itsx_cluster_get_stats(const itsx_ctx *c, itsx_cluster_stats *st)
+{
+    CHECK_CTX(c);
+    if (st) *st = c->clstats;
+    return ITSX_OK;
+}
+
+int itsx_cluster_dtable(double id, int32_t lmax, int32_t *dmax)
+{
+    if (!(id > 0.5 && id <= 1.0) || lmax < 0 || !dmax) return ITSX_EINVAL;
+    cluster_dtable(id, lmax, dmax);
     return ITSX_OK;
 }
 
@@ -587,6 +629,7 @@ int itsx_trim_set_map(itsx_ctx *c, const int32_t *uid, int64_t nreads, int64_t n
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     c->nreads = nreads;
     c->n_unique = n_unique;
+    c->cl_active = false;
     c->total_bases = 0;       // no resident read bytes: itsx_trim_* must be given seq/qual/off
     c->map_external = true;
     return ITSX_OK;
@@ -597,7 +640,7 @@ static int check_trim(itsx_ctx *c, int mode, int64_t nreads)
     if (c->stream_open) { c->err = "trim: a streamed upload is still open (itsx_reads_end)"; return ITSX_EINVAL; }
     if (mode < 0 || mode > 2) { c->err = "trim: mode must be 0, 1 or 2"; return ITSX_EINVAL; }
     if (nreads != c->nreads) { c->err = "trim: read count differs from the dereplicated set"; return ITSX_EINVAL; }
-    if (c->npos != c->n_unique) { c->err = "trim: position table does not cover every unique sequence"; return ITSX_EINVAL; }
+    if (c->npos != map_rows(c)) { c->err = "trim: position table does not cover every unique sequence"; return ITSX_EINVAL; }
     return ITSX_OK;
 }
 

@@ -310,6 +310,7 @@ int derep_run(itsx_ctx *c)
     ds.n_reads = n;
     ds.bytes_ascii = total;
     c->n_unique = 0;
+    c->cl_active = false;
     if (n == 0) return ITSX_OK;
     if (n >= 0x7fffffffLL) { c->err = "derep: more than 2^31-1 reads in one call"; return ITSX_ELIMIT; }
 

@@ -138,6 +138,13 @@ struct itsx_ctx {
     bool map_external = false;        // d_uid installed by itsx_trim_set_map (no resident read bytes)
     int key_bits = 64;
     itsx_derep_stats dstats{};
+    // clustering of the derep classes (cluster.cu): while cl_active, d_uid maps reads to centroid rows and the search set is
+    // the cl_ncent centroids; d_cl_class keeps the exact class of every read
+    bool cl_active = false;
+    int64_t cl_ncent = 0;
+    itsx_cluster_stats clstats{};
+    DevBuf d_cl_class, d_cl_order, d_cl_u, d_cl_tab, d_cl_r, d_cl_seg, d_cl_key, d_cl_val, d_cl_cnt, d_cl_cand, d_cl_acc;
+    DevBuf d_cl_edge, d_cl_beg, d_cl_state, d_cl_rres, d_cl_row, d_cl_out, d_cl_crow;
 
     // searched sequences (uniques): nibble-coded residues
     int64_t nseq = 0;
@@ -293,8 +300,14 @@ __device__ __forceinline__ void warp_copy(const uint8_t *__restrict__ src, uint8
 }
 #endif
 
-// stage entry points (implemented in derep.cu / search.cu / trim.cu)
+// rows of the position table the resident read -> row map (d_uid) points into: centroids after itsx_cluster, else classes
+inline int64_t map_rows(const itsx_ctx *c) { return c->cl_active ? c->cl_ncent : c->n_unique; }
+
+// stage entry points (implemented in derep.cu / search.cu / trim.cu / cluster.cu)
 int derep_run(itsx_ctx *c);                                   // reads already in d_ascii/d_off
+int cluster_run(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *order, int64_t *n_centroids);
+void cluster_dtable(double id, int32_t lmax, int32_t *D);
+int search_build_seqs_from_reads(itsx_ctx *c, const int32_t *d_first, int64_t nseq);   // resident reads d_first[0..nseq)
 int search_upload_profiles(itsx_ctx *c);
 int search_build_seqs_from_derep(itsx_ctx *c);                // uniques -> d_seqw
 int search_build_seqs_from_host(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64_t nseq);

@@ -2377,6 +2377,13 @@ int search_build_seqs_from_derep(itsx_ctx *c)
     return ITSX_OK;
 }
 
+int search_build_seqs_from_reads(itsx_ctx *c, const int32_t *d_first, int64_t nseq)
+{
+    c->shard_first = 0;
+    c->shard_n = -1;
+    return build_seqs(c, c->d_ascii.as<uint8_t>(), c->d_off.as<int64_t>(), d_first, nseq);
+}
+
 int search_build_seqs_from_host(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64_t nseq)
 {
     // staged through separate buffers so that the reads of a previous itsx_derep stay resident

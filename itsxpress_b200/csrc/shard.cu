@@ -229,6 +229,7 @@ int itsx_shard_owner_derep(itsx_ctx *c, const uint64_t *rec, int64_t nrec, const
     c->nreads = nrec;
     c->total_bases = nbytes;
     c->n_unique = 0;
+    c->cl_active = false;
     c->map_external = false;
     c->pos_valid = false;
     c->sh_G = 0;

@@ -95,9 +95,10 @@ def write_uc(rep_index, strand, ids, lengths, order, batch=None):
     return dst[:got].tobytes()
 
 
-def write_uc_py(rep_index, strand, ids, lengths, order):
+def write_uc_py(rep_index, strand, ids, lengths, order, identity=None):
     """uc.txt as `vsearch --uc` for --fastx_uniques: per cluster an S row then its H rows in input order,
-    then one C row per cluster; 10 tab-separated columns."""
+    then one C row per cluster; 10 tab-separated columns.  ``identity`` (percent per read) fills the H rows' identity
+    column, as --cluster_size writes it; without it every H row is 100.0."""
     rep_index = np.asarray(rep_index)
     n = len(rep_index)
     order = np.asarray(order).tolist()
@@ -111,8 +112,9 @@ def write_uc_py(rep_index, strand, ids, lengths, order):
     for c, r in enumerate(order):
         lines.append("S\t%d\t%d\t*\t*\t*\t*\t*\t%s\t*\n" % (c, int(lengths[r]), ids[r]))
         for i in members[c]:
-            lines.append("H\t%d\t%d\t100.0\t%s\t0\t0\t*\t%s\t%s\n" %
-                         (c, int(lengths[i]), "-" if strand is not None and strand[i] else "+", ids[i], ids[r]))
+            lines.append("H\t%d\t%d\t%.1f\t%s\t0\t0\t*\t%s\t%s\n" %
+                         (c, int(lengths[i]), 100.0 if identity is None else float(identity[i]),
+                          "-" if strand is not None and strand[i] else "+", ids[i], ids[r]))
     for c, r in enumerate(order):
         lines.append("C\t%d\t%d\t*\t*\t*\t*\t*\t%s\t*\n" % (c, 1 + len(members[c]), ids[r]))
     return "".join(lines).encode()

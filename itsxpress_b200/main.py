@@ -4,8 +4,10 @@ reference's itsxpress/main.py (parser :74-170, workflow :486-654), driving the B
 
 Stage order is the reference's: [merge pairs] -> dereplicate -> build the runtime profile set -> search ->
 ItsPosition -> Dedup -> write trimmed reads -> count reads.  Pair merging runs on the GPU as well
-(SeqSample._merge_reads -> itsx_merge_pairs).  --trim-ccs orientation and --cluster_id < 1 still need vsearch
-(they are outside the GPU path) and fail the way the reference fails when vsearch is absent.
+(SeqSample._merge_reads -> itsx_merge_pairs), and so does clustering at --cluster_id < 1 (SeqSample.cluster ->
+itsx_cluster: the exact derep's classes clustered greedily, DESIGN.md section 6; ITSX_CLUSTER=vsearch runs vsearch
+--cluster_size instead).  --trim-ccs orientation still needs vsearch and fails the way the reference fails when vsearch
+is absent.
 """
 import argparse
 import contextlib

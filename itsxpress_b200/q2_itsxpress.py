@@ -2,8 +2,10 @@
 trim_pair :156, trim_pair_output_unmerged :194, main :232-364) on top of the GPU path.
 
 Per sample (derep clusters, Z and domZ are per sample upstream, :273-296): check the FASTQs, [merge pairs],
-dereplicate, build the runtime profile set, search, ItsPosition, Dedup, write gzipped output named after the
-input file into a Casava-1.8 single-lane-per-sample directory.
+dereplicate (or, with cluster_id < 1, cluster the dereplicated classes on the GPU: SeqSample.cluster), build the
+runtime profile set, search, ItsPosition, Dedup, write gzipped output named after the input file into a Casava-1.8
+single-lane-per-sample directory.  Samples with cluster_id < 1 always take this per-sample loop, never the batched
+multi-sample pass (_can_batch).
 
 ``per_sample_sequences`` is duck-typed exactly as upstream uses it: ``.manifest.view(pd.DataFrame)`` must give
 a frame indexed by sample id with columns ``forward`` [, ``reverse``].  When q2_types is installed the real
