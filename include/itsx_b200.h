@@ -332,7 +332,7 @@ int  itsx_run_resident(itsx_ctx *ctx, const itsx_search_params *prm, itsx_run_st
 int  itsx_run_fetch(itsx_ctx *ctx, int64_t *n_kept, int64_t *total, int32_t *kept_index, int64_t *out_off,
                     uint8_t *out_seq, uint8_t *out_qual);
 /* ---- clustering below 100 % identity: replaces `vsearch --cluster_size --id X --strand both` (SeqSample.py:133-176) ----
- * Runs on the exact classes of the resident derep (itsx_derep / itsx_derep_resident, one sample).  Classes are taken in
+ * Runs on the exact classes of the resident derep (itsx_derep / itsx_derep_resident).  Classes are taken in
  * `order` (unique indices in processing order; NULL = abundance descending, then first occurrence).  ed is unit-cost
  * Levenshtein distance over the derep's normalised residues, min over both strands of the later class ('+' on a tie);
  * with L the longer length a pair is accepted iff (L - ed) / L >= id.  A class becomes a centroid iff no earlier centroid
@@ -340,12 +340,19 @@ int  itsx_run_fetch(itsx_ctx *ctx, int64_t *n_kept, int64_t *total, int32_t *kep
  * no k-mer heuristics, terminal gaps count (DESIGN.md §6).
  * Afterwards the search set is the centroids' first reads in processing order (row r = r-th centroid), and the resident
  * read -> row map that itsx_trim_* / itsx_derep_map read gives every read its centroid's row; itsx_derep_clusters still
- * returns the exact classes.  ITSX_ELIMIT when the longest class allows more than ITSX_CLUSTER_MAXD edits,
- * ITSX_EINVAL with sample ids set.  The next itsx_derep* / itsx_reads_upload / itsx_reads_begin resets the clustering. */
+ * returns the exact classes.  ITSX_ELIMIT when the longest class allows more than ITSX_CLUSTER_MAXD edits.
+ * Several samples (itsx_reads_set_samples): per_sample = 1 clusters every sample on its own in the same call, and with
+ * sample ids set per_sample = 0 is ITSX_EINVAL; without sample ids per_sample has no effect.  A class is then compared
+ * only with classes of its own sample (the sample id seeds the index keys, and a hit of another sample is dropped before
+ * verification), so each sample gets exactly the centroids, per-class centroid / strand / ed and relative order of
+ * centroid rows that a call on that sample alone gives with `order` restricted to it.  `order` is any permutation of
+ * the unique indices (the samples need not be contiguous in it; the default order restricts to the default order of
+ * each sample alone), centroid rows follow it across samples, and every centroid row of the search set keeps its
+ * sample, so itsx_search counts domZ per (sample, profile) over the centroids. */
 typedef struct {
     double  id;             /* identity threshold, 0.5 < id <= 1 */
     int32_t strand_both;    /* must be 1 */
-    int32_t reserved;
+    int32_t per_sample;     /* 1: cluster each sample on its own when sample ids are set (else they are refused) */
 } itsx_cluster_params;
 typedef struct {
     int64_t n_unique, n_centroids;
@@ -364,6 +371,9 @@ int  itsx_cluster(itsx_ctx *ctx, const itsx_cluster_params *prm, const int32_t *
 int  itsx_cluster_fetch(itsx_ctx *ctx, int32_t *centroid_row_of_unique, uint8_t *strand_of_unique, int32_t *ed_of_unique,
                         int32_t *unique_of_row);
 int  itsx_cluster_get_stats(const itsx_ctx *ctx, itsx_cluster_stats *st);
+/* test hook: keep only the low `bits` bits of the segment keys of itsx_cluster (forces key collisions, also between
+ * samples); 64 = normal */
+int  itsx_cluster_set_key_bits(itsx_ctx *ctx, int bits);
 /* host only: dmax[L] = the largest ed with (L - ed) / L >= id for L = 0 .. lmax (the acceptance table of itsx_cluster) */
 int  itsx_cluster_dtable(double id, int32_t lmax, int32_t *dmax);
 /* number of kernel launches issued by this ctx so far (bench.py's gpu_launches) */

@@ -51,7 +51,7 @@ class DerepStats(C.Structure):
 
 
 class ClusterParams(C.Structure):
-    _fields_ = [("id", C.c_double), ("strand_both", C.c_int32), ("reserved", C.c_int32)]
+    _fields_ = [("id", C.c_double), ("strand_both", C.c_int32), ("per_sample", C.c_int32)]
 
 
 class ClusterStats(C.Structure):
@@ -113,7 +113,7 @@ SYMBOLS = [
     "itsx_gz_open", "itsx_gz_read", "itsx_gz_eof", "itsx_gz_close", "itsx_gz_tune", "itsx_gz_stat",
     "itsx_host_last_error", "itsx_fastq_index", "itsx_fastq_cut", "itsx_bytes_gather", "itsx_fastq_format", "itsx_domtbl_format",
     "itsx_fastq_labels", "itsx_uc_format", "itsx_repfa_format",
-    "itsx_cluster", "itsx_cluster_fetch", "itsx_cluster_get_stats", "itsx_cluster_dtable",
+    "itsx_cluster", "itsx_cluster_fetch", "itsx_cluster_get_stats", "itsx_cluster_dtable", "itsx_cluster_set_key_bits",
 ]
 
 
@@ -157,6 +157,7 @@ def lib():
     L.itsx_cluster_fetch.argtypes = [vp, vp, vp, vp, vp]
     L.itsx_cluster_get_stats.argtypes = [vp, C.POINTER(ClusterStats)]
     L.itsx_cluster_dtable.argtypes = [C.c_double, i32, vp]
+    L.itsx_cluster_set_key_bits.argtypes = [vp, C.c_int]
     L.itsx_search_default_params.argtypes = [C.POINTER(SearchParams)]
     L.itsx_search_default_params.restype = None
     L.itsx_search.argtypes = [vp, C.POINTER(SearchParams)]
@@ -414,11 +415,12 @@ class Context:
         self._chk(lib().itsx_derep_set_key_bits(self._h, int(bits)))
 
     # ---- clustering ---------------------------------------------------------------------------
-    def cluster(self, cluster_id, order=None):
+    def cluster(self, cluster_id, order=None, per_sample=False):
         """Greedy clustering of the resident derep's classes at identity ``cluster_id`` (itsx_cluster).  ``order``: unique
         indices in processing order (None: abundance descending, then first occurrence).  Returns the centroid count;
-        the search set becomes the centroids and the read -> row map their rows."""
-        prm = ClusterParams(float(cluster_id), 1, 0)
+        the search set becomes the centroids and the read -> row map their rows.  ``per_sample``: with sample ids set
+        (set_samples), cluster every sample on its own; without it sample ids are refused."""
+        prm = ClusterParams(float(cluster_id), 1, int(bool(per_sample)))
         o = None if order is None else np.ascontiguousarray(order, dtype=np.int32)
         nc = C.c_int64()
         self._chk(lib().itsx_cluster(self._h, C.byref(prm), _p(o), C.byref(nc)))
@@ -430,6 +432,10 @@ class Context:
         ed, uor = np.empty(n_unique, np.int32), np.empty(n_centroids, np.int32)
         self._chk(lib().itsx_cluster_fetch(self._h, _p(row), _p(strand), _p(ed), _p(uor)))
         return row, strand, ed, uor
+
+    def cluster_set_key_bits(self, bits):
+        """test hook: itsx_cluster keeps only the low ``bits`` bits of its segment keys (64 = normal)"""
+        self._chk(lib().itsx_cluster_set_key_bits(self._h, int(bits)))
 
     def cluster_stats(self):
         st = ClusterStats()

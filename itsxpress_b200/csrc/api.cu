@@ -432,6 +432,14 @@ int itsx_cluster(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *ord
     return cluster_run(c, prm, order, n_centroids);
 }
 
+int itsx_cluster_set_key_bits(itsx_ctx *c, int bits)
+{
+    CHECK_CTX(c);
+    if (bits < 1 || bits > 64) return ITSX_EINVAL;
+    c->cl_key_bits = bits;
+    return ITSX_OK;
+}
+
 int itsx_cluster_fetch(itsx_ctx *c, int32_t *centroid_row_of_unique, uint8_t *strand_of_unique, int32_t *ed_of_unique,
                        int32_t *unique_of_row)
 {

@@ -21,6 +21,12 @@
 // Losslessness: if ed(u, v) <= d with d <= K(len_v), at least one of the K(len_v)+1 segments of v is untouched by the
 // alignment and occurs exactly in u's strand at its own position shifted by at most d.  Every such lookup is made, so
 // no accepted pair is missed; a 64-bit key collision only adds a candidate that verification rejects.
+//
+// Per sample (sample ids set, per_sample = 1): a class is only ever compared with classes of its own sample.  The sample
+// id seeds every segment key, so a template shared by many samples does not return one index hit per sample, and
+// query_kernel drops any hit of another sample, so a key collision between samples never reaches verify_kernel (which
+// would accept two similar sequences whatever their samples).  With no edge between samples, the rounds resolve every
+// sample exactly as a call on that sample alone with the same relative order would.
 #include <cub/cub.cuh>
 #include "itsx_internal.h"
 
@@ -54,20 +60,29 @@ __device__ __forceinline__ unsigned long long mix64(unsigned long long k)
     k ^= k >> 33;
     return k;
 }
-__device__ unsigned long long seg_key(const uint8_t *__restrict__ s, int L, int rc, int q, int len, int Lv, int j)
+// key of segment j of a class of length Lv in sample smp (0 without per-sample clustering: the keys of one sample are
+// those of a call without samples): seg_key(seg_seed(Lv, j, smp), residues)
+__device__ __forceinline__ unsigned long long seg_seed(int Lv, int j, int smp)
 {
-    unsigned long long h = mix64(((unsigned long long)Lv << 20) ^ (unsigned long long)j ^ 0x9E3779B97F4A7C15ull);
+    return mix64(((unsigned long long)(uint32_t)smp << 40) ^ ((unsigned long long)Lv << 20) ^ (unsigned long long)j ^
+                 0x9E3779B97F4A7C15ull);
+}
+__device__ __forceinline__ unsigned long long seg_key(unsigned long long h, const uint8_t *__restrict__ s, int L, int rc,
+                                                      int q, int len)
+{
     for (int m = 0; m < len; m++) h = (h ^ res_at(s, L, q + m, rc)) * 0x100000001b3ull;
     return mix64(h);
 }
-// segment j of k over a class of length L: [j*L/k, (j+1)*L/k)
-__device__ __forceinline__ int seg_lo(int L, int k, int j) { return (int)((int64_t)j * L / k); }
+// segment j of k over a class of length L: [j*L/k, (j+1)*L/k); j*L/k = j*(L/k) + j*(L%k)/k exactly, in 32 bits (j <= k)
+__device__ __forceinline__ int seg_lo(int L, int k, int j) { return j * (L / k) + j * (L % k) / k; }
 
 inline unsigned nblk(int64_t n, int b) { return (unsigned)((n + b - 1) / b); }
 
+// sample (per read) is null without per-sample clustering; rsample[r] is then 0
 __global__ void prep_kernel(const int32_t *__restrict__ order, const int32_t *__restrict__ first,
-                            const int64_t *__restrict__ off, const int32_t *__restrict__ K, int64_t nu,
-                            int32_t *__restrict__ rfirst, int32_t *__restrict__ rlen, int64_t *__restrict__ nseg,
+                            const int64_t *__restrict__ off, const int32_t *__restrict__ K,
+                            const int32_t *__restrict__ sample, int64_t nu, int32_t *__restrict__ rfirst,
+                            int32_t *__restrict__ rlen, int32_t *__restrict__ rsample, int64_t *__restrict__ nseg,
                             int32_t *__restrict__ rank_of, int32_t *__restrict__ present)
 {
     int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -77,6 +92,7 @@ __global__ void prep_kernel(const int32_t *__restrict__ order, const int32_t *__
     const int L = (int)(off[f + 1] - off[f]);
     rfirst[r] = f;
     rlen[r] = L;
+    rsample[r] = sample ? sample[f] : 0;
     rank_of[u] = (int32_t)r;
     nseg[r] = L > 0 ? K[L] + 1 : 0;
     atomicAdd(&present[L], 1);
@@ -84,8 +100,8 @@ __global__ void prep_kernel(const int32_t *__restrict__ order, const int32_t *__
 
 __global__ void seg_kernel(const uint8_t *__restrict__ ascii, const int64_t *__restrict__ off,
                            const int32_t *__restrict__ rfirst, const int32_t *__restrict__ rlen,
-                           const int64_t *__restrict__ segoff, int64_t nu,
-                           unsigned long long *__restrict__ key, int32_t *__restrict__ val)
+                           const int32_t *__restrict__ rsample, const int64_t *__restrict__ segoff, int64_t nu,
+                           unsigned long long kmask, unsigned long long *__restrict__ key, int32_t *__restrict__ val)
 {
     int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= nu) return;
@@ -95,40 +111,46 @@ __global__ void seg_kernel(const uint8_t *__restrict__ ascii, const int64_t *__r
     const uint8_t *s = ascii + off[rfirst[r]];
     for (int j = 0; j < k; j++) {
         const int a = seg_lo(L, k, j), b = seg_lo(L, k, j + 1);
-        key[o + j] = seg_key(s, L, 0, a, b - a, L, j);
+        key[o + j] = seg_key(seg_seed(L, j, rsample[r]), s, L, 0, a, b - a) & kmask;
         val[o + j] = (int32_t)r;
     }
 }
 
-// thread t = (rank, strand, partner-length slot); pass 0 counts the candidates of t, pass 1 writes them at out[base[t]]
-__global__ void __launch_bounds__(128)
+// thread t = (rank, strand, partner-length slot); pass 0 counts the candidates of t, pass 1 writes them at out[base[t]].
+// 10 blocks per SM leave ptxas room for the loop state without spills (left to itself it takes 32 registers and spills).
+__global__ void __launch_bounds__(128, 10)
 query_kernel(const uint8_t *__restrict__ ascii, const int64_t *__restrict__ off, const int32_t *__restrict__ rfirst,
-             const int32_t *__restrict__ rlen, int64_t nu, int W, const int32_t *__restrict__ D,
-             const int32_t *__restrict__ K, const int32_t *__restrict__ lo, const int32_t *__restrict__ hi,
+             const int32_t *__restrict__ rlen, const int32_t *__restrict__ rsample, int64_t nu, int W,
+             const int32_t *__restrict__ D, const int32_t *__restrict__ K, const int32_t *__restrict__ lo,
+             const int32_t *__restrict__ hi,
              const int32_t *__restrict__ present, const unsigned long long *__restrict__ skey,
-             const int32_t *__restrict__ sval, int64_t nrec, int pass, int64_t *__restrict__ count,
+             const int32_t *__restrict__ sval, int64_t nrec, unsigned long long kmask, int pass,
+             int64_t *__restrict__ count,
              const int64_t *__restrict__ base, unsigned long long *__restrict__ out)
 {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= nu * 2 * W) return;
-    const int64_t r = t / (2 * W);
-    const int rc = (int)((t / W) & 1), slot = (int)(t % W);
+    const int t32 = (int)t;                                    // nu * 2 * W < 2^31 (cluster_run)
+    const int r = t32 / (2 * W);
+    const int rc = (t32 / W) & 1, slot = t32 % W;
     const int Lu = rlen[r];
     const int Lv = lo[Lu] + slot;
     int64_t n = 0;
     if (Lu > 0 && Lv > 0 && Lv <= hi[Lu] && present[Lv] > 0) {
         const uint8_t *s = ascii + off[rfirst[r]];
-        const int d = D[max(Lu, Lv)], k = K[Lv] + 1;
+        const int d = D[max(Lu, Lv)], k = K[Lv] + 1, smp = rsample[r];
         int64_t w = pass ? base[t] : 0;
-        for (int j = 0; j < k; j++) {
-            const int a = seg_lo(Lv, k, j), len = seg_lo(Lv, k, j + 1) - a;
+        for (int j = 0, a = 0, b; j < k; j++, a = b) {
+            b = seg_lo(Lv, k, j + 1);
+            const int len = b - a;
+            const unsigned long long seed = seg_seed(Lv, j, smp);
             for (int q = max(0, a - d); q <= a + d && q + len <= Lu; q++) {
-                const unsigned long long h = seg_key(s, Lu, rc, q, len, Lv, j);
+                const unsigned long long h = seg_key(seed, s, Lu, rc, q, len) & kmask;
                 int64_t x = 0, y = nrec;                               // lower bound of h
                 while (x < y) { const int64_t m = (x + y) >> 1; if (skey[m] < h) x = m + 1; else y = m; }
                 for (; x < nrec && skey[x] == h; x++) {
                     const int32_t v = sval[x];
-                    if (v >= r) continue;
+                    if (v >= r || rsample[v] != smp) continue;
                     if (pass) out[w++] = ((unsigned long long)r << 32) | (uint32_t)v;
                     n++;
                 }
@@ -304,7 +326,10 @@ int cluster_run(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *orde
         c->err = "cluster: no dereplicated reads are resident (itsx_derep / itsx_derep_resident first)";
         return ITSX_EINVAL;
     }
-    if (c->have_samples) { c->err = "cluster: the reads carry sample ids (clustering runs on one sample)"; return ITSX_EINVAL; }
+    if (c->have_samples && !prm->per_sample) {
+        c->err = "cluster: the reads carry sample ids (set per_sample to cluster each sample on its own)";
+        return ITSX_EINVAL;
+    }
     if (nu >= (1ll << 31) - 1) { c->err = "cluster: more than 2^31-2 unique sequences"; return ITSX_ELIMIT; }
     itsx_cluster_stats cs{};
     cs.n_unique = nu;
@@ -377,13 +402,16 @@ int cluster_run(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *orde
     CUDA_TRY(c, cudaMemsetAsync(present, 0, ((size_t)lmax + 1) * 4, st));
 
     // ---- pigeonhole index: K(L)+1 segments per class, sorted by key ------------------------------------------------
-    CUDA_TRY(c, c->d_cl_r.ensure(nu1 * 4 * 3));
-    int32_t *rfirst = c->d_cl_r.as<int32_t>(), *rlen = rfirst + nu1, *rank_of = rlen + nu1;
+    CUDA_TRY(c, c->d_cl_r.ensure(nu1 * 4 * 4));
+    int32_t *rfirst = c->d_cl_r.as<int32_t>(), *rlen = rfirst + nu1, *rank_of = rlen + nu1, *rsample = rank_of + nu1;
+    const int32_t *sample = c->have_samples ? c->d_sample.as<int32_t>() : nullptr;
     CUDA_TRY(c, c->d_cl_seg.ensure((nu1 + 1) * 8 * 2));
     int64_t *nseg = c->d_cl_seg.as<int64_t>(), *segoff = nseg + nu1 + 1;
     int64_t nrec = 0;
+    const unsigned long long kmask = c->cl_key_bits >= 64 ? ~0ull : ((1ull << c->cl_key_bits) - 1ull);
     if (nu) {
-        prep_kernel<<<nblk(nu + 1, 256), 256, 0, st>>>(order, first, off, dK, nu, rfirst, rlen, nseg, rank_of, present);
+        prep_kernel<<<nblk(nu + 1, 256), 256, 0, st>>>(order, first, off, dK, sample, nu, rfirst, rlen, rsample, nseg,
+                                                       rank_of, present);
         CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, nseg, segoff, (int)nu + 1, st); }));
         CUDA_TRY(c, cudaMemcpyAsync(&nrec, segoff + nu, 8, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(c, cudaStreamSynchronize(st));
@@ -395,7 +423,7 @@ int cluster_run(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *orde
     unsigned long long *key = c->d_cl_key.as<unsigned long long>(), *skey = key + std::max<int64_t>(nrec, 1);
     int32_t *val = c->d_cl_val.as<int32_t>(), *sval = val + std::max<int64_t>(nrec, 1);
     if (nrec) {
-        seg_kernel<<<nblk(nu, 128), 128, 0, st>>>(ascii, off, rfirst, rlen, segoff, nu, key, val);
+        seg_kernel<<<nblk(nu, 128), 128, 0, st>>>(ascii, off, rfirst, rlen, rsample, segoff, nu, kmask, key, val);
         c->launches++;
         CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) {
             return cub::DeviceRadixSort::SortPairs(t, b, key, skey, val, sval, (int)nrec, 0, 64, st);
@@ -411,8 +439,8 @@ int cluster_run(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *orde
     int64_t *cnt = c->d_cl_cnt.as<int64_t>(), *cbase = cnt + T + 1;
     int64_t ncand = 0;
     if (nrec) {
-        query_kernel<<<nblk(T, 128), 128, 0, st>>>(ascii, off, rfirst, rlen, nu, W, dD, dK, dLO, dHI, present, skey, sval, nrec,
-                                                   0, cnt, nullptr, nullptr);
+        query_kernel<<<nblk(T, 128), 128, 0, st>>>(ascii, off, rfirst, rlen, rsample, nu, W, dD, dK, dLO, dHI, present,
+                                                   skey, sval, nrec, kmask, 0, cnt, nullptr, nullptr);
         CUDA_TRY(c, cudaMemsetAsync(cnt + T, 0, 8, st));
         CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, cnt, cbase, (int)T + 1, st); }));
         CUDA_TRY(c, cudaMemcpyAsync(&ncand, cbase + T, 8, cudaMemcpyDeviceToHost, st));
@@ -424,8 +452,8 @@ int cluster_run(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *orde
     CUDA_TRY(c, c->d_cl_cand.ensure(nc1 * 8 * 2));
     unsigned long long *cand = c->d_cl_cand.as<unsigned long long>(), *cand2 = cand + nc1;
     if (ncand) {
-        query_kernel<<<nblk(T, 128), 128, 0, st>>>(ascii, off, rfirst, rlen, nu, W, dD, dK, dLO, dHI, present, skey, sval, nrec,
-                                                   1, nullptr, cbase, cand);
+        query_kernel<<<nblk(T, 128), 128, 0, st>>>(ascii, off, rfirst, rlen, rsample, nu, W, dD, dK, dLO, dHI, present,
+                                                   skey, sval, nrec, kmask, 1, nullptr, cbase, cand);
         c->launches++;
     }
     cs.n_candidates = ncand;

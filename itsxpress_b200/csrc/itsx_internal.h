@@ -142,6 +142,7 @@ struct itsx_ctx {
     // the cl_ncent centroids; d_cl_class keeps the exact class of every read
     bool cl_active = false;
     int64_t cl_ncent = 0;
+    int cl_key_bits = 64;
     itsx_cluster_stats clstats{};
     DevBuf d_cl_class, d_cl_order, d_cl_u, d_cl_tab, d_cl_r, d_cl_seg, d_cl_key, d_cl_val, d_cl_cnt, d_cl_cand, d_cl_acc;
     DevBuf d_cl_edge, d_cl_beg, d_cl_state, d_cl_rres, d_cl_row, d_cl_out, d_cl_crow;

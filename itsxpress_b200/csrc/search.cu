@@ -2363,25 +2363,31 @@ static int build_seqs(itsx_ctx *c, const uint8_t *d_ascii, const int64_t *d_off,
     return ITSX_OK;
 }
 
-int search_build_seqs_from_derep(itsx_ctx *c)
+// the search set = resident reads d_first[0..nseq); with sample ids set, every sequence is of its first read's sample
+static int build_seqs_of_reads(itsx_ctx *c, const int32_t *d_first, int64_t nseq)
 {
-    int rc = build_seqs(c, c->d_ascii.as<uint8_t>(), c->d_off.as<int64_t>(), c->d_first.as<int32_t>(), c->n_unique);
+    int rc = build_seqs(c, c->d_ascii.as<uint8_t>(), c->d_off.as<int64_t>(), d_first, nseq);
     if (rc) return rc;
-    if (c->have_samples && c->n_unique > 0) {
-        CUDA_TRY(c, c->d_seq_sample.ensure((size_t)c->n_unique * 4));
-        seqsample_kernel<<<nblk(c->n_unique, 256), 256, 0, c->stream>>>(c->d_sample.as<int32_t>(), c->d_first.as<int32_t>(),
-                                                                       c->n_unique, c->d_seq_sample.as<int32_t>());
+    if (c->have_samples && nseq > 0) {
+        CUDA_TRY(c, c->d_seq_sample.ensure((size_t)nseq * 4));
+        seqsample_kernel<<<nblk(nseq, 256), 256, 0, c->stream>>>(c->d_sample.as<int32_t>(), d_first, nseq,
+                                                                c->d_seq_sample.as<int32_t>());
         c->launches++;
         CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     }
     return ITSX_OK;
 }
 
+int search_build_seqs_from_derep(itsx_ctx *c)
+{
+    return build_seqs_of_reads(c, c->d_first.as<int32_t>(), c->n_unique);
+}
+
 int search_build_seqs_from_reads(itsx_ctx *c, const int32_t *d_first, int64_t nseq)
 {
     c->shard_first = 0;
     c->shard_n = -1;
-    return build_seqs(c, c->d_ascii.as<uint8_t>(), c->d_off.as<int64_t>(), d_first, nseq);
+    return build_seqs_of_reads(c, d_first, nseq);
 }
 
 int search_build_seqs_from_host(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64_t nseq)

@@ -4,14 +4,16 @@ trim_pair :156, trim_pair_output_unmerged :194, main :232-364) on top of the GPU
 Per sample (derep clusters, Z and domZ are per sample upstream, :273-296): check the FASTQs, [merge pairs],
 dereplicate (or, with cluster_id < 1, cluster the dereplicated classes on the GPU: SeqSample.cluster), build the
 runtime profile set, search, ItsPosition, Dedup, write gzipped output named after the input file into a Casava-1.8
-single-lane-per-sample directory.  Samples with cluster_id < 1 always take this per-sample loop, never the batched
-multi-sample pass (_can_batch).
+single-lane-per-sample directory.  Small samples share one device pass (_process_batch) at any cluster_id; with
+cluster_id < 1 each sample of the pass is clustered on its own, in the order SeqSample.cluster uses.  trim_ccs, and
+below 100 % identity ITSX_CLUSTER=vsearch and ITSX_STREAM=1, keep every sample in the per-sample loop (_can_batch).
 
 ``per_sample_sequences`` is duck-typed exactly as upstream uses it: ``.manifest.view(pd.DataFrame)`` must give
 a frame indexed by sample id with columns ``forward`` [, ``reverse``].  When q2_types is installed the real
 directory formats are used; otherwise `CasavaDir` / `PerSampleDir` below read and write the same on-disk
 layout (``MANIFEST``, ``metadata.yml``, ``<sample>_<n>_L001_R<d>_001.fastq.gz``).
 """
+import logging
 import math
 import os
 import pathlib
@@ -162,9 +164,10 @@ def _process_sample(sample, results, tempdir, threads, taxa, region, paired_in, 
 # ---- several samples in one device pass (SURVEY 8f row 3) ---------------------------------------------------------
 # The reference runs vsearch and hmmsearch once PER SAMPLE (q2_itsxpress.py:273-296), so classes never span samples and
 # domZ is per sample.  libitsx_b200 keeps exactly that while batching: the sample id is part of the derep key and of the
-# class test, reported hits are counted per (sample, profile) (itsx_reads_set_samples).  One pass then carries the
-# merged reads of as many samples as fit BATCH_READS; an artifact of many small samples costs one chain of launches
-# instead of one per sample.  Outputs are byte-identical to the per-sample loop (tests/test_gpu_merge.py).
+# class test, reported hits are counted per (sample, profile) (itsx_reads_set_samples), and with cluster_id < 1 every
+# sample is clustered on its own (itsx_cluster per_sample).  One pass then carries the merged reads of as many samples
+# as fit BATCH_READS; an artifact of many small samples costs one chain of launches instead of one per sample.  Outputs
+# are byte-identical to the per-sample loop (tests/test_gpu_merge.py, tests/test_gpu_cluster_samples.py).
 BATCH_READS = int(os.environ.get("ITSX_Q2_BATCH_READS", "4000000"))      # 0 = the per-sample loop
 
 
@@ -196,9 +199,34 @@ def _batches(rows, paired_in, budget):
     return groups
 
 
+def _cluster_batch(ctx, items, starts, nu, cluster_id):
+    """Every sample of the resident batch clustered on its own at ``cluster_id`` in one itsx_cluster call.  A sample's
+    classes are taken in the order SeqSample.cluster gives them (host.cluster_order over the sample's reads and labels;
+    merged records keep R1's title, so a merged read's label is its R1 id), the samples' orders one after the other.
+    Returns the centroid count; the search set and the read -> row map are the centroids' afterwards."""
+    import numpy as np
+    from . import host
+    first, _ = ctx.derep_clusters(nu)
+    rep = ctx.derep_map(int(starts[-1]))[0]
+    order = [np.zeros(0, np.int64)]
+    for k, it in enumerate(items):
+        a, b = int(starts[k]), int(starts[k + 1])
+        if a < b:
+            ids = it["b1"].ids()
+            labels = [ids[i] for i in it["idx"].tolist()]
+            order.append(np.searchsorted(first, host.cluster_order(rep[a:b] - a, labels) + a))
+    nc = ctx.cluster(cluster_id, np.concatenate(order).astype(np.int32), per_sample=True)
+    st = ctx.cluster_stats()
+    logging.info("GPU clustering of %d samples at %.4g identity, each on its own: %d unique sequences -> %d centroids (%d "
+                 "candidate pairs, %d distinct, %d accepted, %d rounds), %.2f ms on device" %
+                 (len(items), cluster_id, nu, nc, st.n_candidates, st.n_verified, st.n_accepted, st.n_rounds, st.ms_total))
+    return nc
+
+
 def _process_batch(rows, results, tempdir, threads, taxa, region, paired_in, paired_out, reversed_primers,
-                   allow_staggered_reads):
-    """The samples `rows` through ONE derep + search pass; per sample the files the sequential loop writes."""
+                   allow_staggered_reads, cluster_id):
+    """The samples `rows` through ONE derep [+ per-sample clustering] + search pass; per sample the files the sequential
+    loop writes."""
     import numpy as np
     from . import _lib
     from .SeqSample import get_context
@@ -250,7 +278,9 @@ def _process_batch(rows, results, tempdir, threads, taxa, region, paired_in, pai
     n_all = len(off_all) - 1
     ctx.reads_upload(seq_all, off_all)
     ctx.set_samples(sample_of_read, max(len(items), 1))
-    nu = ctx.derep_resident()
+    nrow = nu = ctx.derep_resident()
+    if not math.isclose(cluster_id, 1, rel_tol=1e-05):
+        nrow = _cluster_batch(ctx, items, starts, nu, cluster_id)
     ctx.search()
     if not paired_out:
         # merged / single-end output: the re-expansion of the whole batch in one go, split by sample afterwards
@@ -267,7 +297,7 @@ def _process_batch(rows, results, tempdir, threads, taxa, region, paired_in, pai
         return
     # unmerged output: R1 [start:stop], R2 [tlen-stop : tlen-start] of every pair whose merged read was kept
     _, _, uid = ctx.derep_map(n_all)
-    pos = ctx.positions(nu)
+    pos = ctx.positions(nrow)
     start, stop, tlen = pos["start"].copy(), pos["stop"].copy(), pos["tlen"].copy()
     for k, it in enumerate(items):
         b1, b2 = it["b1"], it["b2"]
@@ -275,7 +305,7 @@ def _process_batch(rows, results, tempdir, threads, taxa, region, paired_in, pai
         uid_pair[it["idx"]] = uid[starts[k]:starts[k + 1]]
         outs = []
         for mode, b, raw in ((2, b1, it["raw1"]), (1, b2, it["raw2"])):
-            ctx.trim_set_map(uid_pair, nu)
+            ctx.trim_set_map(uid_pair, nrow)
             ctx.positions_set(start, stop, tlen)
             kk, oo, os_, oq = ctx.trim_gather(b.n, mode=mode, seq=raw[0], qual=raw[1], off=raw[2])
             outs.append((fq.format_gathered(b, kk, oo, os_, oq, as_array=True), len(kk)))
@@ -290,7 +320,14 @@ READ_AHEAD_BYTES = int(os.environ.get("ITSX_READ_AHEAD_BYTES", str(2 << 30)))
 
 
 def _can_batch(cluster_id, trim_ccs):
-    return BATCH_READS > 0 and math.isclose(cluster_id, 1, rel_tol=1e-05) and not trim_ccs
+    """Whether samples may share device passes: not with trim_ccs (orientation runs per sample).  Below 100 % identity
+    also not when ITSX_CLUSTER=vsearch shells out to vsearch, which clusters one sample per call, nor when ITSX_STREAM=1
+    streams every sample: SeqSample.cluster then has no labels and orders ties by first occurrence, not by label as a
+    batched pass does, so the two could pick different centroids."""
+    if not math.isclose(cluster_id, 1, rel_tol=1e-05) and (os.environ.get("ITSX_CLUSTER", "gpu") == "vsearch" or
+                                                            os.environ.get("ITSX_STREAM", "auto") == "1"):
+        return False
+    return BATCH_READS > 0 and not trim_ccs
 
 
 def _run_rows(rows, results, tempdir, threads, taxa, region, paired_in, paired_out, reversed_primers,
@@ -304,7 +341,7 @@ def _run_rows(rows, results, tempdir, threads, taxa, region, paired_in, paired_o
     for gi, group in enumerate(flat):
         if len(group) > 1:
             _process_batch(group, results, tempdir, threads, taxa, region, paired_in, paired_out, reversed_primers,
-                           allow_staggered_reads)
+                           allow_staggered_reads, cluster_id)
         else:
             # read the next samples' files while this one is on the GPU (fq.READ_AHEAD of them, within ~2 GB of files)
             ahead_bytes = 0
