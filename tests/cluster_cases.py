@@ -29,6 +29,7 @@ def edit(rng, s, k, where=None):
     s = bytearray(s)
     for _ in range(k):
         lo, hi = where if where else (0, len(s))
+        lo = min(lo, len(s) - 1)                                     # (deletions may have shortened s below lo)
         p = int(rng.integers(lo, max(lo + 1, min(hi, len(s)))))
         op = int(rng.integers(3))
         if op == 0:
@@ -57,7 +58,7 @@ def planted(seed, L=250, ntemplates=12, D=1):
         reads.append(T[:L - D - 1])                                 # length difference D + 1 (rejected)
         reads.append(T + T[:D])                                     # longer by D
         x = bytearray(edit(rng, T, D))
-        x[int(rng.integers(L - 1))] = ord("N")
+        x[int(rng.integers(len(x) - 1))] = ord("N")
         reads.append(bytes(x).lower())                              # lower case with an N
         y = bytearray(T)
         y[int(rng.integers(L))] = ord("R")

@@ -102,12 +102,63 @@ int64_t ref_cluster(const uint8_t *seq, const int64_t *off, const int32_t *first
     return nc;
 }
 
-/* the ed (<= d, else d + 1) of two byte strings on the '+' strand, for tests of the greedy's inputs */
-int ref_ed(const uint8_t *a, int n, const uint8_t *b, int m, int d)
+/* the number of unordered pairs of distinct uniques of the same group (group[u]: sample or family of unique u) that are
+ * accepted: min(ed(s_u, s_v), ed(rc(s_u), s_v)) <= D(max(len_u, len_v)).  Brute force over every pair of a group whose
+ * lengths are within D; acceptance is symmetric, so this is the number of accepted edges whatever the order.  Only the
+ * pairs whose first member is at a position in [a0, a1) of the (group, unique) order are counted, so that callers can
+ * split the work. */
+static int cmp_group(const void *x, const void *y)
+{
+    const int64_t *a = x, *b = y;       /* (group, unique) */
+    return a[0] != b[0] ? (a[0] < b[0] ? -1 : 1) : (a[1] < b[1] ? -1 : a[1] > b[1]);
+}
+int64_t ref_accepted_pairs(const uint8_t *seq, const int64_t *off, const int32_t *first, int64_t nu, const int32_t *group,
+                           const int32_t *D, int32_t lmax, int64_t a0, int64_t a1)
+{
+    int64_t *ix = malloc(sizeof(int64_t) * 2 * (nu ? nu : 1));
+    unsigned char **fw = malloc(sizeof(*fw) * (nu ? nu : 1)), **rv = malloc(sizeof(*rv) * (nu ? nu : 1));
+    int *len = malloc(sizeof(int) * (nu ? nu : 1));
+    int *prev = malloc(sizeof(int) * (lmax + 2)), *cur = malloc(sizeof(int) * (lmax + 2));
+    for (int64_t u = 0; u < nu; u++) {
+        const uint8_t *s = seq + off[first[u]];
+        const int L = (int)(off[first[u] + 1] - off[first[u]]);
+        len[u] = L;
+        fw[u] = malloc(L + 1);
+        rv[u] = malloc(L + 1);
+        for (int m = 0; m < L; m++) {
+            fw[u][m] = norm(s[m]);
+            rv[u][L - 1 - m] = comp(norm(s[m]));
+        }
+        ix[2 * u] = group[u];
+        ix[2 * u + 1] = u;
+    }
+    qsort(ix, nu, 2 * sizeof(int64_t), cmp_group);
+    int64_t n = 0;
+    for (int64_t a = a0; a < a1 && a < nu; a++) {
+        const int64_t u = ix[2 * a + 1];
+        for (int64_t b = a + 1; b < nu && ix[2 * b] == ix[2 * a]; b++) {
+            const int64_t v = ix[2 * b + 1];
+            const int L = len[u] > len[v] ? len[u] : len[v], d = D[L];
+            if (abs(len[u] - len[v]) > d) continue;
+            if (ed_within(fw[u], len[u], fw[v], len[v], d, prev, cur) <= d ||
+                ed_within(rv[u], len[u], fw[v], len[v], d, prev, cur) <= d)
+                n++;
+        }
+    }
+    for (int64_t u = 0; u < nu; u++) { free(fw[u]); free(rv[u]); }
+    free(ix); free(fw); free(rv); free(len); free(prev); free(cur);
+    return n;
+}
+
+/* the ed (<= d, else d + 1) of a, or of its reverse complement (rc = 1), against b, for tests of the greedy's inputs */
+int ref_ed(const uint8_t *a, int n, const uint8_t *b, int m, int d, int rc)
 {
     unsigned char *x = malloc(n + 1), *y = malloc(m + 1);
     int *prev = malloc(sizeof(int) * (m + 2)), *cur = malloc(sizeof(int) * (m + 2));
-    for (int i = 0; i < n; i++) x[i] = norm(a[i]);
+    for (int i = 0; i < n; i++) {
+        if (rc) x[n - 1 - i] = comp(norm(a[i]));
+        else x[i] = norm(a[i]);
+    }
     for (int j = 0; j < m; j++) y[j] = norm(b[j]);
     int e = ed_within(x, n, y, m, d, prev, cur);
     free(x); free(y); free(prev); free(cur);

@@ -25,8 +25,10 @@ def lib():
         vp = C.c_void_p
         L.ref_cluster.restype = C.c_int64
         L.ref_cluster.argtypes = [vp, vp, vp, C.c_int64, vp, vp, C.c_int32, vp, vp, vp, vp]
+        L.ref_accepted_pairs.restype = C.c_int64
+        L.ref_accepted_pairs.argtypes = [vp, vp, vp, C.c_int64, vp, vp, C.c_int32, C.c_int64, C.c_int64]
         L.ref_ed.restype = C.c_int
-        L.ref_ed.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.c_int, C.c_int]
+        L.ref_ed.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_int]
         _LIB = L
     return _LIB
 
@@ -59,8 +61,32 @@ def cluster(seq, off, first, order, cluster_id):
     return int(nc), crow, strand, ed, uor[:nc]
 
 
-def ed(a, b, d):
-    return lib().ref_ed(a, len(a), b, len(b), d)
+def accepted_pairs(seq, off, first, cluster_id, group=None):
+    """number of unordered pairs of distinct uniques of the same group (per unique; None: one group) whose ed on either
+    strand is at most D(max length): the n_accepted of itsx_cluster on these uniques"""
+    seq = np.ascontiguousarray(seq, np.uint8)
+    off = np.ascontiguousarray(off, np.int64)
+    first = np.ascontiguousarray(first, np.int32)
+    nu = len(first)
+    group = np.zeros(nu, np.int32) if group is None else np.ascontiguousarray(group, np.int32)
+    assert len(group) == nu
+    lens = (off[first + 1] - off[first]) if nu else np.zeros(1, np.int64)
+    D = _lib.cluster_dtable(cluster_id, int(lens.max()) if nu else 0)
+    f = lib().ref_accepted_pairs
+    if nu < 256:
+        return int(f(_p(seq), _p(off), _p(first), nu, _p(group), _p(D), len(D) - 1, 0, nu))
+    # chunks of the outer loop on threads (ctypes releases the GIL); small chunks even out the triangle
+    import concurrent.futures as cf
+    step = max(1, nu // 256)
+    with cf.ThreadPoolExecutor(os.cpu_count()) as ex:
+        parts = ex.map(lambda a: f(_p(seq), _p(off), _p(first), nu, _p(group), _p(D), len(D) - 1, a, a + step),
+                       range(0, nu, step))
+        return int(sum(parts))
+
+
+def ed(a, b, d, rc=False):
+    """ed(a, b), or ed(rc(a), b) with rc, if at most d, else d + 1"""
+    return lib().ref_ed(a, len(a), b, len(b), d, int(rc))
 
 
 class ClusterOracleContext(OracleContext):

@@ -28,7 +28,7 @@ def resident(ctx, seq, off, sample, n_samples):
 
 
 @pytest.mark.parametrize("given_order", [False, True])
-@pytest.mark.parametrize("X", [0.99, 0.995])
+@pytest.mark.parametrize("X", [0.9, 0.97, 0.99, 0.995])
 def test_per_sample_equals_reference_on_each_sample(gpu_ctx, X, given_order):
     D = int(_lib.cluster_dtable(X, 250)[250])
     samples = S.planted_samples(11, D)
