@@ -344,7 +344,8 @@ int derep_run(itsx_ctx *c)
     CUDA_TRY(c, tl.record(0, st));
     CUDA_TRY(c, cudaMemsetAsync(P + nchunk, 0, 8, st));
     CUDA_TRY(c, cudaMemsetAsync(X + nchunk, 0, 4, st));
-    pack2_kernel<<<nblk(nchunk, 256), 256, 0, st>>>((const uint4 *)ascii, nchunk, P, X);
+    if (nchunk > 0)       // reads that are all empty have no bases to pack, and a grid of 0 blocks is a launch error
+        pack2_kernel<<<nblk(nchunk, 256), 256, 0, st>>>((const uint4 *)ascii, nchunk, P, X);
     CUDA_TRY(c, tl.record(1, st));
     const int32_t *d_samp = c->have_samples ? c->d_sample.as<int32_t>() : nullptr;
     hash_kernel<<<nblk(n, 128), 128, 0, st>>>(ascii, off, P, X, n, keymask, d_samp, c->d_key.as<unsigned long long>(),

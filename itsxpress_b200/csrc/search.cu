@@ -2640,6 +2640,19 @@ static int s1_viterbi(itsx_ctx *c, const S1Call &s, S1Chunk &k)
 }
 
 // Forward / Backward / posterior decoding of the n2 entries: one launch per profile (in pieces) over the side streams
+// scratch of `count` units whose count only sets how much of a worklist runs at once (Forward/Backward pieces, resident
+// envelope warps): when the device cannot hold it -- other contexts on the same GPU hold theirs -- the count is halved
+// (in multiples of `step`) until it fits
+static cudaError_t ensure_scratch(DevBuf &b, size_t unit, int &count, int step)
+{
+    for (;;) {
+        const cudaError_t e = b.ensure(unit * (size_t)count);
+        if (e != cudaErrorMemoryAllocation || count <= step) return e;
+        cudaGetLastError();                 // the failed allocation is not an error of the search
+        count = std::max(step, count / 2 / step * step);
+    }
+}
+
 static int s1_fwdbck(itsx_ctx *c, const S1Call &s, const S1Chunk &k)
 {
     const int n2 = k.n2, Lmax = c->Lmax;
@@ -2651,9 +2664,9 @@ static int s1_fwdbck(itsx_ctx *c, const S1Call &s, const S1Chunk &k)
     // the slab of a launch holds all its tiles (fbdec_kernel reads them back): a profile's worklist goes in pieces of
     // at most two tiles per resident warp, and no more than fit the scratch budget
     const int fb_warps_per_lane = c->sm_count * FB_CTAS_PER_SM * (FB_THREADS / 32);
-    const int fb_piece_tiles = (int)std::max<size_t>(
+    int fb_piece_tiles = (int)std::max<size_t>(
         1, std::min<size_t>((size_t)fb_warps_per_lane * 2, FB_SCRATCH_BUDGET / (slab * NLANE)));
-    CUDA_TRY(c, c->d_spec.ensure(slab * (size_t)fb_piece_tiles * NLANE));
+    CUDA_TRY(c, ensure_scratch(c->d_spec, slab * NLANE, fb_piece_tiles, 1));
     CUDA_TRY(c, c->d_fbscale.ensure((size_t)n2 * 4));
     CUDA_TRY(c, fork_lanes(c, NLANE));
     int lane_rr = 0;
@@ -2833,12 +2846,12 @@ static int s1_envelopes(itsx_ctx *c, const S1Call &s, S1Chunk &k)
         // envelopes are at most Lmax long; scratch per warp of the grid, whose size the budget bounds
         const size_t eslab = (size_t)(c->Lmax + 1) * ENV_ROWF * 32 * 4;
         const int env_wpc = ENV_THREADS / 32;
-        const int env_warps = (int)std::max<size_t>(
+        int env_warps = (int)std::max<size_t>(
             env_wpc, std::min<size_t>(c->sm_count * ENV_CTAS_PER_SM * env_wpc,
                                       ENV_SCRATCH_BUDGET / (eslab * NLANE) / env_wpc * env_wpc));
         const size_t env_smem = (size_t)(ENV_THREADS / 32) * ENV_RING * (ENV_ROWBYTES + 8);
         CUDA_TRY(c, cudaFuncSetAttribute(env_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env_smem));
-        CUDA_TRY(c, c->d_envscratch.ensure(eslab * env_warps * NLANE));
+        CUDA_TRY(c, ensure_scratch(c->d_envscratch, eslab * NLANE, env_warps, env_wpc));
         CUDA_TRY(c, fork_lanes(c, NLANE));
         int lane_rr = 0;
         for (int p = 0; p < P; p++) {

@@ -7,12 +7,15 @@ sharded run needs exactly three exchanges (SURVEY.md 8e):
   1. dereplication, hash-partitioned.  Reads are block-partitioned in input order.  Every rank dereplicates
      its block exactly; each LOCAL unique goes to the owner rank  key64 % G  as one 8-byte record
      (global read index | length << 32) plus its bases: two all-to-alls (records, bases) after one exchange of
-     the 2 G split sizes.  all_to_all delivers in source-rank order and blocks are contiguous, so the arrival
+     the split sizes.  all_to_all delivers in source-rank order and blocks are contiguous, so the arrival
      order IS ascending global read index: the owner's exact derep of what it received (every class verified
      base by base again) picks the global first occurrence without any sort.
   2. profile search.  The owner searches the classes it owns with the profiles replicated; the per-profile
      count of reported hits -- hmmsearch's domZ -- is all-reduced between stage 1 (scores, -T) and stage 2
-     (domE, ItsPosition arg-max).  The same all-reduce carries the number of classes per owner.
+     (domE, ItsPosition arg-max).  The same all-reduce carries the number of classes per owner.  An owner decides
+     in stage 1 which rows are printed whatever domZ turns out to be (the compact row mode); that needs a bound of
+     domZ over the whole sample, the sample's read count, which the split-size exchange of step 1 also carries (one
+     more column: every rank's block read count).
   3. answers.  One 16-byte record {representative's global index | strand << 31, start, stop, tlen} per received
      record returns through the inverse all-to-all; the block's position table (one row per local unique) is
      filled from it and the block is trimmed where it lies.  Rank order = input order.  No global table exists.
@@ -105,6 +108,7 @@ class GpuEngine:
         self.local, self.owner, self.params = local, owner, params
         self.dev = torch.device("cuda", int(local.device))
         self.n = self.nu = self.m = 0
+        self.n_reads_sample = 0
         self.resident = self.resident_qual = False
 
     def _p(self, t):
@@ -151,8 +155,18 @@ class GpuEngine:
                                                       int(bases.shape[0]), self.C.byref(n_own)))
         return int(n_own.value)
 
+    def sample_reads(self, n_reads):
+        """The sample's read count (run_sharded learns it in the split-size exchange).  It bounds any profile's domZ, so
+        params that leave domz_upper at 0 ("this context's sequence count", too small for an owner that searches a
+        share of the classes) get it in a copy in search_stage1; an explicit domz_upper is kept."""
+        self.n_reads_sample = int(n_reads)
+
     def search_stage1(self):
-        self.owner.search_stage1(self.params)
+        from ._lib import SearchParams, default_params
+        prm = default_params() if self.params is None else SearchParams.from_buffer_copy(self.params)
+        if prm.domz_upper == 0:
+            prm.domz_upper = self.n_reads_sample
+        self.owner.search_stage1(prm)
         return self.owner.nreported().astype(np.int64)
 
     def search_stage2(self, nrep_global):
@@ -206,6 +220,7 @@ def run_sharded(engine, comm, seq, off, first_global_index, phases=None, want_re
     local read (int64), strand, keep, lo, hi, n_unique_global, n_owned, nreported[, kept_index, out_off, out_seq,
     out_qual with gather=True; gather="device" leaves the slices in HBM and returns only n_kept / out_bytes]).  Results are identical to the single-GPU path on the concatenated input.
     phases: dict that receives the seconds spent per phase (PHASES), accumulated.
+    seq/off None: the engine's block is resident and its `n` is the block's read count.
     """
     G = comm.world
     t_last = [time.perf_counter()]
@@ -224,8 +239,12 @@ def run_sharded(engine, comm, seq, off, first_global_index, phases=None, want_re
     rec_counts, byte_counts = engine.plan(G)
     rec, bases = engine.pack(first_global_index, int(byte_counts.sum()))
     lap("plan_pack")
-    got = comm.exchange_counts(np.stack([rec_counts, byte_counts], axis=1))
+    # every rank also sends its block's read count: their sum is the sample's, which bounds any profile's domZ
+    n_block = len(off) - 1 if off is not None else engine.n
+    got = comm.exchange_counts(np.stack([rec_counts, byte_counts, np.full(G, n_block, np.int64)], axis=1))
     rrc, rbc = got[:, 0], got[:, 1]
+    if hasattr(engine, "sample_reads"):        # an engine that bounds domZ in stage 1 (GpuEngine's compact row mode)
+        engine.sample_reads(int(got[:, 2].sum()))
     rec_in = comm.all_to_all(rec, rec_counts, rrc, name="records")
     bases_in = comm.all_to_all(bases, byte_counts, rbc, name="bases")
     lap("exchange")
