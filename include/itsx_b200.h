@@ -205,15 +205,16 @@ int  itsx_trim_set_map(itsx_ctx *ctx, const int32_t *uid, int64_t nreads, int64_
  * (NULL: slice the dereplicated reads themselves).  Returns the number kept in *n_kept. */
 int  itsx_trim_bounds(itsx_ctx *ctx, int mode, const int64_t *off_other, int64_t nreads,
                       uint8_t *keep, int32_t *lo, int32_t *hi, int64_t *n_kept);
-/* gather the kept slices of (seq, qual) into back-to-back output buffers on the device and copy
- * them out: out_off[n_kept+1], out_seq/out_qual sized >= total (query with NULLs first via
- * *total).  seq/qual: the records being sliced (host), off: their offsets. */
+/* bounds + gather of the kept slices of (seq, qual) back to back on the device: *n_kept reads, *total bytes (either
+ * may be NULL).  seq/qual: the records being sliced, off: their offsets (host or device; the buffers are free again
+ * when the call returns).  NULL seq / off: the resident reads; NULL qual: the resident qualities when seq and off
+ * are NULL too (itsx_quals_upload), else bases only.  The slices stay on the device until the next trim, run or
+ * upload; itsx_run_fetch copies them out. */
 int  itsx_trim_gather(itsx_ctx *ctx, int mode, const uint8_t *seq, const uint8_t *qual, const int64_t *off,
-                      int64_t nreads, int64_t *n_kept, int64_t *total,
-                      int32_t *kept_index, int64_t *out_off, uint8_t *out_seq, uint8_t *out_qual);
+                      int64_t nreads, int64_t *n_kept, int64_t *total);
 
-/* the same for the RESIDENT reads (itsx_reads_upload / itsx_quals_upload, after itsx_search or itsx_shard_apply): the
- * gathered slices stay on the device; itsx_run_fetch copies them out */
+/* the same for all RESIDENT reads and their qualities, if uploaded (itsx_reads_upload / itsx_quals_upload, after
+ * itsx_search or itsx_shard_apply) */
 int  itsx_trim_gather_resident(itsx_ctx *ctx, int mode, int64_t *n_kept, int64_t *total);
 
 /* ---- paired-end merge (SURVEY 8f row 2) ------------------------------------------------------------------
@@ -303,7 +304,7 @@ int  itsx_run_trim(itsx_ctx *ctx, const uint8_t *seq, const uint8_t *qual, const
                    const itsx_search_params *prm, int32_t *rep_index, int32_t *kept_index, int64_t *out_off,
                    uint8_t *out_seq, uint8_t *out_qual, itsx_run_stats *st);
 /* the same with the reads already resident (itsx_reads_upload [+ itsx_quals_upload]): kernels only.  With the
- * qualities resident the run ends with the re-expansion and itsx_run_fetch copies its result out. */
+ * qualities resident the run ends with the re-expansion, which itsx_run_fetch copies out like that of itsx_trim_gather*. */
 int  itsx_reads_upload(itsx_ctx *ctx, const uint8_t *seq, const int64_t *off, int64_t nreads);
 int  itsx_quals_upload(itsx_ctx *ctx, const uint8_t *qual);      /* qual[off[nreads]] of the resident reads */
 /* Streamed upload -- a FASTQ file too large to sit parsed in host memory (BASELINE configs[3]: 70 GB of text) arrives in
@@ -315,10 +316,9 @@ int  itsx_quals_upload(itsx_ctx *ctx, const uint8_t *qual);      /* qual[off[nre
 int  itsx_reads_begin(itsx_ctx *ctx, int64_t nreads_hint, int64_t bases_hint);
 int  itsx_reads_append(itsx_ctx *ctx, const uint8_t *seq, const uint8_t *qual, const int64_t *off, int64_t nreads);
 int  itsx_reads_end(itsx_ctx *ctx, int64_t *nreads, int64_t *total_bases);
-/* ... and the chunked way out: keep filter + re-expansion of the resident reads [first, first + count) only (mode 0);
- * kept_index is relative to `first`.  Output buffers: worst case count / count + 1 / the range's bases. */
-int  itsx_trim_gather_range(itsx_ctx *ctx, int mode, int64_t first, int64_t count, int64_t *n_kept, int64_t *total,
-                            int32_t *kept_index, int64_t *out_off, uint8_t *out_seq, uint8_t *out_qual);
+/* ... and the chunked way out: itsx_trim_gather_resident over the resident reads [first, first + count) only (mode 0);
+ * the kept_index that itsx_run_fetch then returns is relative to `first`. */
+int  itsx_trim_gather_range(itsx_ctx *ctx, int mode, int64_t first, int64_t count, int64_t *n_kept, int64_t *total);
 /* Several samples in one pass (the loop over samples of q2_itsxpress.py:273-333 runs one vsearch and one hmmsearch PER
  * SAMPLE: classes never span samples and domZ is per sample): sample_of_read[nreads] in [0, n_samples) for the resident
  * reads, set before itsx_derep_resident.  The search then counts reported hits per (sample, profile) -- itsx_nreported /
@@ -329,6 +329,9 @@ int  itsx_reads_set_samples(itsx_ctx *ctx, const int32_t *sample_of_read, int32_
  * re-coding of the representatives for a context that will not search them (the block side of a sharded run) */
 int  itsx_derep_resident(itsx_ctx *ctx, int build_search_set, int64_t *n_unique);
 int  itsx_run_resident(itsx_ctx *ctx, const itsx_search_params *prm, itsx_run_stats *st);
+/* the slices of the last gather (itsx_trim_gather*, itsx_run_resident with qualities): kept_index[n_kept],
+ * out_off[n_kept + 1], out_seq / out_qual [total] (out_qual is left alone when no qualities were gathered).  Any may be
+ * NULL; ITSX_EINVAL when the last trim call gathered nothing. */
 int  itsx_run_fetch(itsx_ctx *ctx, int64_t *n_kept, int64_t *total, int32_t *kept_index, int64_t *out_off,
                     uint8_t *out_seq, uint8_t *out_qual);
 /* ---- clustering below 100 % identity: replaces `vsearch --cluster_size --id X --strand both` (SeqSample.py:133-176) ----
@@ -387,7 +390,7 @@ int64_t itsx_launch_count(const itsx_ctx *ctx);
  *   local:  itsx_reads_upload, itsx_derep_resident(0), itsx_shard_plan, itsx_shard_pack
  *   owner:  itsx_shard_owner_derep, itsx_search_stage1, [all-reduce nreported], itsx_nreported_set,
  *           itsx_search_stage2, itsx_shard_answers
- *   local:  itsx_shard_apply, itsx_trim_bounds / itsx_trim_gather */
+ *   local:  itsx_shard_apply, itsx_trim_bounds / itsx_trim_gather_resident + itsx_run_fetch */
 /* per destination rank g: records (local uniques owned by g) and their bases; one D2H of 2 G counters */
 int  itsx_shard_plan(itsx_ctx *local, int G, int64_t *rec_counts, int64_t *byte_counts);
 /* rec[n_unique_local]: (global read index of the unique's first read) | (length << 32), grouped by owner, ascending
@@ -409,7 +412,7 @@ int  itsx_shard_apply(itsx_ctx *local, const int32_t *ans, int64_t n_unique_loca
 /* ---- host-side FASTQ scanner / packer / formatter (multi-threaded C++, no GPU involved) -------------
  * Replace Biopython's SeqIO.parse / SeqIO.write on the path (SeqSample.py:746-757, 912-945): a decompressed
  * 4-line FASTQ buffer -> offset arrays (title after '@' right-stripped, sequence, quality), packed byte
- * streams for itsx_derep / itsx_trim_*, and FASTQ text from the slices itsx_trim_gather returns. */
+ * streams for itsx_derep / itsx_trim_*, and FASTQ text from the slices itsx_run_fetch returns. */
 const char *itsx_host_last_error(void);
 /* cap == 0: count records only.  Returns the record count or ITSX_EFORMAT / ITSX_EINVAL. */
 int64_t itsx_fastq_index(const uint8_t *buf, int64_t nbytes, int64_t cap, int64_t *t_off, int32_t *t_len,

@@ -174,7 +174,7 @@ def lib():
     L.itsx_positions_set.argtypes = [vp, vp, vp, vp, i64]
     L.itsx_trim_set_map.argtypes = [vp, vp, i64, i64]
     L.itsx_trim_bounds.argtypes = [vp, C.c_int, vp, i64, vp, vp, vp, vp]
-    L.itsx_trim_gather.argtypes = [vp, C.c_int, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp]
+    L.itsx_trim_gather.argtypes = [vp, C.c_int, vp, vp, vp, i64, vp, vp]
     L.itsx_run.argtypes = [vp, vp, vp, i64, C.POINTER(SearchParams), vp, vp, vp, vp, C.POINTER(RunStats)]
     L.itsx_reads_upload.argtypes = [vp, vp, vp, i64]
     L.itsx_run_resident.argtypes = [vp, C.POINTER(SearchParams), C.POINTER(RunStats)]
@@ -185,7 +185,7 @@ def lib():
     L.itsx_reads_begin.argtypes = [vp, i64, i64]
     L.itsx_reads_append.argtypes = [vp, vp, vp, vp, i64]
     L.itsx_reads_end.argtypes = [vp, vp, vp]
-    L.itsx_trim_gather_range.argtypes = [vp, C.c_int, i64, i64, vp, vp, vp, vp, vp, vp]
+    L.itsx_trim_gather_range.argtypes = [vp, C.c_int, i64, i64, vp, vp]
     L.itsx_trim_gather_resident.argtypes = [vp, C.c_int, vp, vp]
     L.itsx_run_trim.argtypes = [vp, vp, vp, vp, i64, C.POINTER(SearchParams), vp, vp, vp, vp, vp, C.POINTER(RunStats)]
     L.itsx_quals_upload.argtypes = [vp, vp]
@@ -523,22 +523,20 @@ class Context:
         self._chk(lib().itsx_trim_bounds(self._h, mode, _p(o), nreads, _p(keep), _p(lo), _p(hi), C.byref(nk)))
         return keep, lo, hi, int(nk.value)
 
-    def trim_gather(self, nreads, mode=0, seq=None, qual=None, off=None, resident_qual=False):
-        """Returns (kept_index, out_off, out_seq, out_qual) with the slices packed back to back.  resident_qual: the
-        qualities of the resident reads were uploaded with quals_upload()."""
+    def trim_gather(self, nreads, mode=0, seq=None, qual=None, off=None):
+        """Returns (kept_index, out_off, out_seq, out_qual) with the slices packed back to back; out_qual is None
+        without qual."""
         nk, tot = C.c_int64(), C.c_int64()
         seq = None if seq is None else np.ascontiguousarray(seq, dtype=np.uint8)
         qual = None if qual is None else np.ascontiguousarray(qual, dtype=np.uint8)
         off = None if off is None else np.ascontiguousarray(off, dtype=np.int64)
         L = lib()
-        self._chk(L.itsx_trim_gather(self._h, mode, _p(seq), _p(qual), _p(off), nreads, C.byref(nk), C.byref(tot),
-                                     None, None, None, None))
+        self._chk(L.itsx_trim_gather(self._h, mode, _p(seq), _p(qual), _p(off), nreads, C.byref(nk), C.byref(tot)))
         ki = np.empty(nk.value, np.int32)
         oo = np.empty(nk.value + 1, np.int64)
         os_ = np.empty(tot.value, np.uint8)
-        oq = np.empty(tot.value, np.uint8) if (qual is not None or resident_qual) else None
-        self._chk(L.itsx_trim_gather(self._h, mode, _p(seq), _p(qual), _p(off), nreads, C.byref(nk), C.byref(tot),
-                                     _p(ki), _p(oo), _p(os_), _p(oq)))
+        oq = np.empty(tot.value, np.uint8) if qual is not None else None
+        self._chk(L.itsx_run_fetch(self._h, None, None, _p(ki), _p(oo), _p(os_), _p(oq)))
         return ki, oo, os_, oq
 
     # ---- gzip writer ----------------------------------------------------------------------------
@@ -620,12 +618,9 @@ class Context:
     def trim_gather_range(self, first, count, nbases, mode=0):
         """(kept_index relative to first, out_off, out_seq, out_qual) of the resident reads [first, first + count);
         nbases = bases of the range (worst-case output size)."""
-        nk, tot = C.c_int64(), C.c_int64()
-        ki, oo = np.empty(count, np.int32), np.empty(count + 1, np.int64)
-        os_, oq = np.empty(nbases, np.uint8), np.empty(nbases, np.uint8)
-        self._chk(lib().itsx_trim_gather_range(self._h, mode, int(first), int(count), C.byref(nk), C.byref(tot), _p(ki),
-                                               _p(oo), _p(os_), _p(oq)))
-        return ki[:nk.value], oo[:nk.value + 1], os_[:tot.value], oq[:tot.value]
+        self._chk(lib().itsx_trim_gather_range(self._h, mode, int(first), int(count), None, None))
+        return self.run_fetch(dict(kept_index=np.empty(count, np.int32), out_off=np.empty(count + 1, np.int64),
+                                   out_seq=np.empty(nbases, np.uint8), out_qual=np.empty(nbases, np.uint8)))
 
     def quals_upload(self, qual):
         qual = np.ascontiguousarray(qual, dtype=np.uint8)
@@ -665,16 +660,17 @@ class Context:
         return int(nk.value), int(tot.value)
 
     def run_fetch(self, out=None):
-        """Gathered slices left on the device by run_resident() / trim_gather_resident().  out: preallocated (pinned)
-        arrays kept_index / out_off / out_seq / out_qual of worst-case size; the returned views are cut to size."""
+        """Gathered slices left on the device by run_resident() / trim_gather_resident() / trim_gather_range().  out:
+        preallocated (pinned) arrays kept_index / out_off / out_seq / out_qual of worst-case size; the returned views
+        are cut to size."""
         nk, tot = C.c_int64(), C.c_int64()
         L = lib()
-        self._chk(L.itsx_run_fetch(self._h, C.byref(nk), C.byref(tot), None, None, None, None))
         if out is None:
+            self._chk(L.itsx_run_fetch(self._h, C.byref(nk), C.byref(tot), None, None, None, None))
             out = dict(kept_index=np.empty(nk.value, np.int32), out_off=np.empty(nk.value + 1, np.int64),
                        out_seq=np.empty(tot.value, np.uint8), out_qual=np.empty(tot.value, np.uint8))
-        self._chk(L.itsx_run_fetch(self._h, None, None, _p(out["kept_index"]), _p(out["out_off"]), _p(out["out_seq"]),
-                                   _p(out["out_qual"])))
+        self._chk(L.itsx_run_fetch(self._h, C.byref(nk), C.byref(tot), _p(out["kept_index"]), _p(out["out_off"]),
+                                   _p(out["out_seq"]), _p(out["out_qual"])))
         return (out["kept_index"][:nk.value], out["out_off"][:nk.value + 1], out["out_seq"][:tot.value],
                 out["out_qual"][:tot.value])
 

@@ -173,17 +173,7 @@ int itsx_reads_upload(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64
     if (nreads < 0 || (nreads > 0 && (!seq || !off))) { c->err = "reads_upload: null buffer"; return ITSX_EINVAL; }
     const int64_t total = nreads ? itsx_peek_i64(off + nreads) : 0;
     if (nreads && itsx_peek_i64(off) != 0) { c->err = "reads_upload: off[0] must be 0"; return ITSX_EINVAL; }
-    c->nreads = nreads;
-    c->total_bases = total;
-    c->n_unique = 0;
-    c->cl_active = false;
-    c->map_external = false;
-    c->pos_valid = false;
-    c->qual_resident = false;
-    c->r_gathered = false;
-    c->have_samples = false;
-    c->n_samples = 1;
-    c->stream_open = false;
+    reset_reads(c, nreads, total);
     const size_t padded = ((size_t)total + 15) / 16 * 16 + 32;
     CUDA_TRY(c, c->d_ascii.ensure(padded));
     CUDA_TRY(c, c->d_off.ensure((size_t)(nreads + 1) * 8));
@@ -220,16 +210,7 @@ int itsx_reads_begin(itsx_ctx *c, int64_t nreads_hint, int64_t bases_hint)
 {
     CHECK_CTX(c);
     CUDA_TRY(c, cudaSetDevice(c->device));
-    c->nreads = 0;
-    c->total_bases = 0;
-    c->n_unique = 0;
-    c->cl_active = false;
-    c->map_external = false;
-    c->pos_valid = false;
-    c->qual_resident = false;
-    c->r_gathered = false;
-    c->have_samples = false;
-    c->n_samples = 1;
+    reset_reads(c, 0, 0);
     c->stream_open = true;
     c->stream_qual = true;
     c->stream_reads = c->stream_bases = 0;
@@ -254,8 +235,6 @@ int itsx_reads_append(itsx_ctx *c, const uint8_t *seq, const uint8_t *qual, cons
     // (DevBuf grows geometrically and keeps what is there)
     CUDA_TRY(c, c->d_ascii.ensure((size_t)(c->stream_bases + nb) + 64, true, st));
     CUDA_TRY(c, c->d_off.ensure((size_t)(c->stream_reads + nreads + 1) * 8, true, st));
-    static thread_local DevBuf t_off;
-    CUDA_TRY(c, t_off.ensure((size_t)(nreads + 1) * 8));
     CUDA_TRY(c, cudaMemcpyAsync(c->d_ascii.as<uint8_t>() + c->stream_bases, seq, (size_t)nb, cudaMemcpyDefault, st));
     if (qual && c->stream_qual) {
         CUDA_TRY(c, c->d_qual.ensure((size_t)(c->stream_bases + nb) + 64, true, st));
@@ -263,8 +242,8 @@ int itsx_reads_append(itsx_ctx *c, const uint8_t *seq, const uint8_t *qual, cons
     } else {
         c->stream_qual = false;
     }
-    CUDA_TRY(c, cudaMemcpyAsync(t_off.p, off, (size_t)(nreads + 1) * 8, cudaMemcpyDefault, st));
-    offset_append_kernel<<<(unsigned)((nreads + 256) / 256), 256, 0, st>>>(t_off.as<int64_t>(), nreads, c->stream_bases,
+    CUDA_TRY(c, stage(c, c->d_stage_off, off, (size_t)(nreads + 1) * 8, 0));
+    offset_append_kernel<<<(unsigned)((nreads + 256) / 256), 256, 0, st>>>(c->d_stage_off.as<int64_t>(), nreads, c->stream_bases,
                                                                            c->d_off.as<int64_t>() + c->stream_reads);
     c->launches++;
     c->stream_reads += nreads;
@@ -292,39 +271,6 @@ int itsx_reads_end(itsx_ctx *c, int64_t *nreads, int64_t *total_bases)
     c->stream_open = false;
     if (nreads) *nreads = c->nreads;
     if (total_bases) *total_bases = total;
-    return ITSX_OK;
-}
-
-/* re-expansion of the resident reads [first, first + count): what a chunked writer asks for, chunk after chunk */
-int itsx_trim_gather_range(itsx_ctx *c, int mode, int64_t first, int64_t count, int64_t *n_kept, int64_t *total,
-                           int32_t *kept_index, int64_t *out_off, uint8_t *out_seq, uint8_t *out_qual)
-{
-    CHECK_CTX(c);
-    CUDA_TRY(c, cudaSetDevice(c->device));
-    if (c->stream_open) { c->err = "trim: a streamed upload is still open (itsx_reads_end)"; return ITSX_EINVAL; }
-    if (mode != 0) { c->err = "trim_gather_range: only mode 0 (the dereplicated reads themselves)"; return ITSX_EINVAL; }
-    if (c->map_external) { c->err = "trim_gather_range: no reads are resident"; return ITSX_EINVAL; }
-    if (c->npos != map_rows(c)) { c->err = "trim: position table does not cover every unique sequence"; return ITSX_EINVAL; }
-    if (first < 0 || count < 0 || first + count > c->nreads) { c->err = "trim_gather_range: range outside the reads"; return ITSX_EINVAL; }
-    if (!n_kept || !total) return ITSX_EINVAL;
-    cudaStream_t st = c->stream;
-    CUDA_TRY(c, c->r_keep.ensure((size_t)count + 16));
-    CUDA_TRY(c, c->r_lo.ensure((size_t)count * 4 + 16));
-    CUDA_TRY(c, c->r_hi.ensure((size_t)count * 4 + 16));
-    int64_t nk = 0;
-    int rc = trim_bounds_dev(c, 0, nullptr, count, c->r_keep.as<uint8_t>(), c->r_lo.as<int32_t>(), c->r_hi.as<int32_t>(), &nk,
-                             first);
-    if (rc) return rc;
-    rc = trim_gather_dev(c, c->d_ascii.as<uint8_t>(), c->qual_resident ? c->d_qual.as<uint8_t>() : nullptr,
-                         c->d_off.as<int64_t>() + first, count, c->r_keep.as<uint8_t>(), c->r_lo.as<int32_t>(),
-                         c->r_hi.as<int32_t>(), n_kept, total, c->r_ki, c->r_oo, c->r_os, c->r_oq);
-    if (rc) return rc;
-    c->r_gathered = false;
-    if (kept_index && *n_kept) CUDA_TRY(c, cudaMemcpyAsync(kept_index, c->r_ki.p, (size_t)*n_kept * 4, cudaMemcpyDefault, st));
-    if (out_off) CUDA_TRY(c, cudaMemcpyAsync(out_off, c->r_oo.p, (size_t)(*n_kept + 1) * 8, cudaMemcpyDefault, st));
-    if (out_seq && *total) CUDA_TRY(c, cudaMemcpyAsync(out_seq, c->r_os.p, (size_t)*total, cudaMemcpyDefault, st));
-    if (out_qual && *total && c->qual_resident) CUDA_TRY(c, cudaMemcpyAsync(out_qual, c->r_oq.p, (size_t)*total, cudaMemcpyDefault, st));
-    CUDA_TRY(c, cudaStreamSynchronize(st));
     return ITSX_OK;
 }
 
@@ -635,10 +581,10 @@ int itsx_trim_set_map(itsx_ctx *c, const int32_t *uid, int64_t nreads, int64_t n
     CUDA_TRY(c, c->d_uid.ensure((size_t)std::max<int64_t>(nreads, 1) * 4));
     if (nreads) CUDA_TRY(c, cudaMemcpyAsync(c->d_uid.p, uid, (size_t)nreads * 4, cudaMemcpyDefault, c->stream));
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
-    c->nreads = nreads;
+    const bool pos_valid = c->pos_valid;       // a position table installed before the map stays (include/itsx_b200.h)
+    reset_reads(c, nreads, 0);                 // no resident read bytes: itsx_trim_* must be given seq/qual/off
+    c->pos_valid = pos_valid;
     c->n_unique = n_unique;
-    c->cl_active = false;
-    c->total_bases = 0;       // no resident read bytes: itsx_trim_* must be given seq/qual/off
     c->map_external = true;
     return ITSX_OK;
 }
@@ -660,118 +606,79 @@ int itsx_trim_bounds(itsx_ctx *c, int mode, const int64_t *off_other, int64_t nr
     int rc = check_trim(c, mode, nreads);
     if (rc) return rc;
     if (c->map_external && !off_other) { c->err = "trim: offsets are required after itsx_trim_set_map"; return ITSX_EINVAL; }
-    static thread_local DevBuf t_off, t_keep, t_lo, t_hi;
-    CUDA_TRY(c, t_keep.ensure((size_t)nreads + 16));
-    CUDA_TRY(c, t_lo.ensure((size_t)nreads * 4 + 16));
-    CUDA_TRY(c, t_hi.ensure((size_t)nreads * 4 + 16));
-    const int64_t *d_off = nullptr;
-    if (off_other) {
-        CUDA_TRY(c, t_off.ensure((size_t)(nreads + 1) * 8));
-        CUDA_TRY(c, cudaMemcpyAsync(t_off.p, off_other, (size_t)(nreads + 1) * 8, cudaMemcpyDefault, c->stream));
-        d_off = t_off.as<int64_t>();
-    }
-    rc = trim_bounds_dev(c, mode, d_off, nreads, t_keep.as<uint8_t>(), t_lo.as<int32_t>(), t_hi.as<int32_t>(), n_kept);
+    if (off_other) CUDA_TRY(c, stage(c, c->d_stage_off, off_other, (size_t)(nreads + 1) * 8, 0));
+    rc = trim_bounds_dev(c, mode, off_other ? c->d_stage_off.as<int64_t>() : nullptr, 0, nreads);
     if (rc) return rc;
+    if (n_kept) *n_kept = c->r_nkept;
     if (nreads) {
-        if (keep) CUDA_TRY(c, cudaMemcpyAsync(keep, t_keep.p, (size_t)nreads, cudaMemcpyDefault, c->stream));
-        if (lo) CUDA_TRY(c, cudaMemcpyAsync(lo, t_lo.p, (size_t)nreads * 4, cudaMemcpyDefault, c->stream));
-        if (hi) CUDA_TRY(c, cudaMemcpyAsync(hi, t_hi.p, (size_t)nreads * 4, cudaMemcpyDefault, c->stream));
+        if (keep) CUDA_TRY(c, cudaMemcpyAsync(keep, c->r_keep.p, (size_t)nreads, cudaMemcpyDefault, c->stream));
+        if (lo) CUDA_TRY(c, cudaMemcpyAsync(lo, c->r_lo.p, (size_t)nreads * 4, cudaMemcpyDefault, c->stream));
+        if (hi) CUDA_TRY(c, cudaMemcpyAsync(hi, c->r_hi.p, (size_t)nreads * 4, cudaMemcpyDefault, c->stream));
         CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     }
     return ITSX_OK;
 }
 
 int itsx_trim_gather(itsx_ctx *c, int mode, const uint8_t *seq, const uint8_t *qual, const int64_t *off,
-                     int64_t nreads, int64_t *n_kept, int64_t *total,
-                     int32_t *kept_index, int64_t *out_off, uint8_t *out_seq, uint8_t *out_qual)
+                     int64_t nreads, int64_t *n_kept, int64_t *total)
 {
     CHECK_CTX(c);
     CUDA_TRY(c, cudaSetDevice(c->device));
     int rc = check_trim(c, mode, nreads);
     if (rc) return rc;
-    if (!n_kept || !total) return ITSX_EINVAL;
     if (c->map_external && !off) { c->err = "trim: offsets are required after itsx_trim_set_map"; return ITSX_EINVAL; }
-    if (c->map_external && !seq && (out_seq || out_off || kept_index)) {
-        c->err = "trim: sequence bytes are required after itsx_trim_set_map";
-        return ITSX_EINVAL;
-    }
-    static thread_local DevBuf t_off, t_seq, t_qual, t_keep, t_lo, t_hi, t_ki, t_oo, t_os, t_oq;
-    cudaStream_t st = c->stream;
-    const bool query = !out_seq && !out_off && !kept_index;
-    CUDA_TRY(c, t_keep.ensure((size_t)nreads + 16));
-    CUDA_TRY(c, t_lo.ensure((size_t)nreads * 4 + 16));
-    CUDA_TRY(c, t_hi.ensure((size_t)nreads * 4 + 16));
-    const int64_t *d_off = nullptr;
-    const int64_t tot_in = (off && nreads) ? itsx_peek_i64(off + nreads) : 0;
-    if (off) {
-        CUDA_TRY(c, t_off.ensure((size_t)(nreads + 1) * 8));
-        CUDA_TRY(c, cudaMemcpyAsync(t_off.p, off, (size_t)(nreads + 1) * 8, cudaMemcpyDefault, st));
-        d_off = t_off.as<int64_t>();
-    }
-    int64_t nk = 0;
-    rc = trim_bounds_dev(c, mode, d_off, nreads, t_keep.as<uint8_t>(), t_lo.as<int32_t>(), t_hi.as<int32_t>(), &nk);
+    if (c->map_external && !seq) { c->err = "trim: sequence bytes are required after itsx_trim_set_map"; return ITSX_EINVAL; }
+    const int64_t bases = (off && nreads) ? itsx_peek_i64(off + nreads) : 0;
+    if (off) CUDA_TRY(c, stage(c, c->d_stage_off, off, (size_t)(nreads + 1) * 8, 0));
+    rc = trim_bounds_dev(c, mode, off ? c->d_stage_off.as<int64_t>() : nullptr, 0, nreads);
     if (rc) return rc;
-    if (query) {
-        int64_t tot = 0;
-        if (nreads) {
-            CUDA_TRY(c, cudaMemcpyAsync(&tot, c->d_list2.as<int64_t>() + nreads, 8, cudaMemcpyDefault, st));
-            CUDA_TRY(c, cudaStreamSynchronize(st));
-        }
-        *n_kept = nk;
-        *total = tot;
-        return ITSX_OK;
-    }
     const uint8_t *d_seq = c->d_ascii.as<uint8_t>();
     const uint8_t *d_qual = nullptr;
     if (seq) {
-        CUDA_TRY(c, t_seq.ensure((size_t)tot_in + 16));
-        if (tot_in) CUDA_TRY(c, cudaMemcpyAsync(t_seq.p, seq, (size_t)tot_in, cudaMemcpyDefault, st));
-        d_seq = t_seq.as<uint8_t>();
+        CUDA_TRY(c, stage(c, c->d_stage_seq, seq, (size_t)bases, 16));
+        d_seq = c->d_stage_seq.as<uint8_t>();
     }
     if (qual) {
-        const int64_t tq = off ? tot_in : c->total_bases;
-        CUDA_TRY(c, t_qual.ensure((size_t)tq + 16));
-        if (tq) CUDA_TRY(c, cudaMemcpyAsync(t_qual.p, qual, (size_t)tq, cudaMemcpyDefault, st));
-        d_qual = t_qual.as<uint8_t>();
+        CUDA_TRY(c, stage(c, c->d_stage_qual, qual, (size_t)(off ? bases : c->total_bases), 16));
+        d_qual = c->d_stage_qual.as<uint8_t>();
     } else if (!seq && !off && c->qual_resident) {
         d_qual = c->d_qual.as<uint8_t>();       // qualities of the resident reads (itsx_quals_upload)
     }
-    rc = trim_gather_dev(c, d_seq, d_qual, d_off ? d_off : c->d_off.as<int64_t>(), nreads, t_keep.as<uint8_t>(),
-                         t_lo.as<int32_t>(), t_hi.as<int32_t>(), n_kept, total, t_ki, t_oo, t_os, t_oq);
+    rc = trim_gather_dev(c, d_seq, d_qual);
     if (rc) return rc;
-    if (kept_index && *n_kept) CUDA_TRY(c, cudaMemcpyAsync(kept_index, t_ki.p, (size_t)*n_kept * 4, cudaMemcpyDefault, st));
-    if (out_off) CUDA_TRY(c, cudaMemcpyAsync(out_off, t_oo.p, (size_t)(*n_kept + 1) * 8, cudaMemcpyDefault, st));
-    if (out_seq && *total) CUDA_TRY(c, cudaMemcpyAsync(out_seq, t_os.p, (size_t)*total, cudaMemcpyDefault, st));
-    if (out_qual && d_qual && *total) CUDA_TRY(c, cudaMemcpyAsync(out_qual, t_oq.p, (size_t)*total, cudaMemcpyDefault, st));
-    CUDA_TRY(c, cudaStreamSynchronize(st));
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));      // the caller's buffers are free again
+    if (n_kept) *n_kept = c->r_nkept;
+    if (total) *total = c->r_total;
     return ITSX_OK;
+}
+
+static int gather_resident(itsx_ctx *c, int mode, int64_t first, int64_t count, int64_t *n_kept, int64_t *total)
+{
+    CHECK_CTX(c);
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    int rc = check_trim(c, mode, c->nreads);
+    if (rc) return rc;
+    if (c->map_external) { c->err = "trim: no reads are resident (itsx_reads_upload first)"; return ITSX_EINVAL; }
+    rc = trim_bounds_dev(c, mode, nullptr, first, count);
+    if (rc) return rc;
+    rc = trim_gather_dev(c, c->d_ascii.as<uint8_t>(), c->qual_resident ? c->d_qual.as<uint8_t>() : nullptr);
+    if (rc) return rc;
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    if (n_kept) *n_kept = c->r_nkept;
+    if (total) *total = c->r_total;
+    return ITSX_OK;
+}
+
+/* re-expansion of the resident reads [first, first + count): what a chunked writer asks for, chunk after chunk */
+int itsx_trim_gather_range(itsx_ctx *c, int mode, int64_t first, int64_t count, int64_t *n_kept, int64_t *total)
+{
+    if (c && mode != 0) { c->err = "trim_gather_range: only mode 0 (the dereplicated reads themselves)"; return ITSX_EINVAL; }
+    return gather_resident(c, mode, first, count, n_kept, total);
 }
 
 int itsx_trim_gather_resident(itsx_ctx *c, int mode, int64_t *n_kept, int64_t *total)
 {
-    CHECK_CTX(c);
-    CUDA_TRY(c, cudaSetDevice(c->device));
-    const int64_t n = c->nreads;
-    int rc = check_trim(c, mode, n);
-    if (rc) return rc;
-    if (c->map_external) { c->err = "trim_gather_resident: no reads are resident"; return ITSX_EINVAL; }
-    CUDA_TRY(c, c->r_keep.ensure((size_t)n + 16));
-    CUDA_TRY(c, c->r_lo.ensure((size_t)n * 4 + 16));
-    CUDA_TRY(c, c->r_hi.ensure((size_t)n * 4 + 16));
-    int64_t nk = 0, nk2 = 0, tot = 0;
-    rc = trim_bounds_dev(c, mode, nullptr, n, c->r_keep.as<uint8_t>(), c->r_lo.as<int32_t>(), c->r_hi.as<int32_t>(), &nk);
-    if (rc) return rc;
-    rc = trim_gather_dev(c, c->d_ascii.as<uint8_t>(), c->qual_resident ? c->d_qual.as<uint8_t>() : nullptr,
-                         c->d_off.as<int64_t>(), n, c->r_keep.as<uint8_t>(), c->r_lo.as<int32_t>(), c->r_hi.as<int32_t>(),
-                         &nk2, &tot, c->r_ki, c->r_oo, c->r_os, c->r_oq);
-    if (rc) return rc;
-    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
-    c->r_nkept = nk2;
-    c->r_total = tot;
-    c->r_gathered = true;
-    if (n_kept) *n_kept = nk2;
-    if (total) *total = tot;
-    return ITSX_OK;
+    return gather_resident(c, mode, 0, c ? c->nreads : 0, n_kept, total);
 }
 
 // ---- whole path ------------------------------------------------------------------------------------------
@@ -797,36 +704,18 @@ static int run_device_part(itsx_ctx *c, const itsx_search_params *prm, itsx_run_
     rc = search_stage2(c);
     if (rc) return rc;
     CUDA_TRY(c, tl.record(3, st));
-    const int64_t n = c->nreads;
-    CUDA_TRY(c, c->r_keep.ensure((size_t)n + 16));
-    CUDA_TRY(c, c->r_lo.ensure((size_t)n * 4 + 16));
-    CUDA_TRY(c, c->r_hi.ensure((size_t)n * 4 + 16));
-    int64_t nk = 0;
-    rc = trim_bounds_dev(c, 0, nullptr, n, c->r_keep.as<uint8_t>(), c->r_lo.as<int32_t>(), c->r_hi.as<int32_t>(), &nk);
+    rc = trim_bounds_dev(c, 0, nullptr, 0, c->nreads);
     if (rc) return rc;
     CUDA_TRY(c, tl.record(4, st));
-    rs->n_reads = n;
-    rs->n_unique = c->n_unique;
-    rs->n_kept = nk;
-    c->r_nkept = nk;
-    c->r_total = 0;
-    c->r_gathered = false;
-    if (n) {
-        int64_t tot = 0;
-        CUDA_TRY(c, cudaMemcpyAsync(&tot, c->d_list2.as<int64_t>() + n, 8, cudaMemcpyDefault, st));
-        CUDA_TRY(c, cudaStreamSynchronize(st));
-        rs->out_bytes = tot;
-        c->r_total = tot;
-    }
     if (c->qual_resident) {
-        int64_t nk2 = 0, tot2 = 0;
-        rc = trim_gather_dev(c, c->d_ascii.as<uint8_t>(), c->d_qual.as<uint8_t>(), c->d_off.as<int64_t>(), n,
-                             c->r_keep.as<uint8_t>(), c->r_lo.as<int32_t>(), c->r_hi.as<int32_t>(), &nk2, &tot2,
-                             c->r_ki, c->r_oo, c->r_os, c->r_oq);
+        rc = trim_gather_dev(c, c->d_ascii.as<uint8_t>(), c->d_qual.as<uint8_t>());
         if (rc) return rc;
-        c->r_gathered = true;
     }
     CUDA_TRY(c, tl.record(6, st));
+    rs->n_reads = c->nreads;
+    rs->n_unique = c->n_unique;
+    rs->n_kept = c->r_nkept;
+    rs->out_bytes = c->r_total;
     return ITSX_OK;
 }
 
@@ -905,16 +794,12 @@ int itsx_run_fetch(itsx_ctx *c, int64_t *n_kept, int64_t *total, int32_t *kept_i
 {
     CHECK_CTX(c);
     CUDA_TRY(c, cudaSetDevice(c->device));
-    if (!c->r_gathered) { c->err = "run_fetch: no gathered output is resident (qualities were not uploaded)"; return ITSX_EINVAL; }
-    cudaStream_t st = c->stream;
-    const int64_t nk = c->r_nkept, tot = c->r_total;
-    if (n_kept) *n_kept = nk;
-    if (total) *total = tot;
-    if (kept_index && nk) CUDA_TRY(c, cudaMemcpyAsync(kept_index, c->r_ki.p, (size_t)nk * 4, cudaMemcpyDefault, st));
-    if (out_off) CUDA_TRY(c, cudaMemcpyAsync(out_off, c->r_oo.p, (size_t)(nk + 1) * 8, cudaMemcpyDefault, st));
-    if (out_seq && tot) CUDA_TRY(c, cudaMemcpyAsync(out_seq, c->r_os.p, (size_t)tot, cudaMemcpyDefault, st));
-    if (out_qual && tot && c->qual_resident) CUDA_TRY(c, cudaMemcpyAsync(out_qual, c->r_oq.p, (size_t)tot, cudaMemcpyDefault, st));
-    CUDA_TRY(c, cudaStreamSynchronize(st));
+    if (!c->r_gathered) { c->err = "run_fetch: no gathered output is resident (nothing gathered since the last trim bounds)"; return ITSX_EINVAL; }
+    if (n_kept) *n_kept = c->r_nkept;
+    if (total) *total = c->r_total;
+    int rc = trim_fetch_dev(c, kept_index, out_off, out_seq, out_qual);
+    if (rc) return rc;
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     return ITSX_OK;
 }
 
@@ -933,13 +818,9 @@ int itsx_run_trim(itsx_ctx *c, const uint8_t *seq, const uint8_t *qual, const in
     int rc = itsx_reads_upload(c, seq, off, nreads);
     if (!rc) rc = itsx_quals_upload(c, qual);
     if (!rc) rc = run_device_part(c, prm, &rs, tl);
+    if (!rc && rep_index && nreads) CUDA_TRY(c, cudaMemcpyAsync(rep_index, c->d_rep.p, (size_t)nreads * 4, cudaMemcpyDefault, st));
+    if (!rc) rc = trim_fetch_dev(c, kept_index, out_off, out_seq, out_qual);
     if (!rc) {
-        const int64_t nk = c->r_nkept, tot = c->r_total;
-        if (rep_index && nreads) CUDA_TRY(c, cudaMemcpyAsync(rep_index, c->d_rep.p, (size_t)nreads * 4, cudaMemcpyDefault, st));
-        if (kept_index && nk) CUDA_TRY(c, cudaMemcpyAsync(kept_index, c->r_ki.p, (size_t)nk * 4, cudaMemcpyDefault, st));
-        if (out_off) CUDA_TRY(c, cudaMemcpyAsync(out_off, c->r_oo.p, (size_t)(nk + 1) * 8, cudaMemcpyDefault, st));
-        if (out_seq && tot) CUDA_TRY(c, cudaMemcpyAsync(out_seq, c->r_os.p, (size_t)tot, cudaMemcpyDefault, st));
-        if (out_qual && tot) CUDA_TRY(c, cudaMemcpyAsync(out_qual, c->r_oq.p, (size_t)tot, cudaMemcpyDefault, st));
         CUDA_TRY(c, tl.record(5, st));
         CUDA_TRY(c, cudaStreamSynchronize(st));
         run_times(rs, tl, true);

@@ -185,14 +185,21 @@ struct itsx_ctx {
     itsx_merge_params mg_tabs_prm{};
     itsx_merge_stats mgstats{};
 
-    // whole-path calls (itsx_run*): qualities of the resident reads, bounds and gathered slices of the last run
+    // qualities of the resident reads (itsx_quals_upload, a streamed upload with qualities)
     DevBuf d_qual;
-    bool qual_resident = false, r_gathered = false;
+    bool qual_resident = false;
     // streamed upload (itsx_reads_begin / append / end): reads and bases appended so far, every chunk brought qualities
     bool stream_open = false, stream_qual = false;
     int64_t stream_reads = 0, stream_bases = 0;
+    // trim (trim.cu): keep / lo / hi of the last trim_bounds_dev over r_n reads with offsets r_off, its kept count and
+    // output bytes; the slices of the last trim_gather_dev (r_gathered; r_gathered_qual: qualities too)
     DevBuf r_keep, r_lo, r_hi, r_ki, r_oo, r_os, r_oq, d_gather;
-    int64_t r_nkept = 0, r_total = 0;
+    const int64_t *r_off = nullptr;
+    int64_t r_n = 0, r_nkept = 0, r_total = 0;
+    bool r_gathered = false, r_gathered_qual = false;
+    // caller-supplied bytes staged for the length of one call (records of itsx_trim_*, sequences of itsx_search_seqs, chunk
+    // offsets of itsx_reads_append): apart from d_ascii / d_off / d_qual so that the resident reads survive
+    DevBuf d_stage_seq, d_stage_qual, d_stage_off;
 
     // one sample sharded over G GPUs (shard.cu): bucket order of the block's uniques, scratch, send / receive staging
     int sh_G = 0;
@@ -304,6 +311,31 @@ __device__ __forceinline__ void warp_copy(const uint8_t *__restrict__ src, uint8
 // rows of the position table the resident read -> row map (d_uid) points into: centroids after itsx_cluster, else classes
 inline int64_t map_rows(const itsx_ctx *c) { return c->cl_active ? c->cl_ncent : c->n_unique; }
 
+// a new read set (nreads reads, total_bases bases) replaces the resident one: nothing derived from the old set stays valid
+// -- derep, clustering, positions, qualities, trim output, sample ids, an open streamed upload
+inline void reset_reads(itsx_ctx *c, int64_t nreads, int64_t total_bases)
+{
+    c->nreads = nreads;
+    c->total_bases = total_bases;
+    c->n_unique = 0;
+    c->cl_active = false;
+    c->map_external = false;
+    c->pos_valid = false;
+    c->qual_resident = false;
+    c->r_gathered = false;
+    c->have_samples = false;
+    c->n_samples = 1;
+    c->stream_open = false;
+}
+
+// bytes of a caller buffer (host or device) -> b, grown to bytes + pad, on c->stream
+inline cudaError_t stage(itsx_ctx *c, DevBuf &b, const void *src, size_t bytes, size_t pad)
+{
+    cudaError_t e = b.ensure(bytes + pad);
+    if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyDefault, c->stream);
+    return e;
+}
+
 // stage entry points (implemented in derep.cu / search.cu / trim.cu / cluster.cu)
 int derep_run(itsx_ctx *c);                                   // reads already in d_ascii/d_off
 int cluster_run(itsx_ctx *c, const itsx_cluster_params *prm, const int32_t *order, int64_t *n_centroids);
@@ -314,9 +346,10 @@ int search_build_seqs_from_derep(itsx_ctx *c);                // uniques -> d_se
 int search_build_seqs_from_host(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64_t nseq);
 int search_stage1(itsx_ctx *c);
 int search_stage2(itsx_ctx *c);
-int trim_bounds_dev(itsx_ctx *c, int mode, const int64_t *d_off_sliced, int64_t nreads,
-                    uint8_t *d_keep, int32_t *d_lo, int32_t *d_hi, int64_t *n_kept, int64_t first = 0);
-int trim_gather_dev(itsx_ctx *c, const uint8_t *d_seq, const uint8_t *d_qual, const int64_t *d_off, int64_t nreads,
-                    const uint8_t *d_keep, const int32_t *d_lo, const int32_t *d_hi,
-                    int64_t *n_kept, int64_t *total, DevBuf &kept_index, DevBuf &out_off, DevBuf &out_seq,
-                    DevBuf &out_qual);
+// trim: bounds of the reads [first, first + count) -- d_off: offsets of caller-staged records, nullptr: the resident
+// reads -- into r_keep / r_lo / r_hi, r_nkept and r_total (one host synchronisation); then the re-expansion of their kept
+// slices of d_seq / d_qual (nullptr: bases only) into r_ki / r_oo / r_os / r_oq; trim_fetch_dev queues the copy of that
+// re-expansion to caller buffers (any may be NULL; the caller synchronises)
+int trim_bounds_dev(itsx_ctx *c, int mode, const int64_t *d_off, int64_t first, int64_t count);
+int trim_gather_dev(itsx_ctx *c, const uint8_t *d_seq, const uint8_t *d_qual);
+int trim_fetch_dev(itsx_ctx *c, int32_t *kept_index, int64_t *out_off, uint8_t *out_seq, uint8_t *out_qual);

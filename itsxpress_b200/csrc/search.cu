@@ -2392,18 +2392,14 @@ int search_build_seqs_from_reads(itsx_ctx *c, const int32_t *d_first, int64_t ns
 
 int search_build_seqs_from_host(itsx_ctx *c, const uint8_t *seq, const int64_t *off, int64_t nseq)
 {
-    // staged through separate buffers so that the reads of a previous itsx_derep stay resident
-    static thread_local DevBuf t_ascii, t_off;
     const int64_t total = nseq ? itsx_peek_i64(off + nseq) : 0;
-    CUDA_TRY(c, t_ascii.ensure((size_t)total + 64));
-    CUDA_TRY(c, t_off.ensure((size_t)(nseq + 1) * 8));
-    if (total) CUDA_TRY(c, cudaMemcpyAsync(t_ascii.p, seq, (size_t)total, cudaMemcpyDefault, c->stream));
-    if (nseq) CUDA_TRY(c, cudaMemcpyAsync(t_off.p, off, (size_t)(nseq + 1) * 8, cudaMemcpyDefault, c->stream));
+    CUDA_TRY(c, stage(c, c->d_stage_seq, seq, (size_t)total, 64));
+    CUDA_TRY(c, stage(c, c->d_stage_off, off, nseq ? (size_t)(nseq + 1) * 8 : 0, 8));
     c->shard_first = 0;
     c->shard_n = -1;
     c->have_samples = false;       // caller-supplied sequences are one sample
     c->n_samples = 1;
-    return build_seqs(c, t_ascii.as<uint8_t>(), t_off.as<int64_t>(), nullptr, nseq);
+    return build_seqs(c, c->d_stage_seq.as<uint8_t>(), c->d_stage_off.as<int64_t>(), nullptr, nseq);
 }
 
 constexpr int NLANE = 8;                   // side streams of the per-profile launches

@@ -226,17 +226,8 @@ int itsx_shard_owner_derep(itsx_ctx *c, const uint64_t *rec, int64_t nrec, const
     CUDA_TRY(c, cudaSetDevice(c->device));
     if (nrec < 0 || nbytes < 0 || (nrec && !rec) || (nbytes && !bases)) { c->err = "shard_owner_derep: bad argument"; return ITSX_EINVAL; }
     cudaStream_t st = c->stream;
-    c->nreads = nrec;
-    c->total_bases = nbytes;
-    c->n_unique = 0;
-    c->cl_active = false;
-    c->map_external = false;
-    c->pos_valid = false;
+    reset_reads(c, nrec, nbytes);
     c->sh_G = 0;
-    c->have_samples = false;
-    c->n_samples = 1;
-    c->qual_resident = false;
-    c->r_gathered = false;
     const size_t padded = ((size_t)nbytes + 15) / 16 * 16 + 32;
     CUDA_TRY(c, c->d_ascii.ensure(padded));
     CUDA_TRY(c, c->d_off.ensure((size_t)(nrec + 1) * 8));

@@ -98,70 +98,83 @@ gather_kernel(const uint8_t *__restrict__ seq, const uint8_t *__restrict__ qual,
 
 }  // namespace
 
-int trim_bounds_dev(itsx_ctx *c, int mode, const int64_t *d_off_sliced, int64_t nreads,
-                    uint8_t *d_keep, int32_t *d_lo, int32_t *d_hi, int64_t *n_kept, int64_t first)
+int trim_bounds_dev(itsx_ctx *c, int mode, const int64_t *d_off, int64_t first, int64_t count)
 {
     cudaStream_t st = c->stream;
     if (!c->pos_valid) { c->err = "trim: no position table (run itsx_search or itsx_positions_set first)"; return ITSX_EINVAL; }
-    if (first < 0 || nreads < 0 || first + nreads > c->nreads) {
+    if (first < 0 || count < 0 || first + count > c->nreads) {
         c->err = "trim: read range outside the dereplicated set";
         return ITSX_EINVAL;
     }
-    if (nreads == 0) { if (n_kept) *n_kept = 0; return ITSX_OK; }
-    CUDA_TRY(c, c->d_flag.ensure((size_t)(nreads + 1) * 4));
-    CUDA_TRY(c, c->d_scan.ensure((size_t)(nreads + 1) * 4));
-    CUDA_TRY(c, c->d_list.ensure((size_t)(nreads + 1) * 8));
-    CUDA_TRY(c, c->d_list2.ensure((size_t)(nreads + 1) * 8));
+    c->r_gathered = false;
+    c->r_n = count;
+    c->r_off = d_off ? d_off : c->d_off.as<int64_t>() + first;
+    c->r_nkept = c->r_total = 0;
+    CUDA_TRY(c, c->r_keep.ensure((size_t)count + 16));
+    CUDA_TRY(c, c->r_lo.ensure((size_t)count * 4 + 16));
+    CUDA_TRY(c, c->r_hi.ensure((size_t)count * 4 + 16));
+    if (count == 0) return ITSX_OK;
+    // keep flags and slice lengths, and their exclusive scans (kept rank, output offset): what trim_gather_dev reads
+    CUDA_TRY(c, c->d_flag.ensure((size_t)(count + 1) * 4));
+    CUDA_TRY(c, c->d_scan.ensure((size_t)(count + 1) * 4));
+    CUDA_TRY(c, c->d_list.ensure((size_t)(count + 1) * 8));
+    CUDA_TRY(c, c->d_list2.ensure((size_t)(count + 1) * 8));
     int32_t *kf = c->d_flag.as<int32_t>(), *ks = c->d_scan.as<int32_t>();
     int64_t *ol = c->d_list.as<int64_t>(), *os = c->d_list2.as<int64_t>();
-    bounds_kernel<<<nblk(nreads, 256), 256, 0, st>>>(c->d_uid.as<int32_t>() + first, c->d_pos.as<int32_t>(), c->npos,
-                                                     d_off_sliced ? d_off_sliced : c->d_off.as<int64_t>() + first, nreads, mode,
-                                                     d_keep, d_lo, d_hi, kf, ol);
-    CUDA_TRY(c, cudaMemsetAsync(kf + nreads, 0, 4, st));
-    CUDA_TRY(c, cudaMemsetAsync(ol + nreads, 0, 8, st));
-    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, kf, ks, (int)nreads + 1, st); },
-                        [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, ol, os, (int)nreads + 1, st); }));
+    bounds_kernel<<<nblk(count, 256), 256, 0, st>>>(c->d_uid.as<int32_t>() + first, c->d_pos.as<int32_t>(), c->npos, c->r_off,
+                                                    count, mode, c->r_keep.as<uint8_t>(), c->r_lo.as<int32_t>(),
+                                                    c->r_hi.as<int32_t>(), kf, ol);
+    CUDA_TRY(c, cudaMemsetAsync(kf + count, 0, 4, st));
+    CUDA_TRY(c, cudaMemsetAsync(ol + count, 0, 8, st));
+    CUDA_TRY(c, cub_run(c, [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, kf, ks, (int)count + 1, st); },
+                        [&](void *t, size_t &b) { return cub::DeviceScan::ExclusiveSum(t, b, ol, os, (int)count + 1, st); }));
     c->launches += 3;
     int32_t nk = 0;
-    CUDA_TRY(c, cudaMemcpyAsync(&nk, ks + nreads, 4, cudaMemcpyDeviceToHost, st));
+    int64_t tot = 0;
+    CUDA_TRY(c, cudaMemcpyAsync(&nk, ks + count, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaMemcpyAsync(&tot, os + count, 8, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     CUDA_TRY(c, cudaGetLastError());
-    if (n_kept) *n_kept = nk;
+    c->r_nkept = nk;
+    c->r_total = tot;
     return ITSX_OK;
 }
 
-// must follow trim_bounds_dev on the same stream (uses its scans)
-int trim_gather_dev(itsx_ctx *c, const uint8_t *d_seq, const uint8_t *d_qual, const int64_t *d_off, int64_t nreads,
-                    const uint8_t *d_keep, const int32_t *d_lo, const int32_t *d_hi,
-                    int64_t *n_kept, int64_t *total, DevBuf &kept_index, DevBuf &out_off, DevBuf &out_seq,
-                    DevBuf &out_qual)
+int trim_gather_dev(itsx_ctx *c, const uint8_t *d_seq, const uint8_t *d_qual)
 {
-    (void)d_keep;
     cudaStream_t st = c->stream;
-    int32_t *kf = c->d_flag.as<int32_t>(), *ks = c->d_scan.as<int32_t>();
-    int64_t *os = c->d_list2.as<int64_t>();
-    int32_t nk = 0;
-    int64_t tot = 0;
-    if (nreads > 0) {
-        CUDA_TRY(c, cudaMemcpyAsync(&nk, ks + nreads, 4, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(c, cudaMemcpyAsync(&tot, os + nreads, 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(c, cudaStreamSynchronize(st));
+    const int64_t n = c->r_n, nk = c->r_nkept, tot = c->r_total;
+    CUDA_TRY(c, c->r_ki.ensure((size_t)std::max<int64_t>(nk, 1) * 4));
+    CUDA_TRY(c, c->r_oo.ensure((size_t)(nk + 1) * 8));
+    CUDA_TRY(c, c->r_os.ensure((size_t)std::max<int64_t>(tot, 1)));
+    if (d_qual) CUDA_TRY(c, c->r_oq.ensure((size_t)std::max<int64_t>(tot, 1)));
+    if (n == 0) {
+        CUDA_TRY(c, cudaMemsetAsync(c->r_oo.p, 0, 8, st));
+    } else {
+        CUDA_TRY(c, c->d_gather.ensure((size_t)std::max<int64_t>(nk, 1) * sizeof(GatherRec)));
+        kept_index_kernel<<<nblk(n + 1, 256), 256, 0, st>>>(c->d_flag.as<int32_t>(), c->d_scan.as<int32_t>(),
+                                                            c->d_list2.as<int64_t>(), c->r_off, c->r_lo.as<int32_t>(),
+                                                            c->r_hi.as<int32_t>(), n, c->r_ki.as<int32_t>(),
+                                                            c->r_oo.as<int64_t>(), c->d_gather.as<GatherRec>());
+        if (nk > 0)
+            gather_kernel<<<nblk(nk * GATHER_W, 256), 256, 0, st>>>(d_seq, d_qual, c->d_gather.as<GatherRec>(), nk,
+                                                                    c->r_os.as<uint8_t>(),
+                                                                    d_qual ? c->r_oq.as<uint8_t>() : nullptr);
+        c->launches += 2;
+        CUDA_TRY(c, cudaGetLastError());
     }
-    *n_kept = nk;
-    *total = tot;
-    CUDA_TRY(c, kept_index.ensure((size_t)std::max(nk, 1) * 4));
-    CUDA_TRY(c, out_off.ensure((size_t)(nk + 1) * 8));
-    CUDA_TRY(c, out_seq.ensure((size_t)std::max<int64_t>(tot, 1)));
-    if (d_qual) CUDA_TRY(c, out_qual.ensure((size_t)std::max<int64_t>(tot, 1)));
-    if (nreads == 0) { CUDA_TRY(c, cudaMemsetAsync(out_off.p, 0, 8, st)); return ITSX_OK; }
-    CUDA_TRY(c, c->d_gather.ensure((size_t)std::max(nk, 1) * sizeof(GatherRec)));
-    kept_index_kernel<<<nblk(nreads + 1, 256), 256, 0, st>>>(kf, ks, os, d_off, d_lo, d_hi, nreads, kept_index.as<int32_t>(),
-                                                             out_off.as<int64_t>(), c->d_gather.as<GatherRec>());
-    if (nk > 0)
-        gather_kernel<<<nblk((int64_t)nk * GATHER_W, 256), 256, 0, st>>>(d_seq, d_qual, c->d_gather.as<GatherRec>(), nk,
-                                                                         out_seq.as<uint8_t>(),
-                                                                         d_qual ? out_qual.as<uint8_t>() : nullptr);
-    c->launches += 2;
-    CUDA_TRY(c, cudaGetLastError());
+    c->r_gathered = true;
+    c->r_gathered_qual = d_qual != nullptr;
+    return ITSX_OK;
+}
+
+int trim_fetch_dev(itsx_ctx *c, int32_t *kept_index, int64_t *out_off, uint8_t *out_seq, uint8_t *out_qual)
+{
+    cudaStream_t st = c->stream;
+    const int64_t nk = c->r_nkept, tot = c->r_total;
+    if (kept_index && nk) CUDA_TRY(c, cudaMemcpyAsync(kept_index, c->r_ki.p, (size_t)nk * 4, cudaMemcpyDefault, st));
+    if (out_off) CUDA_TRY(c, cudaMemcpyAsync(out_off, c->r_oo.p, (size_t)(nk + 1) * 8, cudaMemcpyDefault, st));
+    if (out_seq && tot) CUDA_TRY(c, cudaMemcpyAsync(out_seq, c->r_os.p, (size_t)tot, cudaMemcpyDefault, st));
+    if (out_qual && tot && c->r_gathered_qual) CUDA_TRY(c, cudaMemcpyAsync(out_qual, c->r_oq.p, (size_t)tot, cudaMemcpyDefault, st));
     return ITSX_OK;
 }

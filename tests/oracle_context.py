@@ -261,7 +261,7 @@ class OracleContext:
         idx = np.repeat(off[ki + base] + lo[ki] - oo[:-1], lens) + np.arange(int(oo[-1]), dtype=np.int64)
         return ki, oo, seq[idx], None if qual is None else qual[idx]
 
-    def trim_gather(self, nreads, mode=0, seq=None, qual=None, off=None, resident_qual=False):
+    def trim_gather(self, nreads, mode=0, seq=None, qual=None, off=None):
         self._note("trim_gather")
         off = np.ascontiguousarray(off, dtype=np.int64)
         assert nreads == len(off) - 1 == len(self._map[0])
